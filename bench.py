@@ -603,6 +603,39 @@ def bench_genome(a):
     print(json.dumps(line))
 
 
+def world_size():
+    return int(os.environ.get("WORLD_SIZE", "1"))
+
+
+DUMP_RECORDS = 1 << 15
+DUMP_QUAL_VALUES = 1 << 23                                       # 32 MiB of float32 qualities
+DUMP_LIMIT = 64 << 20
+
+
+def dump_outputs(d, bb, res):
+    """What a caller of the timed path receives (cg_download after the last cg_run), as .npy files in d, DUMP_LIMIT bytes at most
+    (about 20 MB at C2): the rewritten quality strings of a fixed sample of up to DUMP_RECORDS records (seed 0; float32,
+    concatenated in sample order, at most DUMP_QUAL_VALUES values, with each sampled record's index and length), the BED events
+    (tid, pos, tag; float64; a fixed sample of rows, seed 1, in list order when the whole list would not fit) and the 19 counters
+    (float64, in COUNTER_NAMES order).  The inputs are seeded, so two builds given the same arguments can be compared file for file."""
+    import crumble_b200 as cb
+    os.makedirs(d, exist_ok=True)
+    off, ln = bb.offsets(), bb.lengths()
+    idx = np.sort(np.random.default_rng(0).choice(off.size, min(DUMP_RECORDS, off.size), replace=False))
+    idx = idx[np.cumsum(ln[idx].astype(np.int64)) <= DUMP_QUAL_VALUES]
+    qual = np.concatenate([res["qual"][int(off[i]): int(off[i]) + int(ln[i])] for i in idx]) if idx.size else np.zeros(0, np.uint8)
+    ev = res["events"]
+    arrays = {"qual_sample": qual.astype(np.float32), "qual_sample_records": idx.astype(np.float64), "qual_sample_lengths": ln[idx].astype(np.float64),
+              "counters": np.array([res["counters"][k] for k in cb.COUNTER_NAMES], dtype=np.float64)}
+    rows = (DUMP_LIMIT - 4096 - sum(a.nbytes for a in arrays.values())) // 24          # 4096: room for the five .npy headers
+    if len(ev) > rows:
+        ev = ev[np.sort(np.random.default_rng(1).choice(len(ev), rows, replace=False))]
+    arrays["events"] = np.stack([ev["tid"], ev["pos"], ev["tag"]], axis=1).astype(np.float64) if len(ev) else np.zeros((0, 3))
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_LIMIT - 4096
+    for name, arr in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), arr)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -616,10 +649,13 @@ def main():
     ap.add_argument("--no-pack", action="store_true", help="upload the plain 4-bit / 8-bit arrays instead of the batcher's compact planes")
     ap.add_argument("--replicas", action="store_true", help="N > 1: one private copy of the workload per GPU (weak scaling) instead of region shards of one contig")
     ap.add_argument("--no-parity", action="store_true", help="N > 1: skip the whole-contig comparison rank 0 makes after the timed regions")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="one GPU: write what the last timed step computed as DIR/<name>.npy (see dump_outputs)")
     a = ap.parse_args()
+    if a.dump_outputs and (a.impl == "reference" or a.workload == "C5" or world_size() > 1):
+        raise SystemExit("--dump-outputs is supported for the one-GPU run of the resident chain only")
     if a.warmup < 3 and a.impl != "reference":
         a.warmup = 3
-    rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1"))
+    rank = int(os.environ.get("RANK", "0")); world = world_size()
     local = int(os.environ.get("LOCAL_RANK", "0"))
     if a.impl == "reference":
         if a.workload == "C5" and a.scale == 1.0:
@@ -693,6 +729,11 @@ def main():
         dist.all_reduce(tmax, op=dist.ReduceOp.MAX); dist.all_reduce(tot_bases, op=dist.ReduceOp.SUM)
     dev_ms_max = float(tmax.item()); all_bases = float(tot_bases.item())
     value = all_bases * a.steps / (dev_ms_max * 1e-3)
+    if a.dump_outputs:
+        res = g.download(batch)
+        if res["n_events"] > len(res["events"]):
+            res = g.download(batch, events_cap=res["n_events"])
+        dump_outputs(a.dump_outputs, bb, res)
 
     # ---- end to end: pinned host SoA -> C ABI -> host quality buffer, copies inside the timed region
     qout = torch.empty(max(int(batch.qual_bytes), 1), dtype=torch.uint8, pin_memory=True).numpy()

@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """Regenerates the golden fixtures from oracle/_ref (the reference's own sources compiled
-verbatim; needs /root/reference at build time, so this only runs in the build container).
+verbatim: make -C oracle ref REF=<crumble source tree>).
 
     python tests/golden/make_golden.py
+    python tests/golden/make_golden.py --oracle-runs recorded.jsonl ...
 
 Outputs (committed):
   golden.json                      sha256 of the rewritten quality bytes, BED text and -v counters for
@@ -10,6 +11,12 @@ Outputs (committed):
   edge_cases.<tag>.qual.txt        rewritten quality strings of tests/golden/edge_cases.sam, one read per line
   edge_cases.<tag>.bed             BED output for the same runs
   ref_columns.tiny.-9.txt          the reference's own -DDEBUG per-column dump (call / score / preserve mark)
+  oracle_runs.json                 (--oracle-runs) the vectors every default oracle run of the tests is pinned to (tests/util.py):
+                                   the JSON lines that `CRUMBLE_ORACLE_RECORD=recorded.jsonl pytest tests` appends, merged, plus the
+                                   sha256 of the -DDEBUG per-column lines test_gpu_columns_match_reference_debug_dump checks; made
+                                   with the oracle of record (the reference when oracle/_ref is built, else the restatement), and each
+                                   labelled with it ("made_by"); restatement vectors on golden.json's inputs say whether they equal
+                                   the reference's vector there ("equals_reference")
 """
 import hashlib
 import json
@@ -22,7 +29,7 @@ ROOT = HERE.parent.parent
 sys.path.insert(0, str(ROOT)); sys.path.insert(0, str(ROOT / "tests"))
 import numpy as np  # noqa: E402
 import crumble_b200 as cb  # noqa: E402
-from util import run_oracle, valid_mask  # noqa: E402
+from util import REF_BIN, run_oracle, valid_mask  # noqa: E402
 
 SETS = {"tiny": ("tiny", 1.0, 3), "c1s": ("C1", 0.1, 11), "c2s": ("C2", 1 / 512, 5), "c4s": ("C4", 0.02, 4)}
 ARGS = [["-9"], ["-8"], ["-7"], ["-5"], ["-3"], ["-1"], ["-1", "-B"], ["-9", "-Y0.1"], ["-5", "-q30"], ["-9", "-U30"],
@@ -41,6 +48,46 @@ EDGE = {"l9": ["-9"], "l1B": ["-1", "-B"], "l5q30": ["-5", "-q30"], "l3U35": ["-
         "l9r": ["-9", "-r", "chrA:900-1600"], "l1r": ["-1", "-r", "chrA:1200-2100"]}
 
 
+def oracle_runs(recorded):
+    import hashlib as H
+    import os, tempfile
+    from util import STORED, oracle_bin, stored_key
+    from test_gpu_parity import debug_dump_lines
+    runs = {}
+    for path in recorded:
+        for line in open(path):
+            for k, v in json.loads(line).items():
+                assert runs.setdefault(k, v) == v, f"two different vectors recorded for {k!r}"
+    for name, g in json.load(open(HERE / "golden.json")).items():
+        data, _, _ = cb.simulate(g["preset"], g["scale"], g["seed"])
+        for args, exp in g["runs"].items():
+            v = runs.get(stored_key(H.sha256(data.tobytes()).hexdigest(), args.split()))
+            if v is not None and v["made_by"] != "reference":
+                v["equals_reference"] = v["qual_sha256"] == exp["qual_sha256"] and v["counters"] == exp["counters"] and \
+                    v["bed_sha256"] == H.sha256(exp["bed"].encode()).hexdigest()
+    binary, kind = oracle_bin()
+    for preset, scale, seed, args in (("tiny", 1.0, 3, ["-9"]), ("C1", 0.25, 11, ["-9"]), ("C1", 0.25, 11, ["-1"])):
+        data, _, _ = cb.simulate(preset, scale, seed)
+        with tempfile.TemporaryDirectory() as td:
+            fin, dump = os.path.join(td, "i.ubam"), os.path.join(td, "cols.bin")
+            data.tofile(fin)
+            if kind == "reference":
+                dbg = subprocess.run([str(binary.parent / "crumble_ref_debug"), "-z"] + args + [fin, "mem:x"], stdout=subprocess.PIPE, text=True, check=True).stdout
+                lines = []
+                for l in dbg.splitlines():
+                    if l.startswith("Depth "):
+                        e = l.split("\t")
+                        lines.append("\t".join([e[0].split(" ")[1]] + e[1:4] + [e[4] if len(e) > 4 and e[4] == "*" else ""]))
+            else:
+                subprocess.run([str(binary), "-z"] + args + [fin, "mem:x"], check=True, env=dict(os.environ, ORACLE_COLUMN_DUMP=dump))
+                lines = debug_dump_lines(np.fromfile(dump, dtype=cb.api.COLUMN_DTYPE))
+        runs["columns " + stored_key(H.sha256(data.tobytes()).hexdigest(), args)] = {
+            "sha256": H.sha256("\n".join(lines).encode()).hexdigest(), "made_by": "reference" if kind == "reference" else "restatement"}
+    with open(STORED, "w") as f:                                # one vector per line
+        f.write("{\n" + ",\n".join(f"{json.dumps(k)}: {json.dumps(runs[k], sort_keys=True)}" for k in sorted(runs)) + "\n}\n")
+    print(f"{len(runs)} oracle vectors written ({kind})")
+
+
 def main():
     ref = ROOT / "oracle" / "_ref" / "crumble_ref"
     assert ref.exists(), "build oracle/_ref first (make -C oracle ref)"
@@ -52,7 +99,7 @@ def main():
         gold[name] = {"preset": preset, "scale": scale, "seed": seed, "reads": nr, "aligned_bases": nb,
                       "input_sha256": hashlib.sha256(data.tobytes()).hexdigest(), "runs": {}}
         for a in ARGS:
-            r = run_oracle(data, a, kind="reference")
+            r = run_oracle(data, a, binary=REF_BIN, kind="reference")
             gold[name]["runs"][" ".join(a)] = {"qual_sha256": hashlib.sha256(r["qual"][m].tobytes()).hexdigest(),
                                                "bed": r["bed"], "counters": r["counters"]}
         if name in OPT_SETS:
@@ -60,7 +107,7 @@ def main():
             bedf.write_text(KEEP_BED[name])
             gold[name]["opt_runs"] = {}
             for a in OPT_ARGS:
-                r = run_oracle(data, [str(bedf) if x == "BED" else x for x in a], kind="reference")
+                r = run_oracle(data, [str(bedf) if x == "BED" else x for x in a], binary=REF_BIN, kind="reference")
                 gold[name]["opt_runs"][" ".join(a)] = {"qual_sha256": hashlib.sha256(r["qual"][m].tobytes()).hexdigest(),
                                                        "bed": r["bed"], "counters": r["counters"]}
         bb.close()
@@ -95,4 +142,7 @@ def main():
 
 
 if __name__ == "__main__":
-    main()
+    if sys.argv[1:2] == ["--oracle-runs"]:
+        oracle_runs(sys.argv[2:])
+    else:
+        main()

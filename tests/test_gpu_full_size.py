@@ -1,4 +1,5 @@
-"""BASELINE.json's full-size configurations on the GPU against the reference's own code (oracle/_ref) at the SAME size:
+"""BASELINE.json's full-size configurations on the GPU against the CPU oracle at the SAME size (tests/util.py: the reference's own code
+when oracle/_ref is built, else the restatement pinned to the stored vectors of tests/golden/oracle_runs.json):
 synthetic chr20 (64 Mb at 30x: 1.29e7 reads, 1.92e9 aligned bases) at -9 (configs[1]) and -1 -B (configs[2]) over the whole file,
 the 1 Mb region (configs[0]) and the 1000x amplicon panel (configs[3]); plus slicing invariance at full size."""
 import numpy as np
@@ -18,24 +19,24 @@ def _bytes_of(off, ln):
 
 
 def _start_reference(fin, td, tag, args):
-    """the verbatim reference (oracle/_ref) on the whole file, in the background: one core, about 75 s for chr20 at 30x"""
+    """the oracle of record on the whole file, in the background: one core, about 75 s for chr20 at 30x"""
     import os, subprocess
     from util import oracle_bin
     binary, kind = oracle_bin()
-    assert kind == "reference"
     fout, fbed = os.path.join(td, f"out.{tag}.ubam"), os.path.join(td, f"out.{tag}.bed")
     pr = subprocess.Popen([str(binary), "-z", "-v"] + args + ["-b", fbed, "-O", "bam,raw", fin, fout], stdout=subprocess.DEVNULL, stderr=subprocess.PIPE, text=True)
-    return pr, fout, fbed
+    return pr, fout, fbed, kind, args
 
 
-def _collect_reference(pr, fout, fbed):
-    from util import parse_counters
+def _collect_reference(pr, fout, fbed, kind, args, data_sha256):
+    from util import parse_counters, pin_to_stored
     err = pr.communicate()[1]
     assert pr.returncode == 0, err[-2000:]
     out = np.fromfile(fout, dtype=np.uint8)
     rb = cb.BatchBuilder(pinned=False); rb.add_bam_stream(out); rb.finish()
     del out
-    res = {"qual": rb.qual().copy(), "off": rb.offsets(), "len": rb.lengths(), "bed": open(fbed).read(), "counters": parse_counters(err)}
+    res = {"qual": rb.qual().copy(), "off": rb.offsets(), "len": rb.lengths(), "bed": open(fbed).read(), "counters": parse_counters(err), "kind": kind}
+    pin_to_stored(res, data_sha256, args, valid_mask(rb))
     rb.close()
     return res
 
@@ -43,10 +44,11 @@ def _collect_reference(pr, fout, fbed):
 def test_full_size_c2_c3_whole_file_vs_reference():
     """BASELINE.json configs[1] (crumble -9) and configs[2] (crumble -1 -B) on the WHOLE synthetic chr20 (64 Mb, 30x: 1.29e7 reads,
     1.92e9 aligned bases): every quality byte, the BED text and the 19 counters of the GPU path against the reference's own code
-    (oracle/_ref) run over the whole file, one process per option set, while the GPU does its part; plus slicing invariance
+    (or the pinned restatement) run over the whole file, one process per option set, while the GPU does its part; plus slicing invariance
     (resident == streamed at two chunk sizes) at this size."""
-    import os, tempfile
+    import hashlib, os, tempfile
     data, n_reads, n_bases = cb.simulate("C2", 1.0, seed=2)
+    data_sha256 = hashlib.sha256(data.tobytes()).hexdigest()
     assert n_reads > 12_000_000 and n_bases > 1_900_000_000
     names = header_names(data)
     tmpdir = "/dev/shm" if os.path.isdir("/dev/shm") else None
@@ -77,7 +79,7 @@ def test_full_size_c2_c3_whole_file_vs_reference():
             g.close()
         off, ln = bb.offsets(), bb.lengths()
         for k in runs:
-            ref = _collect_reference(*procs[k])
+            ref = _collect_reference(*procs[k], data_sha256)
             assert np.array_equal(ref["off"], off) and np.array_equal(ref["len"], ln), f"{k}: the reference wrote different records"
             nbad = int((got[k]["qual"] != ref["qual"][mask]).sum())
             assert nbad == 0, f"{k}: {nbad} of {int(mask.sum())} quality bytes differ from the reference run over the whole file"

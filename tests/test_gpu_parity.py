@@ -226,30 +226,51 @@ def test_gpu_columns_bit_exact():
         g.close()
 
 
+def debug_dump_lines(cols):
+    """processed columns as the reference's -DDEBUG printout shows them (snp_score.c:1545-1573): tid, position, depth, call or het call
+    with its score, preserve mark"""
+    proc = cols[(cols["flags"] & 8) != 0]
+    out = []
+    for c in proc:
+        s = ("%c/%c %4d" % ("ACGT*"[c["het_call"] // 5], "ACGT*"[c["het_call"] % 5], c["het_phred"])) if c["het_phred"] > 0 else ("%c   %4d" % ("ACGT*N"[c["call"]], c["phred"]))
+        out.append("%d\t%d\t%d\t%s\t%s" % (c["tid"], c["pos"] + 1, c["n_plp"], s, "*" if c["flags"] & 1 else ""))
+    return out
+
+
 @pytest.mark.parametrize("name,args", [("tiny", ["-9"]), ("c1s", ["-9"]), ("c1s", ["-1"])], ids=lambda v: "".join(v) if isinstance(v, list) else v)
 def test_gpu_columns_match_reference_debug_dump(name, args):
     """the same per-column dump against the REFERENCE's own -DDEBUG printout (snp_score.c:1545-1573; oracle/_ref/crumble_ref_debug,
-    compiled from the reference's sources): position, depth, call or het call, score, and the preserve mark, for every processed column"""
-    from util import REF_BIN
+    compiled from the reference's sources): position, depth, call or het call, score, and the preserve mark, for every processed column.
+    Without oracle/_ref: tiny -9 is checked against the reference's printout stored in tests/golden/ref_columns.tiny.-9.txt (the first
+    20000 processed columns of chr1), and every case's whole printout against its stored sha256 in tests/golden/oracle_runs.json (key
+    "columns <input> <options>"), which names the oracle that made it; the c1s hashes were made by the restatement, so for c1s this is a
+    check against the restatement pinned in the repository, not against the reference."""
+    from util import REF_BIN, STORED, stored_key
     dbg_bin = REF_BIN.parent / "crumble_ref_debug"
-    assert dbg_bin.exists(), f"{dbg_bin} is missing (make -C oracle ref where /root/reference exists)"
     data, bb, batch, mask = dataset(name)
     g = cb.Crumble(params_from_args(args), device=0)
     cols = g.process(batch, want_columns=True)["columns"]
     g.close()
+    got = debug_dump_lines(cols)
+    assert len(got) > 1000
+    if not dbg_bin.exists():
+        ref_file = GDIR / f"ref_columns.{name}.{''.join(args)}.txt"
+        if ref_file.exists():
+            exp = [l.rstrip("\n").split("\t") for l in open(ref_file)]
+            chr1 = [c.split("\t")[1:] for c in got if c.startswith("0\t")][: len(exp)]
+            assert len(chr1) == len(exp)
+            for e, c in zip(exp, chr1):
+                assert e[:3] + [e[3] if len(e) > 3 else ""] == c, (e, c)
+        exp = json.load(open(STORED))["columns " + stored_key(hashlib.sha256(data.tobytes()).hexdigest(), args)]
+        assert hashlib.sha256("\n".join(got).encode()).hexdigest() == exp["sha256"], f"differs from the printout stored by the {exp['made_by']}"
+        return
     with tempfile.TemporaryDirectory() as td:
         fin = os.path.join(td, "i.ubam"); data.tofile(fin)
         txt = subprocess.run([str(dbg_bin), "-z"] + args + [fin, "mem:x"], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True, check=True).stdout
     exp = [l.split("\t") for l in txt.splitlines() if l.startswith("Depth ")]
-    proc = cols[(cols["flags"] & 8) != 0]
-    assert len(proc) == len(exp) and len(exp) > 1000
-    het = proc["het_phred"] > 0
-    for i, e in enumerate(exp):
-        c = proc[i]
-        assert int(e[0].split(" ")[1]) == c["tid"] and int(e[1]) == c["pos"] + 1 and int(e[2]) == c["n_plp"], (e, c)
-        s = ("%c/%c %4d" % ("ACGT*"[c["het_call"] // 5], "ACGT*"[c["het_call"] % 5], c["het_phred"])) if het[i] else ("%c   %4d" % ("ACGT*N"[c["call"]], c["phred"]))
-        assert e[3] == s, (e, c)
-        assert (len(e) > 4 and e[4] == "*") == bool(c["flags"] & 1), (e, c)
+    assert len(got) == len(exp)
+    for e, c in zip(exp, got):
+        assert [e[0].split(" ")[1]] + e[1:4] + [e[4] if len(e) > 4 and e[4] == "*" else ""] == c.split("\t"), (e, c)
 
 
 def test_gpu_contig_sharding_invariance():

@@ -40,7 +40,7 @@ def test_port_matches_golden(name):
         assert r["counters"] == exp["counters"], args
 
 
-@pytest.mark.skipif(not REF_BIN.exists(), reason="oracle/_ref not built (needs /root/reference)")
+@pytest.mark.skipif(not REF_BIN.exists(), reason="oracle/_ref not built (make -C oracle ref REF=<crumble source tree>)")
 def test_port_matches_reference_binary_fresh_seed():
     data, _, _ = cb.simulate("C1", 0.05, 777, threads=2)
     bb = cb.BatchBuilder(pinned=False); bb.add_bam_stream(data); bb.finish()

@@ -1,10 +1,19 @@
 """Test helpers: run the CPU oracle on a raw BAM stream and bring its output into the
 same structure-of-arrays layout the GPU path uses.
 
-Oracle choice: oracle/_ref/crumble_ref (the reference's own sources compiled verbatim,
-built where /root/reference exists and shipped as a binary).  A missing binary is an error,
-not a downgrade; oracle/bin/crumble_oracle (this repository's plain-C restatement) is used
-only where a test asks for it by name."""
+Oracle choice: oracle/_ref/crumble_ref (the reference's own sources compiled verbatim with
+make -C oracle ref REF=<crumble source tree>) when it is built; otherwise "stored":
+oracle/bin/crumble_oracle (this repository's plain-C restatement, which reproduces every vector
+of golden.json made with the reference) pinned to tests/golden/oracle_runs.json.  Either way
+the checker's output for every input and option set the parity tests use must equal the stored
+vector (sha256 of the quality bytes and of the BED text, the -v counters), so a change to the
+oracle cannot move the bar.  Every stored vector names the oracle that made it ("made_by":
+"reference" or "restatement"); a restatement vector whose input and options golden.json also
+covers says whether it equals the reference's vector there ("equals_reference").  Run with
+oracle/_ref built and re-record to replace restatement vectors with the reference's own.
+kind="port" runs the restatement unpinned."""
+import hashlib
+import json
 import os
 import re
 import subprocess
@@ -17,21 +26,43 @@ ROOT = Path(__file__).resolve().parent.parent
 REF_BIN = ROOT / "oracle" / "_ref" / "crumble_ref"
 PORT_BIN = ROOT / "oracle" / "bin" / "crumble_oracle"
 EMU_BIN = ROOT / "tests" / "emu" / "emu_crumble"
+STORED = ROOT / "tests" / "golden" / "oracle_runs.json"
 
 
 def oracle_bin(kind=None):
-    """kind None = the checker of record: the verbatim reference (oracle/_ref).  There is no silent downgrade to the port: a parity
-    claim made against the restatement must say so (kind="port", or CRUMBLE_ORACLE=port in the environment)."""
+    """kind None = the checker of record: the verbatim reference when oracle/_ref is built, else the restatement pinned to the stored
+    vectors (kind "stored"); CRUMBLE_ORACLE in the environment overrides the choice."""
     if kind is None:
-        kind = os.environ.get("CRUMBLE_ORACLE", "reference")
+        kind = os.environ.get("CRUMBLE_ORACLE") or ("reference" if REF_BIN.exists() else "stored")
     if kind == "reference":
         if REF_BIN.exists():
             return REF_BIN, "reference"
-        raise FileNotFoundError(f"{REF_BIN} is missing: the parity tests compare with the reference's own code. Build it where /root/reference exists "
-                                "(make -C oracle ref; it travels to the GPU box with the snapshot) or set CRUMBLE_ORACLE=port to knowingly test against the restatement")
-    if kind == "port" and PORT_BIN.exists():
-        return PORT_BIN, "port"
+        raise FileNotFoundError(f"{REF_BIN} is missing: build it with make -C oracle ref REF=<crumble source tree>")
+    if kind in ("port", "stored") and PORT_BIN.exists():
+        return PORT_BIN, kind
     raise FileNotFoundError("no oracle binary: run __graft_entry__.build()")
+
+
+def stored_key(data_sha256, args):
+    return data_sha256 + " " + " ".join(args)
+
+
+def pin_to_stored(res, data_sha256, args, mask):
+    """The oracle's result for this input (sha256 of the uncompressed BAM stream) and these options must equal the stored vector.
+    With CRUMBLE_ORACLE_RECORD=<file> the vector is appended to that file (JSON lines) instead, to extend oracle_runs.json."""
+    got = {"qual_sha256": hashlib.sha256(res["qual"][mask].tobytes()).hexdigest(),
+           "bed_sha256": hashlib.sha256(res["bed"].encode()).hexdigest(), "counters": res["counters"]}
+    key = stored_key(data_sha256, args)
+    rec = os.environ.get("CRUMBLE_ORACLE_RECORD")
+    if rec:
+        with open(rec, "a") as f:
+            f.write(json.dumps({key: dict(got, made_by="reference" if res["kind"] == "reference" else "restatement")}, sort_keys=True) + "\n")
+        return
+    exp = json.load(open(STORED)).get(key)
+    assert exp is not None, f"no stored oracle vector for {key!r} in {STORED.name}"
+    assert got == {k: exp[k] for k in got}, \
+        f"the oracle ({res['kind']}) does not reproduce the stored vector for {key!r} (made by the {exp['made_by']})"
+    res["kind"] = f"{res['kind']}, pinned to a vector made by the {exp['made_by']}"
 
 
 def parse_counters(stderr_text):
@@ -71,6 +102,7 @@ def header_names(data: np.ndarray):
 def run_oracle(data: np.ndarray, args, kind=None, binary=None, timing=False, env_extra=None):
     """Run the oracle CLI on an uncompressed BAM stream; returns quals in batch layout, BED text, counters."""
     import crumble_b200 as cb
+    pinned = binary is None and kind in (None, "reference", "stored")
     if binary is None:
         binary, kind = oracle_bin(kind)
     tmpdir = "/dev/shm" if os.path.isdir("/dev/shm") else None
@@ -92,6 +124,8 @@ def run_oracle(data: np.ndarray, args, kind=None, binary=None, timing=False, env
     m = re.search(r"transcode_seconds=([0-9.]+)", r.stderr)
     res = {"qual": bb.qual().copy(), "pos": bb.positions(), "len": bb.lengths(), "off": bb.offsets(), "bed": bed, "counters": parse_counters(r.stderr), "names": header_names(data),
            "kind": kind, "seconds": float(m[1]) if m else None, "stderr": r.stderr}
+    if pinned:
+        pin_to_stored(res, hashlib.sha256(data.tobytes()).hexdigest(), args, valid_mask(bb))
     bb.close()
     return res
 
