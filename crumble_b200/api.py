@@ -5,7 +5,8 @@ Host-side mirror of the reference interface for the hot path: the option block
 ``transcode`` (1336-2029) expressed as ``Crumble.process(batch)``.
 
 There is no CPU fallback: if the shared library is missing, or no CUDA device is
-usable, every compute call raises.  PyTorch is not needed by this module.
+usable, every compute call raises.  PyTorch is only imported by the device-resident entry
+(``device_batch``, ``Crumble.process_device``); everything else works without it.
 """
 from __future__ import annotations
 
@@ -81,6 +82,24 @@ class Batch(C.Structure):
     ]
 
 
+class DevBatch(C.Structure):
+    """cg_dev_batch: records already in GPU memory as concatenated BAM fields (include/crumble_gpu.h)."""
+    _fields_ = [
+        ("n_reads", C.c_int64),
+        ("tid", C.c_void_p), ("pos", C.c_void_p), ("flag", C.c_void_p), ("mapq", C.c_void_p),
+        ("l_qseq", C.c_void_p), ("n_cigar", C.c_void_p),
+        ("cigar", C.c_void_p), ("n_cigar_total", C.c_int64),
+        ("seq", C.c_void_p), ("seq_len", C.c_int64),
+        ("qual", C.c_void_p), ("qual_len", C.c_int64),
+    ]
+
+
+# the arrays of a cg_dev_batch, their numpy dtypes, and which of them hold one entry per record
+DEV_FIELDS = {"tid": np.int32, "pos": np.int32, "flag": np.uint16, "mapq": np.uint8, "l_qseq": np.int32, "n_cigar": np.uint16,
+              "cigar": np.uint32, "seq": np.uint8, "qual": np.uint8}
+DEV_PER_RECORD = ("tid", "pos", "flag", "mapq", "l_qseq", "n_cigar")
+
+
 class BedEvent(C.Structure):
     _fields_ = [("tid", C.c_int32), ("pos", C.c_int32), ("tag", C.c_int32)]
 
@@ -117,7 +136,7 @@ _sim = None
 
 EXPORTS = [
     "cg_abi_version", "cg_device_count", "cg_create", "cg_destroy", "cg_set_params", "cg_strerror", "cg_last_error",
-    "cg_set_stream", "cg_process", "cg_process_window", "cg_upload", "cg_run", "cg_download", "cg_sync", "cg_last_ms", "cg_last_launches", "cg_last_h2d_bytes",
+    "cg_set_stream", "cg_process", "cg_process_device", "cg_process_window", "cg_upload", "cg_run", "cg_download", "cg_sync", "cg_last_ms", "cg_last_launches", "cg_last_h2d_bytes",
     "cg_algorithmic_bytes", "cg_aligned_bases", "cg_n_columns", "cg_params_default", "cg_params_level",
     "cgb_create", "cgb_destroy", "cgb_reset", "cgb_add", "cgb_add_bam_stream", "cgb_finish", "cgb_bytes", "cgb_reserve", "cgb_pack",
     "cg_carry_export", "cg_carry_import", "cg_carry_is_neutral", "cg_batch_ends", "cg_shard_begin", "cg_shard_carry", "cg_shard_end",
@@ -154,6 +173,7 @@ def load_lib():
     for f in ("cg_process",):
         getattr(lib, f).argtypes = [C.c_void_p, C.POINTER(Batch), C.POINTER(Result)]
     lib.cg_process_window.argtypes = [C.c_void_p, C.POINTER(Batch), C.POINTER(Window), C.POINTER(Result)]
+    lib.cg_process_device.argtypes = [C.c_void_p, C.POINTER(DevBatch), C.c_void_p, C.POINTER(Result)]
     lib.cgb_reserve.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_int64]
     lib.cg_carry_export.argtypes = [C.c_void_p, C.c_void_p]
     lib.cg_carry_import.argtypes = [C.c_void_p, C.c_void_p]
@@ -292,6 +312,7 @@ class Crumble:
         if self.lib.cg_device_count() <= 0:
             raise CrumbleError("no usable CUDA device: the GPU path is mandatory, there is no CPU fallback")
         self.params = params if params is not None else default_params()
+        self.device = device
         err = C.c_int(0)
         self.h = self.lib.cg_create(C.byref(self.params), device, C.byref(err))
         if not self.h:
@@ -348,6 +369,66 @@ class Crumble:
         if want_columns:
             out["columns"] = cols[: int(res.n_columns)]
         return out
+
+    def process_device(self, tensors: dict, out=None, want_columns: bool = False, events_cap: int = 1 << 16):
+        """Records already in GPU memory (cg_process_device): ``tensors`` holds the concatenated BAM fields of ``device_batch`` as
+        contiguous 1-D tensors on this context's device; the rewritten qualities land in ``out`` (same layout, may be ``tensors["qual"]``
+        itself) or in a new tensor from torch's caching allocator.  Runs on torch's current stream of the device, so work queued there
+        before the call is its input and work queued after it sees the result.  Returns {"qual", "events", "counters"[, "columns"]}."""
+        import torch
+        dev = torch.device("cuda", self.device)
+        t = {}
+        for k, dt in DEV_FIELDS.items():
+            x = tensors.get(k)
+            if not isinstance(x, torch.Tensor):
+                raise CrumbleError(f"process_device: {k} must be a torch tensor")
+            if x.device != dev:
+                raise CrumbleError(f"process_device: {k} is on {x.device}, the context runs on {dev}")
+            if x.dtype != _torch_dtype(dt):
+                raise CrumbleError(f"process_device: {k} must be {_torch_dtype(dt)}, not {x.dtype}")
+            if x.dim() != 1 or not x.is_contiguous():
+                raise CrumbleError(f"process_device: {k} must be a contiguous 1-D tensor")
+            t[k] = x
+        n = t["tid"].numel()
+        for k in DEV_PER_RECORD:
+            if t[k].numel() != n:
+                raise CrumbleError(f"process_device: {k} has {t[k].numel()} entries, tid has {n}: one per record")
+        qual_len = t["qual"].numel()
+        if out is None:
+            out = torch.empty(qual_len, dtype=torch.uint8, device=dev)
+        elif not isinstance(out, torch.Tensor) or out.device != dev or out.dtype != torch.uint8 or out.dim() != 1 or not out.is_contiguous() \
+                or out.numel() != qual_len:
+            raise CrumbleError(f"process_device: out must be a contiguous uint8 tensor of {qual_len} bytes on {dev}")
+        db = DevBatch(n_reads=n, n_cigar_total=t["cigar"].numel(), seq_len=t["seq"].numel(), qual_len=qual_len)
+        for k in DEV_FIELDS:
+            setattr(db, k, t[k].data_ptr() or None)
+        self.set_stream(torch.cuda.current_stream(dev).cuda_stream)
+        events_cap = max(events_cap, getattr(self, "_events_hint", 0))
+        ev = np.zeros(events_cap, dtype=EVENT_DTYPE)
+        res = Result(events=ev.ctypes.data_as(C.POINTER(BedEvent)), events_cap=events_cap)
+        cols = None
+        if want_columns:
+            cap = int(getattr(self, "_ncols_hint", 0)) or 1
+            cols = np.zeros(cap, dtype=COLUMN_DTYPE)
+            res.columns, res.columns_cap = cols.ctypes.data_as(C.POINTER(Column)), cap
+        _check(self.lib, self.lib.cg_process_device(self.h, C.byref(db), out.data_ptr() or None, C.byref(res)), self.h)
+        if res.n_events > events_cap or (want_columns and res.n_columns > res.columns_cap):
+            # still on the device: fetch again with room for everything; the call is not repeated (it may have rewritten in place)
+            if res.n_events > events_cap:
+                events_cap = self._events_hint = int(res.n_events)
+                ev = np.zeros(events_cap, dtype=EVENT_DTYPE)
+            res2 = Result(events=ev.ctypes.data_as(C.POINTER(BedEvent)), events_cap=events_cap)
+            if want_columns:
+                if res.n_columns > res.columns_cap:
+                    self._ncols_hint = int(res.n_columns)
+                    cols = np.zeros(self._ncols_hint, dtype=COLUMN_DTYPE)
+                res2.columns, res2.columns_cap = cols.ctypes.data_as(C.POINTER(Column)), len(cols)
+            _check(self.lib, self.lib.cg_download(self.h, C.byref(res2)), self.h)
+            res = res2
+        r = {"qual": out, "events": ev[: int(res.n_events)], "counters": {k: int(res.counters[i]) for i, k in enumerate(COUNTER_NAMES)}}
+        if want_columns:
+            r["columns"] = cols[: int(res.n_columns)]
+        return r
 
     def process_window(self, batch: Batch, window: Window, events_cap: int = 1 << 16, pinned_out=None):
         """One call of a chain (cg_process_window): ``batch`` = read halo + new records, ``window`` = the columns it owns.
@@ -551,6 +632,55 @@ def sub_batch(batch: Batch, i0: int, i1: int):
             for k in range(16):
                 b.qual_dict[k] = batch.qual_dict[k]
     return b, tuple(keep)
+
+
+def _torch_dtype(np_dtype):
+    import torch
+    return {np.int32: torch.int32, np.uint16: torch.uint16, np.uint8: torch.uint8, np.uint32: torch.uint32}[np_dtype]
+
+
+def _strip(buf: np.ndarray, off: np.ndarray, ln: np.ndarray, unit: int, packed: bool) -> np.ndarray:
+    """bytes [off[i], off[i] + ln[i]) of every record, back to back.  A packed batch lays records out in whole rows of `unit` bytes with
+    the padding at the end of each record's last row: a row mask strips it without an index per byte."""
+    total = int(ln.sum())
+    if total == 0:
+        return buf[:0].copy()
+    if packed and buf.size % unit == 0:
+        rows = (ln + unit - 1) // unit
+        keep = np.full(buf.size // unit, unit, np.uint8)
+        has = rows > 0
+        keep[(off[has] // unit + rows[has] - 1)] = (ln[has] - unit * (rows[has] - 1)).astype(np.uint8)
+        return buf.reshape(-1, unit)[np.arange(unit, dtype=np.uint8)[None, :] < keep[:, None]]
+    start = np.cumsum(ln) - ln
+    return buf[np.arange(total, dtype=np.int64) + np.repeat(off - start, ln)]
+
+
+def concat_fields(batch: Batch) -> dict:
+    """A host Batch (from BatchBuilder) as the concatenated BAM fields of cg_dev_batch, in numpy: the per-record arrays as they are,
+    the CIGARs, sequences (ceil(l/2) bytes) and qualities (l bytes) of the records back to back without the batcher's padding."""
+    n = int(batch.n_reads)
+
+    def arr(ptr, dtype, count):
+        return np.ctypeslib.as_array(ptr, shape=(count,)).astype(dtype, copy=True) if count else np.zeros(0, dtype)
+    f = {k: arr(getattr(batch, k), DEV_FIELDS[k], n) for k in DEV_PER_RECORD}
+    ln = f["l_qseq"].astype(np.int64)
+    off = arr(batch.off, np.int64, n)
+    packed = batch.packed == 1
+    cig = arr(batch.cigar, np.uint32, int(batch.n_cigar_total))
+    f["cigar"] = _strip(cig, arr(batch.cigar_off, np.int64, n), f["n_cigar"].astype(np.int64), 1, False) if not packed else cig
+    f["seq"] = _strip(np.ctypeslib.as_array(batch.seq, shape=(int(batch.seq_bytes),)) if batch.seq_bytes else np.zeros(0, np.uint8),
+                      off // 2, (ln + 1) // 2, 4, packed)
+    f["qual"] = _strip(np.ctypeslib.as_array(batch.qual, shape=(int(batch.qual_bytes),)) if batch.qual_bytes else np.zeros(0, np.uint8),
+                       off, ln, 8, packed)
+    return f
+
+
+def device_batch(batch: Batch, device) -> dict:
+    """The records of a host Batch as torch tensors on `device` (an index or a torch.device) in the layout ``Crumble.process_device``
+    takes: what a GPU-side BAM decoder would hand over."""
+    import torch
+    dev = torch.device("cuda", device) if isinstance(device, int) else torch.device(device)
+    return {k: torch.from_numpy(v).to(dev) for k, v in concat_fields(batch).items()}
 
 
 def plan_region_shards(batch: Batch, n_shards: int):

@@ -69,14 +69,6 @@ CG_HD uint32_t cg_bases8(uint32_t X) {
     return ((p1 + p2 * 2u + p3 * 3u) & m) | (0x55555555u & ~m);
 }
 
-CG_HD uint32_t cg_funnel_r(uint32_t lo, uint32_t hi, unsigned sh) {    /* sh in 0..31 */
-#ifdef __CUDA_ARCH__
-    return __funnelshift_r(lo, hi, sh);
-#else
-    return sh ? (lo >> sh) | (hi << (32 - sh)) : lo;
-#endif
-}
-
 /* the eight cells of group k of a SIMPLE read (single M/=/X op, l_qseq == span: query offset == column offset), as four 32-bit words
  * of two cells each.  d_first = 8k - (col0 & 7) is the offset inside the read of the group's first cell (negative in the first
  * group of a read that does not start on a group boundary).  Two aligned 64-bit quality loads and two 32-bit sequence loads are

@@ -1327,6 +1327,7 @@ struct cg_ctx {
     dbuf b_tlo, b_tstart, b_isl, b_cb, b_ev, b_depth, b_dump, b_dsum, b_csum, b_fcol, b_trig, b_twin;
     dbuf b_aggr, b_scal, b_scratch, b_epoch, b_events, b_chain, b_items, b_bed, b_bedpm, b_crec, b_cells, b_seq2, b_qualp, b_exc;
     dbuf b_truns, b_pabs, b_pd8, b_lq8, b_nc8, b_cigx, b_lqd, b_xoff, b_absS;   /* compact planes of the per-record arrays and what their expansion needs */
+    dbuf b_qsrc, b_ssrc, b_dvsum;  /* cg_process_device: where each record starts in the caller's arrays, the sums checked on the host */
     int has_meta; int64_t n_truns, n_pabs, n_cigx;
     int generic;                  /* cg_params_generic(): column and rewrite stages through the plain bodies */
     /* host mirrors */
@@ -1453,7 +1454,8 @@ extern "C" void cg_destroy(cg_ctx *ctx) {
         &ctx->b_seq, &ctx->b_qual, &ctx->b_qout, &ctx->b_jmap, &ctx->b_rspan, &ctx->b_rd, &ctx->b_ks, &ctx->b_ke, &ctx->b_gap, &ctx->b_gapraw,
         &ctx->b_pmax, &ctx->b_orig, &ctx->b_rbf, &ctx->b_glist, &ctx->b_tlo, &ctx->b_tstart, &ctx->b_isl, &ctx->b_cb, &ctx->b_ev, &ctx->b_depth, &ctx->b_dump,
         &ctx->b_dsum, &ctx->b_csum, &ctx->b_fcol, &ctx->b_trig, &ctx->b_twin, &ctx->b_aggr, &ctx->b_scal, &ctx->b_scratch, &ctx->b_epoch, &ctx->b_events, &ctx->b_chain, &ctx->b_items, &ctx->b_bed, &ctx->b_bedpm, &ctx->b_saved, &ctx->b_crec, &ctx->b_cells, &ctx->b_seq2, &ctx->b_qualp, &ctx->b_exc, &ctx->b_cqmask, &ctx->b_cqexc, &ctx->b_cqblk,
-        &ctx->b_truns, &ctx->b_pabs, &ctx->b_pd8, &ctx->b_lq8, &ctx->b_nc8, &ctx->b_cigx, &ctx->b_lqd, &ctx->b_xoff, &ctx->b_absS };
+        &ctx->b_truns, &ctx->b_pabs, &ctx->b_pd8, &ctx->b_lq8, &ctx->b_nc8, &ctx->b_cigx, &ctx->b_lqd, &ctx->b_xoff, &ctx->b_absS,
+        &ctx->b_qsrc, &ctx->b_ssrc, &ctx->b_dvsum };
     for (size_t i = 0; i < sizeof(all) / sizeof(all[0]); i++) if (all[i]->p) cudaFree(all[i]->p);
     if (ctx->dT) cudaFree(ctx->dT);
     if (ctx->h_dims) cudaFreeHost(ctx->h_dims);
@@ -2068,6 +2070,125 @@ extern "C" int cg_download(cg_ctx *ctx, cg_result *out) {
     float ms = 0;
     if (cudaEventElapsedTime(&ms, ctx->ev[CG_T_D2H][0], ctx->ev[CG_T_D2H][1]) == cudaSuccess) ctx->ms[CG_T_D2H] = ms; else cudaGetLastError();
     if (cudaEventElapsedTime(&ms, ctx->ev[CG_T_H2D][0], ctx->ev[CG_T_H2D][1]) == cudaSuccess) ctx->ms[CG_T_H2D] = ms; else cudaGetLastError();
+    return 0;
+}
+
+/* ---- records already in GPU memory (cg_process_device) ---------------------------------------------------------------------------
+ * The per-record arrays and the CIGARs are copied device to device into the working buffers (so the caller's buffers are free once
+ * the stream has passed the call) and the batch is treated as packed: the scans cg_run would run rebuild off[] and cigar_off[] here,
+ * two more give where every record starts in the caller's arrays, and all sums are checked at one host synchronisation before any
+ * kernel uses an offset.  k_ingest repacks qualities and sequences into the padded working layout, the resident chain runs as in
+ * cg_run, and k_emit gathers the rewritten qualities into the caller's concatenated layout.  One warp per record; the per-item
+ * bodies (cg_pipeline.h) are the emulation's. */
+#define IO_THREADS 256
+__global__ void __launch_bounds__(IO_THREADS) k_ingest(const __grid_constant__ CgIngest I, int64_t n) {
+    const int64_t r = ((int64_t)blockIdx.x * IO_THREADS + threadIdx.x) >> 5;
+    if (r >= n) return;
+    const int ng = (I.l_qseq[r] + 7) >> 3;
+    for (int k = threadIdx.x & 31; k < ng; k += 32) cg_ingest_group(&I, r, k);
+}
+__global__ void __launch_bounds__(IO_THREADS) k_emit(const __grid_constant__ CgEmit E, int64_t n) {
+    const int64_t r = ((int64_t)blockIdx.x * IO_THREADS + threadIdx.x) >> 5;
+    if (r >= n) return;
+    const int nw = cg_emit_words(&E, r);
+    for (int j = threadIdx.x & 31; j < nw; j += 32) cg_emit_word(&E, r, j);
+}
+struct LdLen { const int32_t *lq; __device__ int64_t operator()(int64_t i) const { return (int64_t)lq[i]; } };
+struct LdHalf { const int32_t *lq; __device__ int64_t operator()(int64_t i) const { return ((int64_t)lq[i] + 1) >> 1; } };
+struct LdNeg { const int32_t *lq; __device__ int64_t operator()(int64_t i) const { return lq[i] < 0 ? 1 : 0; } };
+struct LdNCig64 { const uint16_t *nc; __device__ int64_t operator()(int64_t i) const { return (int64_t)nc[i]; } };
+struct StExcl32of64 { int32_t *p; __device__ void operator()(int64_t i, int64_t, int64_t ex) const { p[i] = (int32_t)ex; } };
+struct StNone { __device__ void operator()(int64_t, int64_t, int64_t) const {} };
+
+static int dev_ptr_check(cg_ctx *ctx, const void *p, int64_t count, const char *name) {
+    if (count == 0) return 0;
+    cudaPointerAttributes a;
+    if (p && cudaPointerGetAttributes(&a, p) == cudaSuccess && a.type == cudaMemoryTypeDevice && a.device == ctx->device) return 0;
+    cudaGetLastError();
+    snprintf(ctx->err, sizeof ctx->err, "cg_dev_batch: %s is not device memory of device %d", name, ctx->device);
+    return CG_ERR_BAD_ARG;
+}
+
+extern "C" int cg_process_device(cg_ctx *ctx, const cg_dev_batch *in, uint8_t *qual_out, cg_result *out) {
+    if (!ctx) return CG_ERR_BAD_ARG;
+    if (!in || !out) { snprintf(ctx->err, sizeof ctx->err, "cg_process_device: no batch or no result"); return CG_ERR_BAD_ARG; }
+    CG_CHECK(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    const int64_t n = in->n_reads;
+    int e;
+    if (n < 0 || in->n_cigar_total < 0 || in->seq_len < 0 || in->qual_len < 0) {
+        snprintf(ctx->err, sizeof ctx->err, "cg_dev_batch: negative count (n_reads %lld, n_cigar_total %lld, seq_len %lld, qual_len %lld)",
+                 (long long)n, (long long)in->n_cigar_total, (long long)in->seq_len, (long long)in->qual_len);
+        return CG_ERR_BAD_ARG;
+    }
+    if (out->qual_out || out->qual_head) { snprintf(ctx->err, sizeof ctx->err, "cg_process_device: the qualities go to qual_out; out->qual_out and out->qual_head must be NULL"); return CG_ERR_BAD_ARG; }
+    if (n > 0x7fffff00LL || in->n_cigar_total > 0x7fffff00LL || in->qual_len + 8 * n >= (1LL << 35)) { snprintf(ctx->err, sizeof ctx->err, "batch too large: split it"); return CG_ERR_BAD_ARG; }
+    if ((e = dev_ptr_check(ctx, in->tid, n, "tid")) || (e = dev_ptr_check(ctx, in->pos, n, "pos")) || (e = dev_ptr_check(ctx, in->flag, n, "flag")) ||
+        (e = dev_ptr_check(ctx, in->mapq, n, "mapq")) || (e = dev_ptr_check(ctx, in->l_qseq, n, "l_qseq")) || (e = dev_ptr_check(ctx, in->n_cigar, n, "n_cigar")) ||
+        (e = dev_ptr_check(ctx, in->cigar, in->n_cigar_total, "cigar")) || (e = dev_ptr_check(ctx, in->seq, in->seq_len, "seq")) ||
+        (e = dev_ptr_check(ctx, in->qual, in->qual_len, "qual")) || (e = dev_ptr_check(ctx, qual_out, in->qual_len, "qual_out"))) return e;
+    ctx->resident = 0; ctx->win_on = 0; ctx->cq_on = 0;
+    ctx->dump_columns = out->columns != NULL;
+    /* working buffers sized for the padded layout: the padded lengths sum to at most qual_len + 7 per record */
+    cg_batch hb; memset(&hb, 0, sizeof hb);
+    hb.n_reads = n; hb.n_cigar_total = in->n_cigar_total; hb.qual_bytes = in->qual_len + 7 * n; hb.seq_bytes = (hb.qual_bytes + 1) / 2; hb.packed = 1;
+    if ((e = alloc_inputs(ctx, &hb))) return e;
+    if ((e = ensure(ctx, &ctx->b_qsrc, ((size_t)n + 1) * 8)) || (e = ensure(ctx, &ctx->b_ssrc, ((size_t)n + 1) * 8)) || (e = ensure(ctx, &ctx->b_dvsum, 64))) return e;
+    CgDev *D = &ctx->D;
+    int64_t padded = 0;
+    if (n > 0) {
+        CG_CHECK(cudaMemcpyAsync(ctx->b_tid.p, in->tid, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
+        CG_CHECK(cudaMemcpyAsync(ctx->b_pos.p, in->pos, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
+        CG_CHECK(cudaMemcpyAsync(ctx->b_flag.p, in->flag, (size_t)n * 2, cudaMemcpyDeviceToDevice, st));
+        CG_CHECK(cudaMemcpyAsync(ctx->b_mapq.p, in->mapq, (size_t)n, cudaMemcpyDeviceToDevice, st));
+        CG_CHECK(cudaMemcpyAsync(ctx->b_lq.p, in->l_qseq, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
+        CG_CHECK(cudaMemcpyAsync(ctx->b_nc.p, in->n_cigar, (size_t)n * 2, cudaMemcpyDeviceToDevice, st));
+        if (in->n_cigar_total) CG_CHECK(cudaMemcpyAsync(ctx->b_cigar.p, in->cigar, (size_t)in->n_cigar_total * 4, cudaMemcpyDeviceToDevice, st));
+        int64_t *sums = (int64_t *)ctx->b_dvsum.p;               /* [0] padded lengths [1] n_cigar [2] l_qseq [3] (l_qseq + 1) / 2 [4] negative l_qseq */
+        LdPad8 lp = { D->l_qseq }; StExcl64 so = { (int64_t *)ctx->b_off.p };
+        LdNCig64 ln = { D->n_cigar }; StExcl32of64 sc = { (int32_t *)ctx->b_coff.p };
+        LdLen ll = { D->l_qseq }; StExcl64 sq = { (int64_t *)ctx->b_qsrc.p };
+        LdHalf lh = { D->l_qseq }; StExcl64 ss = { (int64_t *)ctx->b_ssrc.p };
+        LdNeg lneg = { D->l_qseq }; StNone none;
+        if ((e = run_scan<int64_t, OpSum>(ctx, lp, so, n, (int64_t)0, sums + 0)) || (e = run_scan<int64_t, OpSum>(ctx, ln, sc, n, (int64_t)0, sums + 1)) ||
+            (e = run_scan<int64_t, OpSum>(ctx, ll, sq, n, (int64_t)0, sums + 2)) || (e = run_scan<int64_t, OpSum>(ctx, lh, ss, n, (int64_t)0, sums + 3)) ||
+            (e = run_scan<int64_t, OpSum>(ctx, lneg, none, n, (int64_t)0, sums + 4))) return e;
+        int64_t h[5];
+        CG_CHECK(cudaMemcpyAsync(h, sums, sizeof h, cudaMemcpyDeviceToHost, st));
+        CG_CHECK(cudaStreamSynchronize(st));
+        if (h[4]) { snprintf(ctx->err, sizeof ctx->err, "cg_dev_batch: %lld records have a negative l_qseq", (long long)h[4]); return CG_ERR_BAD_ARG; }
+        if (h[2] != in->qual_len || h[3] != in->seq_len || h[1] != in->n_cigar_total) {
+            snprintf(ctx->err, sizeof ctx->err, "cg_dev_batch: the records hold %lld quality bytes (qual_len %lld), %lld sequence bytes (seq_len %lld), %lld CIGAR operations (n_cigar_total %lld)",
+                     (long long)h[2], (long long)in->qual_len, (long long)h[3], (long long)in->seq_len, (long long)h[1], (long long)in->n_cigar_total);
+            return CG_ERR_BAD_ARG;
+        }
+        padded = h[0];
+    }
+    ctx->qual_bytes = padded; ctx->offsets_ready = 1;
+    const unsigned io_blocks = (unsigned)nblk(n * 32, IO_THREADS);
+    T0(CG_T_H2D);
+    if (n > 0) {
+        const CgIngest I = { D->l_qseq, D->off, (const int64_t *)ctx->b_qsrc.p, (const int64_t *)ctx->b_ssrc.p, in->qual, in->seq,
+                             (uint8_t *)ctx->b_qual.p + CG_FRONT_PAD, (uint8_t *)ctx->b_seq.p + CG_FRONT_PAD };
+        k_ingest<<<io_blocks, IO_THREADS, 0, st>>>(I, n);
+        CG_CHECK(cudaGetLastError());
+    }
+    T1(CG_T_H2D);
+    ctx->resident = 1;
+    if ((e = cg_run(ctx))) return e;
+    T0(CG_T_D2H);
+    if (n > 0 && in->qual_len > 0) {
+        const CgEmit E = { D->l_qseq, D->off, (const int64_t *)ctx->b_qsrc.p, (const uint8_t *)ctx->b_qout.p, qual_out };
+        k_emit<<<io_blocks, IO_THREADS, 0, st>>>(E, n);
+        ctx->launches++;
+        CG_CHECK(cudaGetLastError());
+    }
+    T1(CG_T_D2H);
+    if ((e = download_results(ctx, out, 0))) return e;          /* events, counters, column dump; synchronises the stream */
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, ctx->ev[CG_T_H2D][0], ctx->ev[CG_T_H2D][1]) == cudaSuccess) ctx->ms[CG_T_H2D] = ms; else cudaGetLastError();
+    if (cudaEventElapsedTime(&ms, ctx->ev[CG_T_D2H][0], ctx->ev[CG_T_D2H][1]) == cudaSuccess) ctx->ms[CG_T_D2H] = ms; else cudaGetLastError();
+    ctx->h2d_bytes = 0;
     return 0;
 }
 

@@ -15,6 +15,7 @@
 #ifndef CG_PIPELINE_H
 #define CG_PIPELINE_H
 
+#include <string.h>
 #include "cg_core.h"
 #include "../../include/crumble_gpu.h"
 
@@ -656,6 +657,97 @@ CG_HD uint32_t cg_deep_test(const CgDev *D, int c, int64_t tdepth, int64_t tcol)
         return (ev & CG_EV_REPLAY) ? 0 : 1u << CG_CNT_OVER_DEPTH;
     }
     return 0;
+}
+
+/* ---- stages: ingest / emit (cg_process_device) -------------------------------------------
+ * Records in GPU memory arrive as "concatenated BAM fields" (cg_dev_batch): qualities and sequences back to back at any byte
+ * offset.  ingest moves them into the padded working layout the chain reads (qual at off[r], seq at off[r] / 2, off 8-aligned),
+ * emit moves the rewritten qualities back.  Every access on the working side is an aligned 8- or 4-byte word; the caller's side
+ * is read as whole aligned 32-bit words joined by funnel shifts, and only words holding at least one byte of the record are read. */
+CG_HD uint32_t cg_ld_word(const uint8_t *aligned) {
+#ifdef __CUDA_ARCH__
+    return *(const uint32_t *)aligned;
+#else
+    uint32_t v; memcpy(&v, aligned, 4); return v;
+#endif
+}
+CG_HD void cg_st_word(uint8_t *aligned, uint32_t v) {
+#ifdef __CUDA_ARCH__
+    *(uint32_t *)aligned = v;
+#else
+    memcpy(aligned, &v, 4);
+#endif
+}
+CG_HD void cg_st_dword(uint8_t *aligned, uint64_t v) {
+#ifdef __CUDA_ARCH__
+    *(uint64_t *)aligned = v;
+#else
+    memcpy(aligned, &v, 8);
+#endif
+}
+CG_HD uint32_t cg_funnel_r(uint32_t lo, uint32_t hi, unsigned sh) {    /* sh in 0..31 (also used by cg_cells.h) */
+#ifdef __CUDA_ARCH__
+    return __funnelshift_r(lo, hi, sh);
+#else
+    return sh ? (lo >> sh) | (hi << (32 - sh)) : lo;
+#endif
+}
+/* bytes [p, p + n), 1 <= n <= 8, as a little-endian word, zero above byte n: the (at most three) aligned words that hold them */
+CG_HD uint64_t cg_gather8(const uint8_t *p, int n) {
+    const uintptr_t a = (uintptr_t)p & ~(uintptr_t)3, end = (uintptr_t)p + (uintptr_t)n;
+    const uint32_t sh = ((uint32_t)(uintptr_t)p & 3u) * 8u;
+    const uint8_t *w = (const uint8_t *)a;
+    const uint32_t w0 = cg_ld_word(w), w1 = a + 4 < end ? cg_ld_word(w + 4) : 0u, w2 = a + 8 < end ? cg_ld_word(w + 8) : 0u;
+    const uint64_t v = (uint64_t)cg_funnel_r(w0, w1, sh) | ((uint64_t)cg_funnel_r(w1, w2, sh) << 32);
+    return n >= 8 ? v : v & ((1ull << (8 * n)) - 1);
+}
+
+typedef struct CgIngest {
+    const int32_t *l_qseq; const int64_t *off;       /* working layout: off[] = running sum of (l_qseq + 7) & ~7 */
+    const int64_t *qsrc, *ssrc;                      /* running sums of l_qseq and (l_qseq + 1) / 2: record r in the caller's arrays */
+    const uint8_t *qual_in, *seq_in;                 /* the caller's concatenated arrays */
+    uint8_t *qual, *seq;                             /* working arrays (past their front padding) */
+} CgIngest;
+
+/* ingest, one item per (record r, group k < (l_qseq + 7) / 8): working qual bytes [off + 8k, off + 8k + 8) and seq bytes
+ * [off/2 + 4k, off/2 + 4k + 4).  Bytes past the record are zero, as the host batcher leaves its padding (cg_host.cpp, cgb_add);
+ * the record's last seq byte is copied whole, so an odd-length record keeps its phantom low nibble (SURVEY §9.3). */
+CG_HD void cg_ingest_group(const CgIngest *I, int64_t r, int k) {
+    const int L = I->l_qseq[r];
+    const int64_t o = I->off[r];
+    const int nq = L - 8 * k;
+    uint64_t q = 0; uint32_t s = 0;
+    if (nq > 0) {
+        const int ns = ((L + 1) >> 1) - 4 * k;                                  /* > 0 whenever nq > 0 */
+        q = cg_gather8(I->qual_in + I->qsrc[r] + 8 * k, nq < 8 ? nq : 8);
+        s = (uint32_t)cg_gather8(I->seq_in + I->ssrc[r] + 4 * k, ns < 4 ? ns : 4);
+    }
+    cg_st_dword(I->qual + o + 8 * k, q);
+    cg_st_word(I->seq + (o >> 1) + 4 * k, s);
+}
+
+typedef struct CgEmit {
+    const int32_t *l_qseq; const int64_t *off, *qdst;   /* qdst = qsrc of CgIngest: the concatenated layout */
+    const uint8_t *qout;                               /* rewritten qualities, working layout */
+    uint8_t *qual_out;                                 /* the caller's concatenated array */
+} CgEmit;
+
+/* emit, one item per (record r, j < cg_emit_words): the 8-byte aligned words of the caller's array that hold bytes of record r.
+ * A word wholly inside the record takes one aligned store; the first and last word, shared with the neighbours, take byte stores. */
+CG_HD int cg_emit_words(const CgEmit *E, int64_t r) {
+    const int L = E->l_qseq[r];
+    if (L <= 0) return 0;
+    const uintptr_t d0 = (uintptr_t)(E->qual_out + E->qdst[r]);
+    return (int)(((d0 + (uintptr_t)L - 1) >> 3) - (d0 >> 3) + 1);
+}
+CG_HD void cg_emit_word(const CgEmit *E, int64_t r, int j) {
+    const int64_t L = E->l_qseq[r];
+    uint8_t *dst = E->qual_out + E->qdst[r];
+    const int64_t x = -(int64_t)((uintptr_t)dst & 7) + 8 * (int64_t)j;        /* record byte at the word's first address */
+    const int64_t x0 = x > 0 ? x : 0, x1 = x + 8 < L ? x + 8 : L;
+    const uint64_t v = cg_gather8(E->qout + E->off[r] + x0, (int)(x1 - x0));
+    if (x0 == x && x1 == x + 8) cg_st_dword(dst + x, v);
+    else for (int64_t b = x0; b < x1; b++) dst[b] = (uint8_t)(v >> (8 * (b - x0)));
 }
 
 #endif /* CG_PIPELINE_H */

@@ -192,6 +192,29 @@ int cg_sync(cg_ctx *ctx);
  * slice i of the kernel chain starts when chunk i has landed.  Results do not depend on it. */
 int cg_set_chunk_bytes(cg_ctx *ctx, int64_t bytes);
 
+/* ---- records already in GPU memory: "concatenated BAM fields" ----------------------------
+ * What a GPU BAM decoder or a torch pipeline naturally holds; no offset arrays.  Every pointer is device memory of the
+ * context's device (NULL is allowed where its count is 0).  Records in input (coordinate-sorted) order, types as cg_batch. */
+typedef struct cg_dev_batch {
+    int64_t n_reads;
+    const int32_t  *tid, *pos;  const uint16_t *flag;  const uint8_t *mapq;
+    const int32_t  *l_qseq;     const uint16_t *n_cigar;
+    const uint32_t *cigar;  int64_t n_cigar_total;  /* records' CIGARs back to back */
+    const uint8_t  *seq;    int64_t seq_len;        /* record i: (l_qseq[i]+1)/2 bytes, BAM nibble order, back to back, each record starts on a byte */
+    const uint8_t  *qual;   int64_t qual_len;       /* record i: l_qseq[i] bytes, back to back; qual_len = sum of l_qseq */
+} cg_dev_batch;
+
+/* qual_out: device, qual_len bytes, same concatenated layout; may equal in->qual (rewrite in place).
+ * out: events, counters and the optional column dump, exactly as for cg_process; out->qual_out and out->qual_head must be NULL.
+ * Runs on the context's stream (cg_set_stream).  The three sums (qual_len, seq_len, n_cigar_total) are checked on the device
+ * before anything uses them: CG_ERR_BAD_ARG when they disagree, when a count is negative or when a pointer is not device memory
+ * of the context's device.  On return the counters and events are on the host; qual_out is written in stream order, so work
+ * queued later on the same stream sees it.  The caller's input buffers are free once the stream has passed the call.
+ * Afterwards the batch is resident as after cg_upload + cg_run: cg_run may time the chain on it again, and cg_download
+ * (qual_out = NULL) re-fetches a longer event list.  cg_last_ms(CG_T_H2D / CG_T_D2H) time the ingest and emit kernels,
+ * and cg_last_h2d_bytes reads 0. */
+int cg_process_device(cg_ctx *ctx, const cg_dev_batch *in, uint8_t *qual_out, cg_result *out);
+
 /* ---- chained calls: a coordinate-sorted stream of any length in bounded memory ------------
  * (region shards with a read halo, SURVEY.md §8(e): the reference keeps its state in a streaming loop, snp_score.c:1437-1975)
  * The caller cuts the stream wherever it likes.  Let X be the position of the first record AFTER call k (same contig),
