@@ -17,8 +17,6 @@
 #include <stdlib.h>
 #include <string.h>
 #include <time.h>
-#include <pthread.h>
-#include <unistd.h>
 #include "cg_host.h"
 #include "cg_column_lean.h"
 
@@ -216,15 +214,15 @@ __global__ void k_gap(const __grid_constant__ CgDev D, const int32_t *n_pile, in
     int j = blockIdx.x * blockDim.x + threadIdx.x;
     if (j < *n_pile) gapraw[j] = cg_gap_of(&D, j);
 }
-__global__ void k_finish_read(const __grid_constant__ CgDev D, const int32_t *n_pile, int32_t *dims) {
+__global__ void k_finish_read(const __grid_constant__ CgDev D, const int32_t *n_pile, int32_t *n_cols) {
     int j = blockIdx.x * blockDim.x + threadIdx.x;
     int np = *n_pile;
     if (j < np) {
         cg_finish_read(&D, j, D.ks[0]);
-        if (j == np - 1) dims[1] = D.pmaxcol[j];     /* n_cols */
+        if (j == np - 1) *n_cols = D.pmaxcol[j];
         if (D.glist && !(D.rd[j].rf & CG_RF_SIMPLE)) D.glist[atomicAdd(D.n_glist, 1)] = j;   /* k_cells_general's work list */
     }
-    if (j == 0 && np == 0) dims[1] = 0;
+    if (j == 0 && np == 0) *n_cols = 0;
 }
 /* device scalars -> MAPPED pinned host memory, written by the SMs: a cudaMemcpy would queue behind the bulk quality
  * downloads on the D2H copy engine and stall the host's per-slice sync by a whole chunk */
@@ -928,32 +926,7 @@ __device__ __forceinline__ void rw_mbar_wait(unsigned long long *bar, uint32_t p
     if (!ok) __trap();
 }
 
-/* the compact output of one record (thread per record): mask bytes of its words into mk[], returns the number of exception bytes */
-__device__ __forceinline__ int rw_compact_count(const uint8_t *q, int L, uint32_t dom, uint8_t *mk) {
-    const uint64_t D8 = (uint64_t)dom * 0x0101010101010101ULL;
-    int cnt = 0;
-    for (int w = 0; 8 * w < L; w++) {
-        const uint64_t x = *reinterpret_cast<const uint64_t *>(q + 8 * w) ^ D8;          /* zero bytes where equal */
-        const uint64_t nz = ((x & 0x7f7f7f7f7f7f7f7fULL) + 0x7f7f7f7f7f7f7f7fULL) | x;  /* bit 7 of every non-zero byte */
-        uint32_t m8 = 0;
-#pragma unroll
-        for (int k = 0; k < 8; k++) m8 |= (uint32_t)((~nz >> (8 * k + 7)) & 1ULL) << k;
-        const int rem = L - 8 * w;
-        if (rem < 8) m8 |= 0xffu << rem;                                                 /* padding: "equal" */
-        m8 &= 0xffu;
-        mk[w] = (uint8_t)m8;
-        cnt += 8 - __popc(m8);
-    }
-    return cnt;
-}
-__device__ __forceinline__ void rw_compact_emit(const uint8_t *q, int L, const uint8_t *mk, uint8_t *dst) {
-    for (int w = 0; 8 * w < L; w++) {
-        uint32_t x = (~(uint32_t)mk[w]) & 0xffu;
-        while (x) { const int k = __ffs(x) - 1; x &= x - 1; *dst++ = q[8 * w + k]; }
-    }
-}
-
-__global__ void __launch_bounds__(RW_THREADS) k_rewrite(const __grid_constant__ CgDev D, int64_t rec_begin, int64_t rec_end, int64_t blk_base) {
+__global__ void __launch_bounds__(RW_THREADS) k_rewrite(const __grid_constant__ CgDev D, int64_t rec_begin, int64_t rec_end) {
     __shared__ RwSmem S;
     const CgDevParams *P = &D.P;
     const CgTables *T = D.T;
@@ -1011,26 +984,10 @@ __global__ void __launch_bounds__(RW_THREADS) k_rewrite(const __grid_constant__ 
     }
     __syncthreads();
     const long long qa = S.rng[0], qbytes = S.rng[1], ca = S.rng[4], cbytes = S.rng[5];
-    if (qbytes == 0) { if (D.cq_mask && threadIdx.x == 0) D.cq_blk[blk_base + blockIdx.x] = 0; return; }   /* nothing but empty records */
+    if (qbytes == 0) return;                                   /* nothing but empty records */
     if (cbytes < 0) {                                          /* ranges too long for the staging buffers */
         const int64_t r = base + threadIdx.x;
         if (r < rec_end) cg_rewrite(&D, r, nf);
-        if (D.cq_mask) {                                       /* compact form straight from the flat output (each record's words are its own) */
-            __shared__ int cnts[RW_THREADS];
-            __shared__ unsigned long long fb_base;
-            int cnt = 0;
-            if (r < rec_end && L > 0) cnt = rw_compact_count(D.qual_out + off, L, (uint32_t)D.cq_dom, D.cq_mask + (off >> 3));
-            cnts[threadIdx.x] = cnt;
-            __syncthreads();
-            if (threadIdx.x == 0) {
-                unsigned long long tot = 0;
-                for (int i = 0; i < RW_THREADS; i++) { const int c = cnts[i]; cnts[i] = (int)tot; tot += (unsigned long long)c; }
-                fb_base = atomicAdd(D.cq_count, tot);
-                D.cq_blk[blk_base + blockIdx.x] = (int64_t)fb_base;
-            }
-            __syncthreads();
-            if (cnt) rw_compact_emit(D.qual_out + off, L, D.cq_mask + (off >> 3), D.cq_exc + fb_base + (unsigned)cnts[threadIdx.x]);
-        }
         return;
     }
     const int nwords = (int)(qbytes >> 3);
@@ -1199,34 +1156,6 @@ __global__ void __launch_bounds__(RW_THREADS) k_rewrite(const __grid_constant__ 
             else rw_pblock_rle(S.q + m.qoff, S.wmap + (m.qoff >> 3), (int)(m.lk & RW_L_M), P->pblock, P->qcap);
         }
     }
-    /* ---- phase C': compact output (mask + exceptions) instead of the flat range ---- */
-    if (D.cq_mask) {
-        __syncthreads();
-        for (int i = threadIdx.x; i < (nwords + 3) >> 2; i += RW_THREADS) reinterpret_cast<uint32_t *>(S.wmap)[i] = 0xffffffffu;   /* words of no record: all "equal" */
-        __syncthreads();
-        const RwMeta m = S.m[threadIdx.x];
-        const int Lm = ((m.lk >> RW_KIND_SH) & 3u) ? (int)(m.lk & RW_L_M) : 0;
-        const int cnt = Lm ? rw_compact_count(S.q + m.qoff, Lm, (uint32_t)D.cq_dom, S.wmap + (m.qoff >> 3)) : 0;
-        /* exclusive prefix of the counts over the block's records */
-        int inc = cnt;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) { const int u = __shfl_up_sync(0xffffffffu, inc, o); if (lane >= o) inc += u; }
-        if (lane == 31) S.red[w][3] = inc;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            long long tot = 0;
-            for (int i = 0; i < RW_THREADS / 32; i++) { const long long c = S.red[i][3]; S.red[i][3] = tot; tot += c; }
-            const unsigned long long b0 = atomicAdd(D.cq_count, (unsigned long long)tot);
-            S.red[0][2] = (long long)b0;
-            D.cq_blk[blk_base + blockIdx.x] = (int64_t)b0;
-        }
-        __syncthreads();
-        if (cnt) rw_compact_emit(S.q + m.qoff, Lm, S.wmap + (m.qoff >> 3), D.cq_exc + S.red[0][2] + S.red[w][3] + (inc - cnt));
-        /* the mask bytes of the block's own words [lo, hi8) */
-        const long long lo = S.red[0][0], hi8 = (S.red[0][1] + 7) & ~7LL;
-        for (long long i = ((lo - qa) >> 3) + threadIdx.x; i < ((hi8 - qa) >> 3); i += RW_THREADS) D.cq_mask[(qa >> 3) + i] = S.wmap[i];
-        return;
-    }
     /* ---- phase C: the block's output range ---- */
     asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");
     __syncthreads();
@@ -1315,7 +1244,56 @@ struct dbuf { void *p; size_t cap; };
 
 #define CG_MAX_CHUNKS 32
 struct CgBounds { int64_t rb[CG_MAX_CHUNKS]; int32_t n; };
-struct CgSlice { int t0, t1, c0, c1, jb, je, kb, ke, chunk, save_after, synced; int64_t r0, r1; };   /* see slice_A / slice_B */
+struct CgSlice { int t0, t1, c0, c1, jb, je, kb, ke, chunk, save_after; int64_t r0, r1; };   /* see slice_A / slice_B */
+
+/* The device scalar block (b_scal): the chain's scalars and counters, both carries, the chunk bounds and a scratch carry; run_prep
+ * zeroes it.  Its head is mirrored into mapped pinned memory (cg_ctx::h_dims), copied there at the host's synchronisations or written
+ * there directly by k_publish and k_find_col.  Every field keeps a fixed byte offset, checked below. */
+struct CgScalHead {
+    int32_t n_pile;               /* pileup reads */
+    int32_t n_cols;
+    int32_t n_islands;
+    int32_t n_flagged;            /* of the slice */
+    int32_t maxdepth;
+    int32_t err;                  /* device-side error code */
+    int32_t n_events;             /* BED events */
+    int32_t pad7;
+    int32_t beyond;               /* CgDev::beyond */
+    int32_t window_max;           /* most candidate reads of one tile */
+    int32_t n_sitem;              /* STR items of the slice */
+    int32_t next_col;             /* in the mirror only: the next call's first column (k_find_col) */
+    int64_t qual_total;           /* a packed batch: padded quality bytes */
+    int32_t cigar_total;          /* a packed batch: CIGAR operations */
+    int32_t pad15;
+    int64_t cell_groups;          /* cell matrix */
+    struct { int32_t tile_counter, pad; unsigned long long item_bound; } slice;   /* reset before each column stage: k_column's tile counter, STR item bound */
+    int32_t pad22[2];
+};
+struct CgScalars {
+    CgScalHead h;
+    int32_t n_glist;              /* reads with a non-trivial CIGAR */
+    int32_t pad25[7];
+    unsigned long long counters[CG_N_COUNTERS];
+    char pad_counters[512 - 128 - 8 * CG_N_COUNTERS];
+    CgChainCarry chain;
+    char pad_chain[640 - 512 - sizeof(CgChainCarry)];
+    CgEpochCarry epoch;
+    char pad_epoch[768 - 640 - sizeof(CgEpochCarry)];
+    int64_t bounds[3 * CG_MAX_CHUNKS];                     /* k_bounds */
+    char pad_bounds[1600 - 768 - 8 * 3 * CG_MAX_CHUNKS];
+    CgChainCarry chain_import;    /* cg_shard_end paints from the carry the shard imported */
+    char pad_end[2048 - 1600 - sizeof(CgChainCarry)];
+};
+#define CG_SCAL_AT(f, off) static_assert(offsetof(CgScalars, f) == (off), "scalar block: " #f " must stay at byte " #off)
+CG_SCAL_AT(h.n_pile, 0); CG_SCAL_AT(h.n_cols, 4); CG_SCAL_AT(h.n_islands, 8); CG_SCAL_AT(h.n_flagged, 12);
+CG_SCAL_AT(h.maxdepth, 16); CG_SCAL_AT(h.err, 20); CG_SCAL_AT(h.n_events, 24); CG_SCAL_AT(h.beyond, 32);
+CG_SCAL_AT(h.window_max, 36); CG_SCAL_AT(h.n_sitem, 40); CG_SCAL_AT(h.next_col, 44); CG_SCAL_AT(h.qual_total, 48);
+CG_SCAL_AT(h.cigar_total, 56); CG_SCAL_AT(h.cell_groups, 64); CG_SCAL_AT(h.slice.tile_counter, 72); CG_SCAL_AT(h.slice.item_bound, 80);
+CG_SCAL_AT(n_glist, 96); CG_SCAL_AT(counters, 128); CG_SCAL_AT(chain, 512); CG_SCAL_AT(epoch, 640); CG_SCAL_AT(bounds, 768);
+CG_SCAL_AT(chain_import, 1600);
+#undef CG_SCAL_AT
+static_assert(sizeof(CgScalHead) == 96, "the mirrored head is 24 int32 slots");
+static_assert(sizeof(CgScalars) == 2048, "scalar block size");
 
 struct cg_ctx {
     int device; cudaStream_t stream; int own_stream;
@@ -1331,8 +1309,8 @@ struct cg_ctx {
     int has_meta; int64_t n_truns, n_pabs, n_cigx;
     int generic;                  /* cg_params_generic(): column and rewrite stages through the plain bodies */
     /* host mirrors */
-    int32_t *d_hdims;             /* device alias of h_dims (mapped pinned memory) */
-    int32_t *h_dims;              /* pinned, mapped: [0] n_pile [1] n_cols [2] n_islands [3] n_flagged [4] maxdepth [5] err [6] n_events [7] n_epochs */
+    CgScalHead *d_hdims;          /* device alias of h_dims (mapped pinned memory) */
+    CgScalHead *h_dims;           /* pinned, mapped: the head of the scalar block */
     unsigned long long *h_counters;
     CgDev D;
     int resident; int dump_columns;
@@ -1344,14 +1322,6 @@ struct cg_ctx {
     int packed, offsets_ready; int64_t h2d_bytes;                           /* offsets rebuilt on the device; bytes copied up by the last call */       /* chained calls: this call's window, the carries of the previous one */
     cudaStream_t s_h2d, s_d2h; cudaEvent_t ev_up[32], ev_done[32], ev_misc;
     char h_carry_init[64];
-    /* compact download of the rewritten qualities (k_rewrite phase C'): device planes, pinned host copies, the slices in flight */
-    dbuf b_cqmask, b_cqexc, b_cqblk;
-    uint8_t *h_cqmask, *h_cqexc; int64_t *h_cqblk; size_t h_cqmask_cap, h_cqexc_cap, h_cqblk_cap;
-    struct CgCqSlice { int64_t r0, r1, blk0, nblk; } cq_sl[2 * CG_MAX_CHUNKS + 2];
-    int cq_on, cq_n, cq_done; int64_t cq_blk_total; unsigned long long cq_exc_copied; int64_t cq_blk_copied;
-    cudaEvent_t cq_ev[2 * CG_MAX_CHUNKS + 2]; int cq_ev_made;
-    pthread_mutex_t cq_mu; pthread_cond_t cq_cv; int cq_ready, cq_quit, cq_sync_made;
-    const cg_batch *cq_in; cg_result *cq_out;
     char *h_carry_io;                                           /* pinned: [0, 128) the state a shard imported, [128, 256) the one it exports */
     CgSlice sl[2 * CG_MAX_CHUNKS + 2]; int n_sl, shard_state, shard_next, shard_save_end, shard_timed; const cg_batch *shard_in;
     cudaEvent_t ev[CG_N_TIMERS][2];
@@ -1435,7 +1405,7 @@ extern "C" cg_ctx *cg_create(const cg_params *p, int device, int *err) {
     ctx->own_stream = 1;
     ctx->hT = (CgTables *)malloc(sizeof(CgTables));
     if (!e && cudaMalloc((void **)&ctx->dT, sizeof(CgTables)) != cudaSuccess) e = CG_ERR_CUDA;
-    if (!e && cudaHostAlloc((void **)&ctx->h_dims, 128, cudaHostAllocMapped) != cudaSuccess) e = CG_ERR_CUDA;
+    if (!e && cudaHostAlloc((void **)&ctx->h_dims, sizeof(CgScalHead), cudaHostAllocMapped) != cudaSuccess) e = CG_ERR_CUDA;
     if (!e && cudaHostGetDevicePointer((void **)&ctx->d_hdims, ctx->h_dims, 0) != cudaSuccess) e = CG_ERR_CUDA;
     if (!e && cudaHostAlloc((void **)&ctx->h_counters, sizeof(unsigned long long) * 32, cudaHostAllocDefault) != cudaSuccess) e = CG_ERR_CUDA;
     if (!e && cudaHostAlloc((void **)&ctx->h_carry_io, 2 * CG_CARRY_BYTES, cudaHostAllocDefault) != cudaSuccess) e = CG_ERR_CUDA;
@@ -1453,7 +1423,7 @@ extern "C" void cg_destroy(cg_ctx *ctx) {
     dbuf *all[] = { &ctx->b_tid, &ctx->b_pos, &ctx->b_flag, &ctx->b_mapq, &ctx->b_lq, &ctx->b_nc, &ctx->b_off, &ctx->b_coff, &ctx->b_cigar,
         &ctx->b_seq, &ctx->b_qual, &ctx->b_qout, &ctx->b_jmap, &ctx->b_rspan, &ctx->b_rd, &ctx->b_ks, &ctx->b_ke, &ctx->b_gap, &ctx->b_gapraw,
         &ctx->b_pmax, &ctx->b_orig, &ctx->b_rbf, &ctx->b_glist, &ctx->b_tlo, &ctx->b_tstart, &ctx->b_isl, &ctx->b_cb, &ctx->b_ev, &ctx->b_depth, &ctx->b_dump,
-        &ctx->b_dsum, &ctx->b_csum, &ctx->b_fcol, &ctx->b_trig, &ctx->b_twin, &ctx->b_aggr, &ctx->b_scal, &ctx->b_scratch, &ctx->b_epoch, &ctx->b_events, &ctx->b_chain, &ctx->b_items, &ctx->b_bed, &ctx->b_bedpm, &ctx->b_saved, &ctx->b_crec, &ctx->b_cells, &ctx->b_seq2, &ctx->b_qualp, &ctx->b_exc, &ctx->b_cqmask, &ctx->b_cqexc, &ctx->b_cqblk,
+        &ctx->b_dsum, &ctx->b_csum, &ctx->b_fcol, &ctx->b_trig, &ctx->b_twin, &ctx->b_aggr, &ctx->b_scal, &ctx->b_scratch, &ctx->b_epoch, &ctx->b_events, &ctx->b_chain, &ctx->b_items, &ctx->b_bed, &ctx->b_bedpm, &ctx->b_saved, &ctx->b_crec, &ctx->b_cells, &ctx->b_seq2, &ctx->b_qualp, &ctx->b_exc,
         &ctx->b_truns, &ctx->b_pabs, &ctx->b_pd8, &ctx->b_lq8, &ctx->b_nc8, &ctx->b_cigx, &ctx->b_lqd, &ctx->b_xoff, &ctx->b_absS,
         &ctx->b_qsrc, &ctx->b_ssrc, &ctx->b_dvsum };
     for (size_t i = 0; i < sizeof(all) / sizeof(all[0]); i++) if (all[i]->p) cudaFree(all[i]->p);
@@ -1461,11 +1431,6 @@ extern "C" void cg_destroy(cg_ctx *ctx) {
     if (ctx->h_dims) cudaFreeHost(ctx->h_dims);
     if (ctx->h_counters) cudaFreeHost(ctx->h_counters);
     if (ctx->h_carry_io) cudaFreeHost(ctx->h_carry_io);
-    if (ctx->h_cqmask) cudaFreeHost(ctx->h_cqmask);
-    if (ctx->h_cqexc) cudaFreeHost(ctx->h_cqexc);
-    if (ctx->h_cqblk) cudaFreeHost(ctx->h_cqblk);
-    for (int i = 0; i < ctx->cq_ev_made; i++) cudaEventDestroy(ctx->cq_ev[i]);
-    if (ctx->cq_sync_made) { pthread_mutex_destroy(&ctx->cq_mu); pthread_cond_destroy(&ctx->cq_cv); }
     for (int i = 0; i < CG_N_TIMERS; i++) for (int k = 0; k < 2; k++) if (ctx->ev[i][k]) cudaEventDestroy(ctx->ev[i][k]);
     if (ctx->s_h2d) { cudaStreamDestroy(ctx->s_h2d); cudaStreamDestroy(ctx->s_d2h); for (int i = 0; i < 32; i++) { cudaEventDestroy(ctx->ev_up[i]); cudaEventDestroy(ctx->ev_done[i]); } cudaEventDestroy(ctx->ev_misc); }
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -1694,10 +1659,6 @@ struct StCompactOff { int32_t *out; const uint16_t *ev; uint16_t mask; int32_t c
 struct StI64Carry { int64_t *p; const CgEpochCarry *cy; __device__ void operator()(int64_t i, int64_t inc, int64_t) const { p[i] = inc + cy->dsum_last; } };
 struct StI32Carry { int32_t *p; const CgEpochCarry *cy; __device__ void operator()(int64_t i, int32_t inc, int32_t) const { p[i] = inc + cy->csum_last; } };
 
-/* scalars on the device (b_scal): int32 [0] n_pile [1] n_cols [2] n_islands [3] n_flagged of the slice [4] maxdepth [5] err
- * [6] n_events [7] - [8] beyond [9] window max [10] STR items [12..13] packed quality bytes [14] packed CIGAR ops
- * [16..17] cell groups [18] tile counter of k_column [20..21] STR item bound of the slice [22..23] compact-download exception count
- * [24] reads with a non-trivial CIGAR; counters at +128 B; chain carry at +512 B; epoch carry at +640 B; bounds at +768 B */
 static int run_prep(cg_ctx *ctx, const CgBounds *bounds, int64_t *h_bounds) {
     cudaStream_t st = ctx->stream;
     CgDev *D = &ctx->D;
@@ -1713,10 +1674,10 @@ static int run_prep(cg_ctx *ctx, const CgBounds *bounds, int64_t *h_bounds) {
         D->P.win_hi_tid = w->hi_tid; D->P.win_hi_pos = w->hi_pos;
     }
     D->bed = (const cg_bed_reg *)ctx->b_bed.p; D->bed_pm = (const int64_t *)ctx->b_bedpm.p;
-    if ((e = ensure(ctx, &ctx->b_scal, 2048))) return e;
-    int32_t *scal = (int32_t *)ctx->b_scal.p;
-    D->counters = (unsigned long long *)((char *)ctx->b_scal.p + 128);
-    D->maxdepth = scal + 4; D->err = scal + 5; D->beyond = scal + 8;
+    if ((e = ensure(ctx, &ctx->b_scal, sizeof(CgScalars)))) return e;
+    CgScalars *scal = (CgScalars *)ctx->b_scal.p;
+    D->counters = scal->counters;
+    D->maxdepth = &scal->h.maxdepth; D->err = &scal->h.err; D->beyond = &scal->h.beyond;
     if ((e = ensure(ctx, &ctx->b_jmap, n1 * 4)) || (e = ensure(ctx, &ctx->b_rspan, n1 * 4)) || (e = ensure(ctx, &ctx->b_rd, n1 * sizeof(CgRead))) ||
         (e = ensure(ctx, &ctx->b_ks, n1 * 8)) || (e = ensure(ctx, &ctx->b_ke, n1 * 8)) || (e = ensure(ctx, &ctx->b_gap, n1 * 8)) ||
         (e = ensure(ctx, &ctx->b_gapraw, n1 * 8)) || (e = ensure(ctx, &ctx->b_pmax, n1 * 4)) || (e = ensure(ctx, &ctx->b_orig, n1 * 4)) ||
@@ -1725,19 +1686,19 @@ static int run_prep(cg_ctx *ctx, const CgBounds *bounds, int64_t *h_bounds) {
     D->ks = (int64_t *)ctx->b_ks.p; D->ke = (int64_t *)ctx->b_ke.p; D->gap = (int64_t *)ctx->b_gap.p;
     D->pmaxcol = (int32_t *)ctx->b_pmax.p; D->orig = (int32_t *)ctx->b_orig.p; D->r_bf = (uint8_t *)ctx->b_rbf.p;
     D->isl = (CgIsland *)ctx->b_isl.p;
-    D->glist = ctx->generic ? NULL : (int32_t *)ctx->b_glist.p; D->n_glist = scal + 24;
+    D->glist = ctx->generic ? NULL : (int32_t *)ctx->b_glist.p; D->n_glist = &scal->n_glist;
     int64_t *gapraw = (int64_t *)ctx->b_gapraw.p;
 
     T0(CG_T_TILES);
-    CG_CHECK(cudaMemsetAsync(ctx->b_scal.p, 0, 2048, st));
+    CG_CHECK(cudaMemsetAsync(scal, 0, sizeof(CgScalars), st));
     {
         CgChainCarry cc; memset(&cc, 0, sizeof cc); cc.bkey = INT64_MIN; cc.ukey = INT64_MIN; cg_win_reset(&cc.w);
         memcpy(ctx->h_carry_init, &cc, sizeof cc);
-        CG_CHECK(cudaMemcpyAsync((char *)ctx->b_scal.p + 512, ctx->h_carry_init, sizeof cc, cudaMemcpyHostToDevice, st));
+        CG_CHECK(cudaMemcpyAsync(&scal->chain, ctx->h_carry_init, sizeof cc, cudaMemcpyHostToDevice, st));
         if (ctx->win_on && !ctx->win.first && ctx->have_saved) {       /* continue where the previous call of the chain stopped */
             const CgSavedCarry *sv = (const CgSavedCarry *)ctx->b_saved.p;
-            CG_CHECK(cudaMemcpyAsync((char *)ctx->b_scal.p + 512, &sv->cc, sizeof(CgChainCarry), cudaMemcpyDeviceToDevice, st));
-            CG_CHECK(cudaMemcpyAsync((char *)ctx->b_scal.p + 640, &sv->ec, sizeof(CgEpochCarry), cudaMemcpyDeviceToDevice, st));
+            CG_CHECK(cudaMemcpyAsync(&scal->chain, &sv->cc, sizeof(CgChainCarry), cudaMemcpyDeviceToDevice, st));
+            CG_CHECK(cudaMemcpyAsync(&scal->epoch, &sv->ec, sizeof(CgEpochCarry), cudaMemcpyDeviceToDevice, st));
         }
     }
     if (n > 0 && ctx->packed && !ctx->offsets_ready) {         /* once per uploaded batch: off = running sum of the padded lengths, cigar_off = running sum of n_cigar */
@@ -1751,9 +1712,9 @@ static int run_prep(cg_ctx *ctx, const CgBounds *bounds, int64_t *h_bounds) {
             ctx->launches += 2;
         }
         LdPad8 lp = { D->l_qseq }; StExcl64 so = { (int64_t *)ctx->b_off.p };
-        if ((e = run_scan<int64_t, OpSum>(ctx, lp, so, n, (int64_t)0, (int64_t *)(scal + 12)))) return e;
+        if ((e = run_scan<int64_t, OpSum>(ctx, lp, so, n, (int64_t)0, &scal->h.qual_total))) return e;
         LdNCig ln = { D->n_cigar }; StExcl32 sc = { (int32_t *)ctx->b_coff.p };
-        if ((e = run_scan<int32_t, OpSum>(ctx, ln, sc, n, 0, scal + 14))) return e;
+        if ((e = run_scan<int32_t, OpSum>(ctx, ln, sc, n, 0, &scal->h.cigar_total))) return e;
         if (ctx->has_meta) {
             LdNcx lx = { (const uint8_t *)ctx->b_nc8.p }; StExcl32 sx = { (int32_t *)ctx->b_xoff.p };
             if ((e = run_scan<int32_t, OpSum>(ctx, lx, sx, n, 0, (int32_t *)NULL))) return e;
@@ -1766,46 +1727,46 @@ static int run_prep(cg_ctx *ctx, const CgBounds *bounds, int64_t *h_bounds) {
     if (n > 0) {
         k_prep_read<<<nblk(n, 256), 256, 0, st>>>(*D); ctx->launches++;
         LdPileFlag lpf = { D->rspan }; StJmap sj = { D->jmap };
-        if ((e = run_scan<int32_t, OpSum>(ctx, lpf, sj, n, 0, scal + 0))) return e;
+        if ((e = run_scan<int32_t, OpSum>(ctx, lpf, sj, n, 0, &scal->h.n_pile))) return e;
         k_prep_keys<<<nblk(n, 256), 256, 0, st>>>(*D); ctx->launches++;
         /* ke := inclusive prefix max (only the first n_pile entries are meaningful; the tail is never read) */
-        CG_CHECK(cudaMemcpyAsync(ctx->h_dims, scal, 64, cudaMemcpyDeviceToHost, st));
+        CG_CHECK(cudaMemcpyAsync(ctx->h_dims, &scal->h, sizeof(CgScalHead), cudaMemcpyDeviceToHost, st));
         CG_CHECK(cudaStreamSynchronize(st));
         if (check_packed) {                                        /* packed = 1 is a promise about the layout: the running sums must end where the buffers do */
-            int64_t qtot; memcpy(&qtot, ctx->h_dims + 12, 8);
-            if (qtot > ctx->qual_bytes || (int64_t)ctx->h_dims[14] > ctx->cigar_total) {
+            const int64_t qtot = ctx->h_dims->qual_total;
+            if (qtot > ctx->qual_bytes || (int64_t)ctx->h_dims->cigar_total > ctx->cigar_total) {
                 snprintf(ctx->err, sizeof ctx->err, "packed batch: the padded lengths sum to %lld quality bytes (buffer holds %lld), the CIGARs to %d operations (buffer holds %lld)",
-                         (long long)qtot, (long long)ctx->qual_bytes, ctx->h_dims[14], (long long)ctx->cigar_total);
+                         (long long)qtot, (long long)ctx->qual_bytes, ctx->h_dims->cigar_total, (long long)ctx->cigar_total);
                 return CG_ERR_BAD_ARG;
             }
         }
-        D->n_pile = ctx->h_dims[0];
+        D->n_pile = ctx->h_dims->n_pile;
     } else D->n_pile = 0;
     const int np = D->n_pile;
     if (np > 0) {
         LdI64 lke = { D->ke }; StI64Incl ske = { D->ke };
         if ((e = run_scan<int64_t, OpMax>(ctx, lke, ske, np, (int64_t)INT64_MIN, (int64_t *)NULL))) return e;
-        k_gap<<<nblk(np, 256), 256, 0, st>>>(*D, scal + 0, gapraw); ctx->launches++;
+        k_gap<<<nblk(np, 256), 256, 0, st>>>(*D, &scal->h.n_pile, gapraw); ctx->launches++;
         LdI64 lg = { gapraw }; StI64Incl sg = { D->gap };
         if ((e = run_scan<int64_t, OpSum>(ctx, lg, sg, np, (int64_t)0, (int64_t *)NULL))) return e;
         LdIslandFlag lif = { gapraw }; StIsland sis = { D->isl, D->ks, D->gap, gapraw };
-        if ((e = run_scan<int32_t, OpSum>(ctx, lif, sis, np, 0, scal + 2))) return e;
-        k_finish_read<<<nblk(np, 256), 256, 0, st>>>(*D, scal + 0, scal); ctx->launches++;
-        if (!ctx->generic) {                                       /* cell matrix: first group of every row, total in scal[16..17] */
+        if ((e = run_scan<int32_t, OpSum>(ctx, lif, sis, np, 0, &scal->h.n_islands))) return e;
+        k_finish_read<<<nblk(np, 256), 256, 0, st>>>(*D, &scal->h.n_pile, &scal->h.n_cols); ctx->launches++;
+        if (!ctx->generic) {                                       /* cell matrix: first group of every row, total in cell_groups */
             if ((e = ensure(ctx, &ctx->b_crec, ((size_t)np + 1) * sizeof(CgCellRec)))) return e;
             D->crec = (CgCellRec *)ctx->b_crec.p;
             LdNgrp lg2 = { D->rd }; StCellRec sc2 = { D->crec, D->rd };
-            if ((e = run_scan<int64_t, OpSum>(ctx, lg2, sc2, np, (int64_t)0, (int64_t *)(scal + 16)))) return e;
+            if ((e = run_scan<int64_t, OpSum>(ctx, lg2, sc2, np, (int64_t)0, &scal->h.cell_groups))) return e;
         }
     }
-    CG_CHECK(cudaMemcpyAsync(ctx->h_dims, scal, 96, cudaMemcpyDeviceToHost, st));
+    CG_CHECK(cudaMemcpyAsync(ctx->h_dims, &scal->h, sizeof(CgScalHead), cudaMemcpyDeviceToHost, st));
     CG_CHECK(cudaStreamSynchronize(st));
-    if (ctx->h_dims[5]) { snprintf(ctx->err, sizeof ctx->err, "device reported error %d while building read records", ctx->h_dims[5]); return ctx->h_dims[5]; }
-    D->n_cols = np > 0 ? ctx->h_dims[1] : 0; D->n_islands = np > 0 ? ctx->h_dims[2] : 0;
+    if (ctx->h_dims->err) { snprintf(ctx->err, sizeof ctx->err, "device reported error %d while building read records", ctx->h_dims->err); return ctx->h_dims->err; }
+    D->n_cols = np > 0 ? ctx->h_dims->n_cols : 0; D->n_islands = np > 0 ? ctx->h_dims->n_islands : 0;
     D->n_tiles = (D->n_cols + 31) / 32;
     D->n_flagged = 0;
     if (np > 0 && !ctx->generic) {
-        int64_t ng; memcpy(&ng, ctx->h_dims + 16, 8);
+        const int64_t ng = ctx->h_dims->cell_groups;
         if (ng >= (1LL << 32)) { snprintf(ctx->err, sizeof ctx->err, "batch too large: split it"); return CG_ERR_BAD_ARG; }
         if ((e = ensure(ctx, &ctx->b_cells, (size_t)ng * 16 + 64))) return e;
         D->cells = (uint16_t *)ctx->b_cells.p;
@@ -1829,13 +1790,13 @@ static int run_prep(cg_ctx *ctx, const CgBounds *bounds, int64_t *h_bounds) {
         k_fill_i32<<<nblk(D->n_tiles + 2, 256), 256, 0, st>>>(D->tile_lo, D->n_tiles + 2, np);
         k_fill_i32<<<nblk(D->n_tiles + 2, 256), 256, 0, st>>>(D->tile_start, D->n_tiles + 2, np);
         k_tile_index<<<nblk(np, 256), 256, 0, st>>>(*D);
-        k_window_max<<<nblk(D->n_tiles, 256), 256, 0, st>>>(*D, scal + 9);
-        k_bounds<<<1, CG_MAX_CHUNKS, 0, st>>>(*D, *bounds, (int64_t *)((char *)ctx->b_scal.p + 768)); ctx->launches += 5;
-        CG_CHECK(cudaMemcpyAsync(ctx->h_dims, scal, 48, cudaMemcpyDeviceToHost, st));
-        CG_CHECK(cudaMemcpyAsync(h_bounds, (char *)ctx->b_scal.p + 768, sizeof(int64_t) * 3 * CG_MAX_CHUNKS, cudaMemcpyDeviceToHost, st));
+        k_window_max<<<nblk(D->n_tiles, 256), 256, 0, st>>>(*D, &scal->h.window_max);
+        k_bounds<<<1, CG_MAX_CHUNKS, 0, st>>>(*D, *bounds, scal->bounds); ctx->launches += 5;
+        CG_CHECK(cudaMemcpyAsync(ctx->h_dims, &scal->h, sizeof(CgScalHead), cudaMemcpyDeviceToHost, st));
+        CG_CHECK(cudaMemcpyAsync(h_bounds, scal->bounds, sizeof scal->bounds, cudaMemcpyDeviceToHost, st));
         CG_CHECK(cudaStreamSynchronize(st));
         /* over-depth (snp_score.c:1673) needs n_plp > -P * mean depth >= -P: impossible when no tile has more than -P candidates */
-        ctx->need_depth = ctx->params.over_depth < 1.0 || (double)ctx->h_dims[9] > ctx->params.over_depth;
+        ctx->need_depth = ctx->params.over_depth < 1.0 || (double)ctx->h_dims->window_max > ctx->params.over_depth;
         ctx->depth_matters = ctx->need_depth;
         if (ctx->win_on) ctx->need_depth = 1;                       /* a later call of the chain may need the running average */
         if (ctx->need_depth) {
@@ -1857,12 +1818,10 @@ static int run_prep(cg_ctx *ctx, const CgBounds *bounds, int64_t *h_bounds) {
  * A single context runs A, B1, B2 slice after slice.  Region shards on several devices (cg_shard_*) run A for all their slices at
  * once, pass the carry from shard to shard through B1 alone, and run B2 concurrently again. */
 
-static void cq_bind(cg_ctx *ctx);
-
 static int slice_A(cg_ctx *ctx, CgSlice *s, int timed) {
     cudaStream_t st = ctx->stream;
     CgDev *D = &ctx->D;
-    int32_t *scal = (int32_t *)ctx->b_scal.p;
+    CgScalars *scal = (CgScalars *)ctx->b_scal.p;
     int e;
     const int ncs = s->c1 > s->c0 ? s->c1 - s->c0 : 0;          /* columns of the sparse passes: the tiles' own, except in chained calls */
     int nfs = 0;
@@ -1874,26 +1833,25 @@ static int slice_A(cg_ctx *ctx, CgSlice *s, int timed) {
         ctx->launches += 2;
     }
     if (timed) { T1(CG_T_CELLS); T0(CG_T_COLUMNS); }
-    D->item_bound = (unsigned long long *)(scal + 20);
+    D->item_bound = &scal->h.slice.item_bound;
     if (s->t1 > s->t0) {
-        CG_CHECK(cudaMemsetAsync(scal + 18, 0, 16, st));        /* tile counter, STR item bound of this slice */
+        CG_CHECK(cudaMemsetAsync(&scal->h.slice, 0, sizeof scal->h.slice, st));
         if (ctx->generic) k_column_generic<<<nblk((int64_t)(s->t1 - s->t0) * 32, 128), 128, 0, st>>>(*D, s->t0, s->t1);
         else {
             /* persistent warps claim tiles from a counter: one warp slot per resident warp, never more warps than tiles */
             int blocks = nblk(s->t1 - s->t0, COL_WARPS);
             if (blocks > 148 * COL_MINB) blocks = 148 * COL_MINB;
-            k_column<<<blocks, COL_WARPS * 32, 0, st>>>(*D, s->t0, s->t1, scal + 18);
+            k_column<<<blocks, COL_WARPS * 32, 0, st>>>(*D, s->t0, s->t1, &scal->h.slice.tile_counter);
         }
         ctx->launches++;
     }
     if (timed) { T1(CG_T_COLUMNS); T0(CG_T_FLAGGED); }
     if (ncs > 0) {
         LdEvFlagOff lf = { D->ev + s->c0, CG_EV_FLAGGED }; StCompactOff sc = { D->fcol + kb, D->ev + s->c0, CG_EV_FLAGGED, s->c0 };
-        if ((e = run_scan<int32_t, OpSum>(ctx, lf, sc, ncs, 0, scal + 3))) return e;
-        k_publish<<<1, 32, 0, st>>>(scal, ctx->d_hdims, 24); ctx->launches++;
+        if ((e = run_scan<int32_t, OpSum>(ctx, lf, sc, ncs, 0, &scal->h.n_flagged))) return e;
+        k_publish<<<1, 32, 0, st>>>((const int32_t *)&scal->h, (int32_t *)ctx->d_hdims, (int)(sizeof(CgScalHead) / 4)); ctx->launches++;
         CG_CHECK(cudaStreamSynchronize(st));
-        nfs = ctx->h_dims[3];
-        s->synced = 1;                                          /* h_dims is current: n_flagged, STR item bound, compact-download exception count */
+        nfs = ctx->h_dims->n_flagged;
     }
     const int ke = kb + nfs;
     if ((e = ensure_keep(ctx, &ctx->b_trig, ((size_t)ke + 1) * sizeof(CgTrig))) || (e = ensure_keep(ctx, &ctx->b_twin, ((size_t)ke + 1) * sizeof(CgWin)))) return e;
@@ -1903,11 +1861,11 @@ static int slice_A(cg_ctx *ctx, CgSlice *s, int timed) {
         int threads = FL_WARPS * 32, blocks = nblk(nfs, FL_WARPS);
         if (blocks > 148 * 8) blocks = 148 * 8;
         /* the item list holds at most what the slice's columns announced (their bound came over with n_flagged) */
-        int64_t ub; memcpy(&ub, ctx->h_dims + 20, 8);
+        const int64_t ub = (int64_t)ctx->h_dims->slice.item_bound;
         if (ub > 0x7fffff00LL) { snprintf(ctx->err, sizeof ctx->err, "too many STR searches in one slice"); return CG_ERR_OVERFLOW; }
         if ((e = ensure(ctx, &ctx->b_items, ((size_t)ub + 1) * sizeof(CgStrItem)))) return e;
-        D->sitem = (CgStrItem *)ctx->b_items.p; D->sitem_cap = ub; D->n_sitem = scal + 10;
-        CG_CHECK(cudaMemsetAsync(scal + 10, 0, 4, st));
+        D->sitem = (CgStrItem *)ctx->b_items.p; D->sitem_cap = ub; D->n_sitem = &scal->h.n_sitem;
+        CG_CHECK(cudaMemsetAsync(&scal->h.n_sitem, 0, sizeof scal->h.n_sitem, st));
         k_flagged<<<blocks, threads, 0, st>>>(*D, kb, ke); ctx->launches++;
         if (ub > 0) {
             int sblocks = nblk(ub, STR_THREADS);
@@ -1926,8 +1884,8 @@ static int slice_A(cg_ctx *ctx, CgSlice *s, int timed) {
 static int slice_B(cg_ctx *ctx, const CgSlice *s, int what, int timed) {
     cudaStream_t st = ctx->stream;
     CgDev *D = &ctx->D;
-    CgChainCarry *ccarry = (CgChainCarry *)((char *)ctx->b_scal.p + 512);
-    CgEpochCarry *ecarry = (CgEpochCarry *)((char *)ctx->b_scal.p + 640);
+    CgChainCarry *ccarry = &((CgScalars *)ctx->b_scal.p)->chain;
+    CgEpochCarry *ecarry = &((CgScalars *)ctx->b_scal.p)->epoch;
     int e;
     const int c0 = s->c0, c1 = s->c1, kb = s->kb, ke = s->ke, nfs = ke - kb;
     const int ncs = c1 > c0 ? c1 - c0 : 0;
@@ -1965,7 +1923,7 @@ static int slice_B(cg_ctx *ctx, const CgSlice *s, int what, int timed) {
     if (timed) { T1(CG_T_CHAIN); T0(CG_T_REWRITE); }
     if ((what & 2) && s->r1 > s->r0) {
         if (ctx->generic) k_rewrite_generic<<<nblk(s->r1 - s->r0, 128), 128, 0, st>>>(*D, s->r0, s->r1);
-        else { cq_bind(ctx); k_rewrite<<<nblk(s->r1 - s->r0, RW_READS), RW_THREADS, 0, st>>>(*D, s->r0, s->r1, ctx->cq_blk_total); }
+        else k_rewrite<<<nblk(s->r1 - s->r0, RW_READS), RW_THREADS, 0, st>>>(*D, s->r0, s->r1);
         ctx->launches++;
     }
     if (timed) T1(CG_T_REWRITE);
@@ -1973,11 +1931,18 @@ static int slice_B(cg_ctx *ctx, const CgSlice *s, int what, int timed) {
     return 0;
 }
 
+static void read_timer(cg_ctx *ctx, int i) {
+    float ms = 0;
+    if (cudaEventElapsedTime(&ms, ctx->ev[i][0], ctx->ev[i][1]) == cudaSuccess) ctx->ms[i] = ms; else cudaGetLastError();
+}
+/* the spans of the last call's uploads and downloads */
+static void read_copy_timers(cg_ctx *ctx) { read_timer(ctx, CG_T_H2D); read_timer(ctx, CG_T_D2H); }
+
 /* ordered BED event list, counters, dump flags; leaves everything small on the host side of the context */
 static int run_finish(cg_ctx *ctx, int timed) {
     cudaStream_t st = ctx->stream;
     CgDev *D = &ctx->D;
-    int32_t *scal = (int32_t *)ctx->b_scal.p;
+    CgScalars *scal = (CgScalars *)ctx->b_scal.p;
     const int nc = D->n_cols;
     int e;
     if (timed) T0(CG_T_EVENTS);
@@ -1986,27 +1951,27 @@ static int run_finish(cg_ctx *ctx, int timed) {
         if (!ctx->b_events.p) { if ((e = ensure(ctx, &ctx->b_events, sizeof(cg_bed_event) * 65536))) return e; }
         ctx->events_cap_dev = (int64_t)(ctx->b_events.cap / sizeof(cg_bed_event));
         LdEvCount le = { D->ev }; StEvents se = { (cg_bed_event *)ctx->b_events.p, D->ev, *D, ctx->events_cap_dev };
-        if ((e = run_scan<int32_t, OpSum>(ctx, le, se, nc, 0, scal + 6))) return e;
+        if ((e = run_scan<int32_t, OpSum>(ctx, le, se, nc, 0, &scal->h.n_events))) return e;
         if (D->want_dump) { k_dump_flags<<<nblk(nc, 256), 256, 0, st>>>(*D); ctx->launches++; }
     }
     if (timed) T1(CG_T_EVENTS);
     T1(CG_T_TOTAL);
-    CG_CHECK(cudaMemcpyAsync(ctx->h_dims, scal, 96, cudaMemcpyDeviceToHost, st));
+    CG_CHECK(cudaMemcpyAsync(ctx->h_dims, &scal->h, sizeof(CgScalHead), cudaMemcpyDeviceToHost, st));
     CG_CHECK(cudaMemcpyAsync(ctx->h_counters, D->counters, sizeof(unsigned long long) * CG_N_COUNTERS, cudaMemcpyDeviceToHost, st));
     CG_CHECK(cudaStreamSynchronize(st));
     CG_CHECK(cudaGetLastError());
     for (int i = 0; i < CG_N_TIMERS; i++) {
         if (i == CG_T_H2D || i == CG_T_D2H) continue;
         if (!timed && i != CG_T_TOTAL && i != CG_T_TILES) continue;
-        float ms = 0; if (cudaEventElapsedTime(&ms, ctx->ev[i][0], ctx->ev[i][1]) == cudaSuccess) ctx->ms[i] = ms; else cudaGetLastError();
+        read_timer(ctx, i);
     }
-    if (ctx->h_dims[5]) { snprintf(ctx->err, sizeof ctx->err, "device reported error %d", ctx->h_dims[5]); return ctx->h_dims[5]; }
-    if (ctx->h_dims[6] > ctx->events_cap_dev) {
+    if (ctx->h_dims->err) { snprintf(ctx->err, sizeof ctx->err, "device reported error %d", ctx->h_dims->err); return ctx->h_dims->err; }
+    if (ctx->h_dims->n_events > ctx->events_cap_dev) {
         /* more BED events than the device list holds: grow and redo the (cheap) ordered scatter */
-        if ((e = ensure(ctx, &ctx->b_events, sizeof(cg_bed_event) * ((size_t)ctx->h_dims[6] + 1024)))) return e;
+        if ((e = ensure(ctx, &ctx->b_events, sizeof(cg_bed_event) * ((size_t)ctx->h_dims->n_events + 1024)))) return e;
         ctx->events_cap_dev = (int64_t)(ctx->b_events.cap / sizeof(cg_bed_event));
         LdEvCount le = { D->ev }; StEvents se = { (cg_bed_event *)ctx->b_events.p, D->ev, *D, ctx->events_cap_dev };
-        if ((e = run_scan<int32_t, OpSum>(ctx, le, se, nc, 0, scal + 6))) return e;
+        if ((e = run_scan<int32_t, OpSum>(ctx, le, se, nc, 0, &scal->h.n_events))) return e;
         CG_CHECK(cudaStreamSynchronize(st));
     }
     ctx->resident = 2;
@@ -2022,7 +1987,6 @@ extern "C" int cg_run(cg_ctx *ctx) {
     int e;
     T0(CG_T_TOTAL);
     if ((e = run_prep(ctx, &B, hb))) return e;
-    ctx->cq_on = 0;                                            /* resident batch: flat output, fetched by cg_download */
     CgSlice sl; memset(&sl, 0, sizeof sl);
     sl.t1 = ctx->D.n_tiles; sl.c1 = ctx->D.n_cols; sl.r1 = ctx->D.n_reads; sl.je = ctx->D.n_pile;
     if ((e = slice_A(ctx, &sl, 1)) || (e = slice_B(ctx, &sl, 3, 1))) return e;
@@ -2033,9 +1997,8 @@ extern "C" int cg_run(cg_ctx *ctx) {
 static int download_results(cg_ctx *ctx, cg_result *out, int q_too) {
     cudaStream_t st = ctx->stream;
     if (q_too) T0(CG_T_D2H);
-    /* after a compact download the flat device buffer was never written: the qualities are already in the caller's buffer */
-    if (q_too && !ctx->cq_on && out->qual_out && ctx->qual_bytes) CG_CHECK(cudaMemcpyAsync(out->qual_out, ctx->b_qout.p, (size_t)ctx->qual_bytes, cudaMemcpyDeviceToHost, st));
-    out->n_events = ctx->h_dims[6];
+    if (q_too && out->qual_out && ctx->qual_bytes) CG_CHECK(cudaMemcpyAsync(out->qual_out, ctx->b_qout.p, (size_t)ctx->qual_bytes, cudaMemcpyDeviceToHost, st));
+    out->n_events = ctx->h_dims->n_events;
     if (out->events && out->n_events) {
         int64_t k = out->n_events < out->events_cap ? out->n_events : out->events_cap;
         if (k) CG_CHECK(cudaMemcpyAsync(out->events, ctx->b_events.p, sizeof(cg_bed_event) * (size_t)k, cudaMemcpyDeviceToHost, st));
@@ -2050,7 +2013,7 @@ static int download_results(cg_ctx *ctx, cg_result *out, int q_too) {
     if (q_too) T1(CG_T_D2H);
     CG_CHECK(cudaStreamSynchronize(st));
     for (int i = 0; i < CG_N_COUNTERS; i++) out->counters[i] = (int64_t)ctx->h_counters[i];
-    if (ctx->h_dims[8]) out->counters[CG_CNT_COLUMNS]++;   /* snp_score.c:1476 runs before the region break at 1516-1517 */
+    if (ctx->h_dims->beyond) out->counters[CG_CNT_COLUMNS]++;   /* snp_score.c:1476 runs before the region break at 1516-1517 */
     if (tmp) {
         for (int c = 0; c < ctx->D.n_cols; c++) {
             if (tmp[c].tid < 0) continue;
@@ -2067,9 +2030,7 @@ extern "C" int cg_download(cg_ctx *ctx, cg_result *out) {
     CG_CHECK(cudaSetDevice(ctx->device));
     int e = download_results(ctx, out, 1);
     if (e) return e;
-    float ms = 0;
-    if (cudaEventElapsedTime(&ms, ctx->ev[CG_T_D2H][0], ctx->ev[CG_T_D2H][1]) == cudaSuccess) ctx->ms[CG_T_D2H] = ms; else cudaGetLastError();
-    if (cudaEventElapsedTime(&ms, ctx->ev[CG_T_H2D][0], ctx->ev[CG_T_H2D][1]) == cudaSuccess) ctx->ms[CG_T_H2D] = ms; else cudaGetLastError();
+    read_copy_timers(ctx);
     return 0;
 }
 
@@ -2127,7 +2088,7 @@ extern "C" int cg_process_device(cg_ctx *ctx, const cg_dev_batch *in, uint8_t *q
         (e = dev_ptr_check(ctx, in->mapq, n, "mapq")) || (e = dev_ptr_check(ctx, in->l_qseq, n, "l_qseq")) || (e = dev_ptr_check(ctx, in->n_cigar, n, "n_cigar")) ||
         (e = dev_ptr_check(ctx, in->cigar, in->n_cigar_total, "cigar")) || (e = dev_ptr_check(ctx, in->seq, in->seq_len, "seq")) ||
         (e = dev_ptr_check(ctx, in->qual, in->qual_len, "qual")) || (e = dev_ptr_check(ctx, qual_out, in->qual_len, "qual_out"))) return e;
-    ctx->resident = 0; ctx->win_on = 0; ctx->cq_on = 0;
+    ctx->resident = 0; ctx->win_on = 0;
     ctx->dump_columns = out->columns != NULL;
     /* working buffers sized for the padded layout: the padded lengths sum to at most qual_len + 7 per record */
     cg_batch hb; memset(&hb, 0, sizeof hb);
@@ -2185,125 +2146,9 @@ extern "C" int cg_process_device(cg_ctx *ctx, const cg_dev_batch *in, uint8_t *q
     }
     T1(CG_T_D2H);
     if ((e = download_results(ctx, out, 0))) return e;          /* events, counters, column dump; synchronises the stream */
-    float ms = 0;
-    if (cudaEventElapsedTime(&ms, ctx->ev[CG_T_H2D][0], ctx->ev[CG_T_H2D][1]) == cudaSuccess) ctx->ms[CG_T_H2D] = ms; else cudaGetLastError();
-    if (cudaEventElapsedTime(&ms, ctx->ev[CG_T_D2H][0], ctx->ev[CG_T_D2H][1]) == cudaSuccess) ctx->ms[CG_T_D2H] = ms; else cudaGetLastError();
+    read_copy_timers(ctx);
     ctx->h2d_bytes = 0;
     return 0;
-}
-
-/* ---- compact download -------------------------------------------------------------------------------------------------------------
- * After the rewrite most quality bytes of a batch are one value (-u, 40 by default).  k_rewrite can leave, instead of the flat strings, one
- * bit per byte ("equals the dominant value") and the other bytes in position order; these cross PCIe (about a fifth of the flat bytes at
- * -9) and a few host threads expand them into the caller's buffer while later slices are still running.  The mask of a slice can be
- * copied as soon as its rewrite is queued; how many exception bytes it produced is known one host synchronisation later (the counter
- * travels with n_flagged of the next slice), so the exception copy trails by one slice. */
-static int cq_grow_pinned(cg_ctx *ctx, void **p, size_t *cap, size_t want) {
-    if (want <= *cap) return 0;
-    if (*p) cudaFreeHost(*p);
-    *p = NULL; *cap = 0;
-    const size_t nc = want + (want >> 3) + 4096;
-    CG_CHECK(cudaHostAlloc(p, nc, cudaHostAllocDefault));
-    *cap = nc;
-    return 0;
-}
-static int cq_begin(cg_ctx *ctx, const cg_batch *in, cg_result *out) {
-    ctx->cq_on = 0; ctx->cq_n = 0; ctx->cq_done = 0; ctx->cq_blk_total = 0; ctx->cq_exc_copied = 0; ctx->cq_blk_copied = 0;
-    ctx->cq_ready = 0; ctx->cq_quit = 0; ctx->cq_in = in; ctx->cq_out = out;
-    /* opt-in (CG_COMPACT_D2H=1): expanding on the host costs about 36 ns of CPU per record; four threads need longer for chr20 than the flat
-     * copy needs on a PCIe 5 x16 link (measured: 126 ms against 48 ms end to end).  It pays on hosts with many idle cores or a narrower link. */
-    if (!in || !(out->qual_out || out->qual_head) || ctx->generic || in->qual_bytes == 0 || !getenv("CG_COMPACT_D2H")) return 0;
-    const size_t qb = (size_t)in->qual_bytes, nblocks = (size_t)in->n_reads / RW_READS + 2 * CG_MAX_CHUNKS + 8;
-    int e;
-    if ((e = ensure(ctx, &ctx->b_cqmask, qb / 8 + 64)) || (e = ensure(ctx, &ctx->b_cqexc, qb + 64)) || (e = ensure(ctx, &ctx->b_cqblk, nblocks * 8))) return e;
-    if ((e = cq_grow_pinned(ctx, (void **)&ctx->h_cqmask, &ctx->h_cqmask_cap, qb / 8 + 64)) || (e = cq_grow_pinned(ctx, (void **)&ctx->h_cqexc, &ctx->h_cqexc_cap, qb + 64)) ||
-        (e = cq_grow_pinned(ctx, (void **)&ctx->h_cqblk, &ctx->h_cqblk_cap, nblocks * 8))) return e;
-    while (ctx->cq_ev_made < 2 * CG_MAX_CHUNKS + 2) { CG_CHECK(cudaEventCreateWithFlags(&ctx->cq_ev[ctx->cq_ev_made], cudaEventDisableTiming)); ctx->cq_ev_made++; }
-    if (!ctx->cq_sync_made) { pthread_mutex_init(&ctx->cq_mu, NULL); pthread_cond_init(&ctx->cq_cv, NULL); ctx->cq_sync_made = 1; }
-    if (!in->packed) CG_CHECK(cudaMemsetAsync(ctx->b_cqmask.p, 0xff, qb / 8 + 64, ctx->stream));   /* a caller's own layout may have gaps between records */
-    ctx->cq_on = 1;
-    return 0;
-}
-/* device pointers of the compact planes into the kernel parameter block (before the rewrite of a slice is launched) */
-static void cq_bind(cg_ctx *ctx) {
-    CgDev *D = &ctx->D;
-    if (!ctx->cq_on) { D->cq_mask = NULL; return; }
-    D->cq_mask = (uint8_t *)ctx->b_cqmask.p; D->cq_exc = (uint8_t *)ctx->b_cqexc.p; D->cq_blk = (int64_t *)ctx->b_cqblk.p;
-    D->cq_count = (unsigned long long *)((int32_t *)ctx->b_scal.p + 22); D->cq_dom = ctx->params.qhigh & 0xff;
-}
-/* a slice's rewrite has been queued: its mask can go home now */
-static int cq_slice_queued(cg_ctx *ctx, const cg_batch *in, int64_t r0, int64_t r1, int chunk) {
-    if (!ctx->cq_on || r1 <= r0) return 0;
-    cg_ctx::CgCqSlice *c = &ctx->cq_sl[ctx->cq_n++];
-    c->r0 = r0; c->r1 = r1; c->blk0 = ctx->cq_blk_total; c->nblk = (r1 - r0 + RW_READS - 1) / RW_READS;
-    ctx->cq_blk_total += c->nblk;
-    const int64_t n = in->n_reads, b0 = in->off[r0] >> 3, b1 = (r1 < n ? in->off[r1] : in->qual_bytes) >> 3;
-    CG_CHECK(cudaEventRecord(ctx->ev_done[chunk], ctx->stream));
-    CG_CHECK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_done[chunk], 0));
-    if (b1 > b0) CG_CHECK(cudaMemcpyAsync(ctx->h_cqmask + b0, (char *)ctx->b_cqmask.p + b0, (size_t)(b1 - b0), cudaMemcpyDeviceToHost, ctx->s_d2h));
-    return 0;
-}
-/* the host has just synchronised with the compute stream and h_dims[22..23] holds the exception count of everything rewritten so far:
- * copy what is new (exceptions and block offsets of the slices queued so far) and hand those slices to the expansion threads */
-static int cq_count_known(cg_ctx *ctx, unsigned long long count) {
-    if (!ctx->cq_on || ctx->cq_done >= ctx->cq_n) return 0;
-    if (count > ctx->cq_exc_copied)
-        CG_CHECK(cudaMemcpyAsync(ctx->h_cqexc + ctx->cq_exc_copied, (char *)ctx->b_cqexc.p + ctx->cq_exc_copied, (size_t)(count - ctx->cq_exc_copied), cudaMemcpyDeviceToHost, ctx->s_d2h));
-    ctx->cq_exc_copied = count;
-    if (ctx->cq_blk_total > ctx->cq_blk_copied)
-        CG_CHECK(cudaMemcpyAsync(ctx->h_cqblk + ctx->cq_blk_copied, (int64_t *)ctx->b_cqblk.p + ctx->cq_blk_copied, (size_t)(ctx->cq_blk_total - ctx->cq_blk_copied) * 8, cudaMemcpyDeviceToHost, ctx->s_d2h));
-    ctx->cq_blk_copied = ctx->cq_blk_total;
-    const int upto = ctx->cq_n;
-    CG_CHECK(cudaEventRecord(ctx->cq_ev[upto - 1], ctx->s_d2h));
-    pthread_mutex_lock(&ctx->cq_mu);
-    ctx->cq_done = upto; ctx->cq_ready = upto;
-    pthread_cond_broadcast(&ctx->cq_cv);
-    pthread_mutex_unlock(&ctx->cq_mu);
-    return 0;
-}
-/* one block of 128 records: memset the dominant value, drop the exceptions in */
-static void cq_expand_block(const cg_batch *in, const cg_result *out, int64_t ra, int64_t rb, const uint8_t *mask, const uint8_t *p, int dom) {
-    for (int64_t r = ra; r < rb; r++) {
-        const int L = in->l_qseq[r];
-        if (L <= 0) continue;
-        const int64_t o = in->off[r];
-        uint8_t *dst = (out->qual_head && o < out->head_bytes) ? out->qual_head + o : (out->qual_out ? out->qual_out + o : NULL);
-        const uint8_t *mk = mask + (o >> 3);
-        if (!dst) { for (int w = 0; 8 * w < L; w++) p += 8 - __builtin_popcount(mk[w]); continue; }
-        memset(dst, dom, (size_t)L);
-        for (int w = 0; 8 * w < L; w++) {
-            unsigned x = (~(unsigned)mk[w]) & 0xffu;
-            while (x) { const int k = __builtin_ctz(x); x &= x - 1; dst[8 * w + k] = *p++; }
-        }
-    }
-}
-struct CqWorker { cg_ctx *ctx; int t, nt; pthread_t th; };
-static void *cq_worker(void *v) {
-    CqWorker *W = (CqWorker *)v;
-    cg_ctx *ctx = W->ctx;
-    cudaSetDevice(ctx->device);
-    int next_ev = -1;                                           /* last event this thread has waited for */
-    for (int i = 0;; i++) {
-        pthread_mutex_lock(&ctx->cq_mu);
-        while (ctx->cq_ready <= i && !ctx->cq_quit) pthread_cond_wait(&ctx->cq_cv, &ctx->cq_mu);
-        const int ready = ctx->cq_ready;
-        pthread_mutex_unlock(&ctx->cq_mu);
-        if (ready <= i) break;                                  /* quit and nothing left */
-        if (next_ev < ready - 1) { cudaEventSynchronize(ctx->cq_ev[ready - 1]); next_ev = ready - 1; }
-        const cg_ctx::CgCqSlice *c = &ctx->cq_sl[i];
-        for (int64_t b = W->t; b < c->nblk; b += W->nt) {
-            const int64_t ra = c->r0 + b * RW_READS, rb = ra + RW_READS < c->r1 ? ra + RW_READS : c->r1;
-            cq_expand_block(ctx->cq_in, ctx->cq_out, ra, rb, ctx->h_cqmask, ctx->h_cqexc + ctx->h_cqblk[c->blk0 + b], ctx->params.qhigh & 0xff);
-        }
-    }
-    return NULL;
-}
-static int cq_threads(void) {
-    const char *e = getenv("CG_EXPAND_THREADS");
-    int t = e ? atoi(e) : 4;
-    const long nc = sysconf(_SC_NPROCESSORS_ONLN);
-    if (t > nc) t = (int)nc;
-    return t < 1 ? 1 : (t > 32 ? 32 : t);
 }
 
 /* the qualities of records [r0, r1) go home on the download stream once everything queued on the compute stream so far is done;
@@ -2324,6 +2169,31 @@ static int enqueue_d2h(cg_ctx *ctx, const cg_batch *in, cg_result *out, int64_t 
     return 0;
 }
 
+/* CG_TRACE: the host-side timeline of a streamed call on stderr (t0 = NULL: off) */
+static void trace_at(const struct timespec *t0, const char *what, int i) {
+    if (!t0) return;
+    struct timespec t1; clock_gettime(CLOCK_MONOTONIC, &t1);
+    fprintf(stderr, "[cg_process] %8.3f ms  %s %d\n", (t1.tv_sec - t0->tv_sec) * 1e3 + (t1.tv_nsec - t0->tv_nsec) * 1e-6, what, i);
+}
+
+/* the end of a streamed call (process_streamed, cg_shard_end), once every slice's downloads are queued: events, counters and dumps,
+ * then both copy streams drained */
+static int finish_streamed(cg_ctx *ctx, cg_result *out, const cg_window *win, int timed, const struct timespec *trace) {
+    cudaEventRecord(ctx->ev[CG_T_D2H][1], ctx->s_d2h);
+    /* a call without any pileup column (placed-unmapped reads in a coverage gap) leaves the state it resumed from untouched */
+    if (win) ctx->have_saved = win->hi_tid >= 0 && (ctx->D.n_cols > 0 || (!win->first && ctx->have_saved));
+    int e = run_finish(ctx, timed);
+    ctx->win_on = 0;
+    if (e) return e;
+    trace_at(trace, "finish done", 0);
+    if ((e = download_results(ctx, out, 0))) return e;
+    CG_CHECK(cudaStreamSynchronize(ctx->s_d2h));
+    trace_at(trace, "d2h drained", 0);
+    CG_CHECK(cudaStreamSynchronize(ctx->s_h2d));
+    read_copy_timers(ctx);
+    return 0;
+}
+
 /* End to end, streamed: the base data goes up in chunks on a copy stream; slice i of the chain starts when chunk i has
  * landed; the qualities of the records it finalises go down on a second copy stream while later chunks still arrive.
  * phase 0: everything (cg_process / cg_process_window).  phase 1: a region shard's part A only (cg_shard_begin): its slices are
@@ -2337,11 +2207,6 @@ static int process_streamed(cg_ctx *ctx, const cg_batch *in, cg_result *out, con
     ctx->win_on = 0; ctx->n_sl = 0; ctx->shard_state = 0;
     ctx->dump_columns = out->columns != NULL;
     if (!res_mode) { ctx->resident = 0; if ((e = alloc_inputs(ctx, in))) return e; }
-    ctx->cq_on = 0;
-    if (!res_mode && (e = cq_begin(ctx, in, out))) return e;
-    CqWorker cqw[32]; int n_cqw = 0;
-#define CQ_STOP() do { if (n_cqw) { pthread_mutex_lock(&ctx->cq_mu); ctx->cq_quit = 1; pthread_cond_broadcast(&ctx->cq_cv); pthread_mutex_unlock(&ctx->cq_mu); \
-        for (int t_ = 0; t_ < n_cqw; t_++) pthread_join(cqw[t_].th, NULL); n_cqw = 0; } } while (0)
     if (win) {                                                 /* one call of a chain (cg_process_window) */
         if ((e = ensure(ctx, &ctx->b_saved, sizeof(CgSavedCarry)))) return e;
         ctx->win = *win; ctx->win_on = 1; ctx->depth_matters = 0;
@@ -2391,28 +2256,21 @@ static int process_streamed(cg_ctx *ctx, const cg_batch *in, cg_result *out, con
     }
     cudaEventRecord(ctx->ev[CG_T_H2D][1], ctx->s_h2d);
     int64_t hb[3 * CG_MAX_CHUNKS];
-    const int trace = getenv("CG_TRACE") != NULL;
-    struct timespec ts0, ts1; clock_gettime(CLOCK_MONOTONIC, &ts0);
-#define CG_TRACE_AT(what, i) do { if (trace) { clock_gettime(CLOCK_MONOTONIC, &ts1); \
-        fprintf(stderr, "[cg_process] %8.3f ms  %s %d\n", (ts1.tv_sec - ts0.tv_sec) * 1e3 + (ts1.tv_nsec - ts0.tv_nsec) * 1e-6, what, i); } } while (0)
+    struct timespec ts0; clock_gettime(CLOCK_MONOTONIC, &ts0);
+    const struct timespec *trace = getenv("CG_TRACE") ? &ts0 : NULL;
     if ((e = run_prep(ctx, &B, hb))) { ctx->win_on = 0; return e; }
-    CG_TRACE_AT("prep done, chunks", nch);
+    trace_at(trace, "prep done, chunks", nch);
     /* chained call: re-open the window the previous call left active, find the column where the state is saved for the next one */
-    CgChainCarry *ccarry = (CgChainCarry *)((char *)ctx->b_scal.p + 512);
-    CgEpochCarry *ecarry = (CgEpochCarry *)((char *)ctx->b_scal.p + 640);
+    CgChainCarry *ccarry = &((CgScalars *)ctx->b_scal.p)->chain;
+    CgEpochCarry *ecarry = &((CgScalars *)ctx->b_scal.p)->epoch;
     int cS = -1;                                               /* -1: nothing to save */
     if (win && ctx->D.n_cols > 0) {
         if (phase == 0 && !win->first && ctx->have_saved) { k_paint_carry<<<1, 32, 0, st>>>(ctx->D, ccarry, win->lo_tid, win->lo_pos); ctx->launches++; }
         if (win->hi_tid >= 0) {
-            k_find_col<<<1, 32, 0, st>>>(ctx->D, win->hi_tid, win->next_lo_pos, ctx->d_hdims + 11); ctx->launches++;
+            k_find_col<<<1, 32, 0, st>>>(ctx->D, win->hi_tid, win->next_lo_pos, &ctx->d_hdims->next_col); ctx->launches++;
             CG_CHECK(cudaStreamSynchronize(st));
-            cS = ctx->h_dims[11];
+            cS = ctx->h_dims->next_col;
         }
-    }
-    if (ctx->cq_on && phase == 0) {                            /* the threads that expand the compact download into the caller's buffer */
-        n_cqw = cq_threads();
-        for (int t = 0; t < n_cqw; t++) { cqw[t].ctx = ctx; cqw[t].t = t; cqw[t].nt = n_cqw; if (pthread_create(&cqw[t].th, NULL, cq_worker, &cqw[t]) != 0) { n_cqw = t; break; } }
-        if (n_cqw == 0) ctx->cq_on = 0;                        /* no helper threads: flat download */
     }
     int tprev = 0, jprev = 0; int64_t rprev = 0;
     if (phase == 0) cudaEventRecord(ctx->ev[CG_T_D2H][0], ctx->s_d2h);
@@ -2424,7 +2282,7 @@ static int process_streamed(cg_ctx *ctx, const cg_batch *in, cg_result *out, con
         if (r1 < rprev) r1 = rprev;
         if (j1 < jprev) j1 = jprev;
         CG_CHECK(cudaStreamWaitEvent(st, ctx->ev_up[i], 0));
-        if (!res_mode && (e = expand_bases(ctx, in, boff[i], boff[i + 1], st))) { ctx->win_on = 0; CQ_STOP(); return e; }
+        if (!res_mode && (e = expand_bases(ctx, in, boff[i], boff[i + 1], st))) { ctx->win_on = 0; return e; }
         const int c0 = tprev * 32 < ctx->D.n_cols ? tprev * 32 : ctx->D.n_cols, c1 = t1 * 32 < ctx->D.n_cols ? t1 * 32 : ctx->D.n_cols;
         /* the slice(s) of this chunk: when the next call's first column cS lies inside, the sparse passes stop there, both carries are
          * saved, and a second slice (no tiles of its own) finishes the columns from cS on */
@@ -2438,43 +2296,22 @@ static int process_streamed(cg_ctx *ctx, const cg_batch *in, cg_result *out, con
             ns = 2; cS = -2;                                   /* saved (or about to be) */
         }
         for (int k = 0; k < ns; k++) {
-            if ((e = slice_A(ctx, &sl[k], res_mode && k == 0))) { ctx->win_on = 0; CQ_STOP(); return e; }   /* stage timers on a resident batch: the slice that owns the tiles */
-            if (phase == 0 && sl[k].synced) {                    /* the exception count of the slices rewritten so far came over with this slice's n_flagged */
-                unsigned long long cnt; memcpy(&cnt, ctx->h_dims + 22, 8);
-                if ((e = cq_count_known(ctx, cnt))) { ctx->win_on = 0; CQ_STOP(); return e; }
-            }
+            if ((e = slice_A(ctx, &sl[k], res_mode && k == 0))) { ctx->win_on = 0; return e; }   /* stage timers on a resident batch: the slice that owns the tiles */
             if (phase == 0) {
-                if ((e = slice_B(ctx, &sl[k], 3, 0))) { ctx->win_on = 0; CQ_STOP(); return e; }
+                if ((e = slice_B(ctx, &sl[k], 3, 0))) { ctx->win_on = 0; return e; }
                 if (sl[k].save_after) { k_carry_save<<<1, 32, 0, st>>>(ccarry, ecarry, (CgSavedCarry *)ctx->b_saved.p); ctx->launches++; }
             } else ctx->sl[ctx->n_sl++] = sl[k];
         }
-        if (phase == 0 && (e = ctx->cq_on ? cq_slice_queued(ctx, in, rprev, r1, i) : enqueue_d2h(ctx, in, out, rprev, r1, i))) { ctx->win_on = 0; CQ_STOP(); return e; }
+        if (phase == 0 && (e = enqueue_d2h(ctx, in, out, rprev, r1, i))) { ctx->win_on = 0; return e; }
         tprev = t1; rprev = r1; jprev = j1;
-        CG_TRACE_AT("slice enqueued (host passed its column sync)", i);
+        trace_at(trace, "slice enqueued (host passed its column sync)", i);
     }
     if (phase != 0) {                                          /* a region shard: the rest follows in cg_shard_carry / cg_shard_end */
         ctx->shard_in = in; ctx->shard_save_end = cS >= 0; ctx->shard_state = 1; ctx->shard_timed = res_mode;
         return 0;
     }
-    cudaEventRecord(ctx->ev[CG_T_D2H][1], ctx->s_d2h);
     if (cS >= 0) { k_carry_save<<<1, 32, 0, st>>>(ccarry, ecarry, (CgSavedCarry *)ctx->b_saved.p); ctx->launches++; }   /* next call starts beyond this batch's columns */
-    /* a call without any pileup column (placed-unmapped reads in a coverage gap) leaves the state it resumed from untouched */
-    if (win) ctx->have_saved = win->hi_tid >= 0 && (ctx->D.n_cols > 0 || (!win->first && ctx->have_saved));
-    e = run_finish(ctx, 0);
-    ctx->win_on = 0;
-    if (!e && ctx->cq_on) { unsigned long long cnt; memcpy(&cnt, ctx->h_dims + 22, 8); e = cq_count_known(ctx, cnt); }   /* run_finish has just synchronised */
-    if (e) { CQ_STOP(); return e; }
-    CG_TRACE_AT("finish done", 0);
-    if ((e = download_results(ctx, out, 0))) { CQ_STOP(); return e; }
-    CQ_STOP();
-    CG_TRACE_AT("compact download expanded", 0);
-    CG_CHECK(cudaStreamSynchronize(ctx->s_d2h));
-    CG_TRACE_AT("d2h drained", 0);
-    CG_CHECK(cudaStreamSynchronize(ctx->s_h2d));
-    float ms = 0;
-    if (cudaEventElapsedTime(&ms, ctx->ev[CG_T_D2H][0], ctx->ev[CG_T_D2H][1]) == cudaSuccess) ctx->ms[CG_T_D2H] = ms; else cudaGetLastError();
-    if (cudaEventElapsedTime(&ms, ctx->ev[CG_T_H2D][0], ctx->ev[CG_T_H2D][1]) == cudaSuccess) ctx->ms[CG_T_H2D] = ms; else cudaGetLastError();
-    return 0;
+    return finish_streamed(ctx, out, win, 0, trace);
 }
 
 /* ---- region shards of one contig on several devices at once (include/crumble_gpu.h) -------------------------------------------
@@ -2495,8 +2332,8 @@ extern "C" int cg_shard_carry(cg_ctx *ctx, const void *carry_in, void *carry_out
     if (ctx->shard_state != 1) return CG_ERR_STATE;
     CG_CHECK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    CgChainCarry *ccarry = (CgChainCarry *)((char *)ctx->b_scal.p + 512);
-    CgEpochCarry *ecarry = (CgEpochCarry *)((char *)ctx->b_scal.p + 640);
+    CgChainCarry *ccarry = &((CgScalars *)ctx->b_scal.p)->chain;
+    CgEpochCarry *ecarry = &((CgScalars *)ctx->b_scal.p)->epoch;
     int e;
     if (!ctx->win.first) {
         if (!carry_in) { snprintf(ctx->err, sizeof ctx->err, "this shard continues a contig: it needs the state of the shard on its left"); return CG_ERR_BAD_ARG; }
@@ -2533,44 +2370,23 @@ extern "C" int cg_shard_end(cg_ctx *ctx, cg_result *out) {
     CG_CHECK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     const cg_batch *in = ctx->shard_in;
-    CgChainCarry *ccarry = (CgChainCarry *)((char *)ctx->b_scal.p + 512);
+    CgChainCarry *imported = &((CgScalars *)ctx->b_scal.p)->chain_import;
     int e;
     ctx->shard_state = 0;
-    ctx->cq_out = out;
-    CqWorker cqw[32]; int n_cqw = 0;
-    if (ctx->cq_on && in) {
-        n_cqw = cq_threads();
-        for (int t = 0; t < n_cqw; t++) { cqw[t].ctx = ctx; cqw[t].t = t; cqw[t].nt = n_cqw; if (pthread_create(&cqw[t].th, NULL, cq_worker, &cqw[t]) != 0) { n_cqw = t; break; } }
-        if (n_cqw == 0) ctx->cq_on = 0;
-    } else ctx->cq_on = 0;
-    for (int k = ctx->shard_next; k < ctx->n_sl; k++) if ((e = slice_B(ctx, &ctx->sl[k], 1, 0))) { ctx->win_on = 0; CQ_STOP(); return e; }
+    for (int k = ctx->shard_next; k < ctx->n_sl; k++) if ((e = slice_B(ctx, &ctx->sl[k], 1, 0))) { ctx->win_on = 0; return e; }
     /* the keep window the shard on the left left open stays active from this shard's first column: the carry area now holds the state
      * after this shard's own triggers, so paint from the imported copy */
     if (!ctx->win.first && ctx->have_saved && ctx->D.n_cols > 0) {
-        CG_CHECK(cudaMemcpyAsync((char *)ctx->b_scal.p + 1600, &((CgSavedCarry *)ctx->h_carry_io)->cc, sizeof(CgChainCarry), cudaMemcpyHostToDevice, st));
-        k_paint_carry<<<1, 32, 0, st>>>(ctx->D, (const CgChainCarry *)((char *)ctx->b_scal.p + 1600), ctx->win.lo_tid, ctx->win.lo_pos); ctx->launches++;
+        CG_CHECK(cudaMemcpyAsync(imported, &((CgSavedCarry *)ctx->h_carry_io)->cc, sizeof(CgChainCarry), cudaMemcpyHostToDevice, st));
+        k_paint_carry<<<1, 32, 0, st>>>(ctx->D, imported, ctx->win.lo_tid, ctx->win.lo_pos); ctx->launches++;
     }
-    (void)ccarry;
     cudaEventRecord(ctx->ev[CG_T_D2H][0], ctx->s_d2h);
     for (int k = 0; k < ctx->n_sl; k++) {
         const CgSlice *s = &ctx->sl[k];
-        if ((e = slice_B(ctx, s, 2, ctx->shard_timed && k == ctx->n_sl - 1))) { ctx->win_on = 0; CQ_STOP(); return e; }   /* the last slice holds the rewrite */
-        if (in && s->r1 > s->r0 && (e = ctx->cq_on ? cq_slice_queued(ctx, in, s->r0, s->r1, s->chunk) : enqueue_d2h(ctx, in, out, s->r0, s->r1, s->chunk))) { ctx->win_on = 0; CQ_STOP(); return e; }
+        if ((e = slice_B(ctx, s, 2, ctx->shard_timed && k == ctx->n_sl - 1))) { ctx->win_on = 0; return e; }   /* the last slice holds the rewrite */
+        if (in && s->r1 > s->r0 && (e = enqueue_d2h(ctx, in, out, s->r0, s->r1, s->chunk))) { ctx->win_on = 0; return e; }
     }
-    cudaEventRecord(ctx->ev[CG_T_D2H][1], ctx->s_d2h);
-    ctx->have_saved = ctx->win.hi_tid >= 0 && (ctx->D.n_cols > 0 || (!ctx->win.first && ctx->have_saved));
-    e = run_finish(ctx, ctx->shard_timed);
-    ctx->win_on = 0;
-    if (!e && ctx->cq_on) { unsigned long long cnt; memcpy(&cnt, ctx->h_dims + 22, 8); e = cq_count_known(ctx, cnt); }
-    if (e) { CQ_STOP(); return e; }
-    if ((e = download_results(ctx, out, 0))) { CQ_STOP(); return e; }
-    CQ_STOP();
-    CG_CHECK(cudaStreamSynchronize(ctx->s_d2h));
-    CG_CHECK(cudaStreamSynchronize(ctx->s_h2d));
-    float ms = 0;
-    if (cudaEventElapsedTime(&ms, ctx->ev[CG_T_D2H][0], ctx->ev[CG_T_D2H][1]) == cudaSuccess) ctx->ms[CG_T_D2H] = ms; else cudaGetLastError();
-    if (cudaEventElapsedTime(&ms, ctx->ev[CG_T_H2D][0], ctx->ev[CG_T_H2D][1]) == cudaSuccess) ctx->ms[CG_T_H2D] = ms; else cudaGetLastError();
-    return 0;
+    return finish_streamed(ctx, out, &ctx->win, ctx->shard_timed, NULL);
 }
 
 extern "C" int cg_process(cg_ctx *ctx, const cg_batch *in, cg_result *out) { return process_streamed(ctx, in, out, NULL, 0); }

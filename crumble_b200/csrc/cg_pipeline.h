@@ -86,10 +86,6 @@ typedef struct CgDev {
     int32_t *n_sitem;         /* how many */
     int64_t sitem_cap;
     unsigned long long *item_bound;   /* running upper bound of the searches the columns processed so far will ask for */
-    /* compact form of the rewritten qualities (k_rewrite, when cq_mask != NULL): one bit per quality byte, set where the byte equals the
-     * dominant value cq_dom (padding counts as equal); the other bytes ("exceptions") in position order, per block of 128 records at
-     * cq_exc[cq_blk[block]], blocks in whatever order they reserved their space */
-    uint8_t *cq_mask; uint8_t *cq_exc; int64_t *cq_blk; unsigned long long *cq_count; int32_t cq_dom;
     CgWin   *twin;            /* window state after each flagged column */
     /* scalars on the device */
     unsigned long long *counters;   /* CG_N_COUNTERS */
