@@ -5,8 +5,8 @@ Host-side mirror of the reference interface for the hot path: the option block
 ``transcode`` (1336-2029) expressed as ``Crumble.process(batch)``.
 
 There is no CPU fallback: if the shared library is missing, or no CUDA device is
-usable, every compute call raises.  PyTorch is only imported by the device-resident entry
-(``device_batch``, ``Crumble.process_device``); everything else works without it.
+usable, every compute call raises.  PyTorch is only imported by the device-resident entries
+(``device_batch``, ``Crumble.process_device``, ``DeviceStream``); everything else works without it.
 """
 from __future__ import annotations
 
@@ -100,6 +100,11 @@ DEV_FIELDS = {"tid": np.int32, "pos": np.int32, "flag": np.uint16, "mapq": np.ui
 DEV_PER_RECORD = ("tid", "pos", "flag", "mapq", "l_qseq", "n_cigar")
 
 
+class StreamOut(C.Structure):
+    """cg_stream_out: what one call of a stream of device records emitted and what the context still holds (include/crumble_gpu.h)."""
+    _fields_ = [("n_records", C.c_int64), ("qual_len", C.c_int64), ("held_records", C.c_int64), ("held_qual_len", C.c_int64)]
+
+
 class BedEvent(C.Structure):
     _fields_ = [("tid", C.c_int32), ("pos", C.c_int32), ("tag", C.c_int32)]
 
@@ -136,7 +141,7 @@ _sim = None
 
 EXPORTS = [
     "cg_abi_version", "cg_device_count", "cg_create", "cg_destroy", "cg_set_params", "cg_strerror", "cg_last_error",
-    "cg_set_stream", "cg_process", "cg_process_device", "cg_process_window", "cg_upload", "cg_run", "cg_download", "cg_sync", "cg_last_ms", "cg_last_launches", "cg_last_h2d_bytes",
+    "cg_set_stream", "cg_process", "cg_process_device", "cg_stream_device", "cg_process_window", "cg_upload", "cg_run", "cg_download", "cg_sync", "cg_last_ms", "cg_last_launches", "cg_last_h2d_bytes",
     "cg_algorithmic_bytes", "cg_aligned_bases", "cg_n_columns", "cg_params_default", "cg_params_level",
     "cgb_create", "cgb_destroy", "cgb_reset", "cgb_add", "cgb_add_bam_stream", "cgb_finish", "cgb_bytes", "cgb_reserve", "cgb_pack",
     "cg_carry_export", "cg_carry_import", "cg_carry_is_neutral", "cg_batch_ends", "cg_shard_begin", "cg_shard_carry", "cg_shard_end",
@@ -174,6 +179,7 @@ def load_lib():
         getattr(lib, f).argtypes = [C.c_void_p, C.POINTER(Batch), C.POINTER(Result)]
     lib.cg_process_window.argtypes = [C.c_void_p, C.POINTER(Batch), C.POINTER(Window), C.POINTER(Result)]
     lib.cg_process_device.argtypes = [C.c_void_p, C.POINTER(DevBatch), C.c_void_p, C.POINTER(Result)]
+    lib.cg_stream_device.argtypes = [C.c_void_p, C.POINTER(DevBatch), C.c_int, C.c_void_p, C.c_int64, C.POINTER(Result), C.POINTER(StreamOut)]
     lib.cgb_reserve.argtypes = [C.c_void_p, C.c_int64, C.c_int64, C.c_int64]
     lib.cg_carry_export.argtypes = [C.c_void_p, C.c_void_p]
     lib.cg_carry_import.argtypes = [C.c_void_p, C.c_void_p]
@@ -377,31 +383,13 @@ class Crumble:
         before the call is its input and work queued after it sees the result.  Returns {"qual", "events", "counters"[, "columns"]}."""
         import torch
         dev = torch.device("cuda", self.device)
-        t = {}
-        for k, dt in DEV_FIELDS.items():
-            x = tensors.get(k)
-            if not isinstance(x, torch.Tensor):
-                raise CrumbleError(f"process_device: {k} must be a torch tensor")
-            if x.device != dev:
-                raise CrumbleError(f"process_device: {k} is on {x.device}, the context runs on {dev}")
-            if x.dtype != _torch_dtype(dt):
-                raise CrumbleError(f"process_device: {k} must be {_torch_dtype(dt)}, not {x.dtype}")
-            if x.dim() != 1 or not x.is_contiguous():
-                raise CrumbleError(f"process_device: {k} must be a contiguous 1-D tensor")
-            t[k] = x
-        n = t["tid"].numel()
-        for k in DEV_PER_RECORD:
-            if t[k].numel() != n:
-                raise CrumbleError(f"process_device: {k} has {t[k].numel()} entries, tid has {n}: one per record")
+        t, db = self._dev_batch(tensors, "process_device")
         qual_len = t["qual"].numel()
         if out is None:
             out = torch.empty(qual_len, dtype=torch.uint8, device=dev)
         elif not isinstance(out, torch.Tensor) or out.device != dev or out.dtype != torch.uint8 or out.dim() != 1 or not out.is_contiguous() \
                 or out.numel() != qual_len:
             raise CrumbleError(f"process_device: out must be a contiguous uint8 tensor of {qual_len} bytes on {dev}")
-        db = DevBatch(n_reads=n, n_cigar_total=t["cigar"].numel(), seq_len=t["seq"].numel(), qual_len=qual_len)
-        for k in DEV_FIELDS:
-            setattr(db, k, t[k].data_ptr() or None)
         self.set_stream(torch.cuda.current_stream(dev).cuda_stream)
         events_cap = max(events_cap, getattr(self, "_events_hint", 0))
         ev = np.zeros(events_cap, dtype=EVENT_DTYPE)
@@ -429,6 +417,38 @@ class Crumble:
         if want_columns:
             r["columns"] = cols[: int(res.n_columns)]
         return r
+
+    def _dev_batch(self, tensors: dict, what: str):
+        """the checked tensors of a device_batch dict and the cg_dev_batch over them"""
+        import torch
+        dev = torch.device("cuda", self.device)
+        t = {}
+        for k, dt in DEV_FIELDS.items():
+            x = tensors.get(k)
+            if not isinstance(x, torch.Tensor):
+                raise CrumbleError(f"{what}: {k} must be a torch tensor")
+            if x.device != dev:
+                raise CrumbleError(f"{what}: {k} is on {x.device}, the context runs on {dev}")
+            if x.dtype != _torch_dtype(dt):
+                raise CrumbleError(f"{what}: {k} must be {_torch_dtype(dt)}, not {x.dtype}")
+            if x.dim() != 1 or not x.is_contiguous():
+                raise CrumbleError(f"{what}: {k} must be a contiguous 1-D tensor")
+            t[k] = x
+        n = t["tid"].numel()
+        for k in DEV_PER_RECORD:
+            if t[k].numel() != n:
+                raise CrumbleError(f"{what}: {k} has {t[k].numel()} entries, tid has {n}: one per record")
+        db = DevBatch(n_reads=n, n_cigar_total=t["cigar"].numel(), seq_len=t["seq"].numel(), qual_len=t["qual"].numel())
+        for k in DEV_FIELDS:
+            setattr(db, k, t[k].data_ptr() or None)
+        return t, db
+
+    def device_stream(self) -> "DeviceStream":
+        """A coordinate-sorted stream of device records pushed in chunks of any size (cg_stream_device); see ``DeviceStream``."""
+        if getattr(self, "_stream", None) is not None and not self._stream.closed:
+            raise CrumbleError("device_stream: a stream is already open on this context")
+        self._stream = DeviceStream(self)
+        return self._stream
 
     def process_window(self, batch: Batch, window: Window, events_cap: int = 1 << 16, pinned_out=None):
         """One call of a chain (cg_process_window): ``batch`` = read halo + new records, ``window`` = the columns it owns.
@@ -529,6 +549,71 @@ class Crumble:
             self.close()
         except Exception:
             pass
+
+
+class DeviceStream:
+    """One stream of records in GPU memory on a context (cg_stream_device).  ``push(tensors)`` appends the next records of the stream (a
+    ``device_batch`` dict, or a chunk of one from ``split_device_batch``) and returns the rewritten qualities of the records that became
+    final, in stream order: {"qual": uint8 CUDA tensor, "n_records", "events", "counters", "held_records"}.  ``close()`` ends the stream
+    and returns the rest the same way.  The concatenated qualities and events and the summed counters of all calls equal one
+    ``process_device`` on the whole stream.  Every call runs on the torch stream that was current at the first push."""
+
+    def __init__(self, g: Crumble):
+        self.g = g
+        self.stream = None
+        self.held_qual_len = 0
+        self.closed = False
+
+    def push(self, tensors: dict | None, events_cap: int = 1 << 16, last: bool = False, out=None):
+        """``out``: a contiguous uint8 CUDA tensor of at least held + new quality bytes (may be ``tensors["qual"]``); by default a new one"""
+        import torch
+        g = self.g
+        if self.closed:
+            raise CrumbleError("push: the stream is closed")
+        if g.params.region_tid >= 0:
+            raise CrumbleError("push: streams and a -r region do not combine")
+        dev = torch.device("cuda", g.device)
+        cur = torch.cuda.current_stream(dev)
+        if self.stream is None:
+            g.set_stream(cur.cuda_stream)
+            self.stream = cur
+        elif cur.cuda_stream != self.stream.cuda_stream:
+            raise CrumbleError("push: the current torch stream is not the one the stream started on")
+        if tensors is None:
+            db, new_len, keep = None, 0, None
+        else:
+            keep, db = g._dev_batch(tensors, "push")
+            new_len = int(db.qual_len)
+        cap = self.held_qual_len + new_len
+        if out is None:
+            out = torch.empty(max(cap, 1), dtype=torch.uint8, device=dev)
+        elif not isinstance(out, torch.Tensor) or out.device != dev or out.dtype != torch.uint8 or out.dim() != 1 or not out.is_contiguous() \
+                or out.numel() < cap:
+            raise CrumbleError(f"push: out must be a contiguous uint8 tensor of at least {cap} bytes on {dev}")
+        events_cap = max(events_cap, 1)
+        ev = np.zeros(events_cap, dtype=EVENT_DTYPE)
+        res = Result(events=ev.ctypes.data_as(C.POINTER(BedEvent)), events_cap=events_cap)
+        so = StreamOut()
+        code = g.lib.cg_stream_device(g.h, C.byref(db) if db is not None else None, 1 if last else 0, out.data_ptr(), out.numel(), C.byref(res), C.byref(so))
+        if code != 0:
+            self.closed = True                             # what this class checks up front cannot fail in C: the rest closes the stream
+            g._stream = None
+        _check(g.lib, code, g.h)
+        if res.n_events > events_cap:                      # the chain's state has moved on: fetch the list again, do not redo
+            ev = np.zeros(int(res.n_events), dtype=EVENT_DTYPE)
+            res2 = Result(events=ev.ctypes.data_as(C.POINTER(BedEvent)), events_cap=int(res.n_events))
+            _check(g.lib, g.lib.cg_download(g.h, C.byref(res2)), g.h)
+            res = res2
+        self.held_qual_len = int(so.held_qual_len)
+        if last:
+            self.closed = True
+            g._stream = None
+        return {"qual": out[: int(so.qual_len)], "n_records": int(so.n_records), "events": ev[: int(res.n_events)],
+                "counters": {k: int(res.counters[i]) for i, k in enumerate(COUNTER_NAMES)}, "held_records": int(so.held_records)}
+
+    def close(self, events_cap: int = 1 << 16):
+        """the last call: everything the context still holds comes out, and the stream ends"""
+        return self.push(None, events_cap=events_cap, last=True)
 
 
 class MultiCrumble:
@@ -681,6 +766,30 @@ def device_batch(batch: Batch, device) -> dict:
     import torch
     dev = torch.device("cuda", device) if isinstance(device, int) else torch.device(device)
     return {k: torch.from_numpy(v).to(dev) for k, v in concat_fields(batch).items()}
+
+
+def split_device_batch(tensors: dict, n_per_chunk: int | None = None, cuts=None) -> list:
+    """Cut a ``device_batch`` dict (torch tensors, or numpy arrays of the same layout) into consecutive chunk dicts, every
+    ``n_per_chunk`` records or before each record index in ``cuts``.  The chunks are views of the input."""
+    n = int(tensors["tid"].shape[0])
+    if cuts is None:
+        if not n_per_chunk or n_per_chunk < 1:
+            raise CrumbleError("split_device_batch: give n_per_chunk >= 1 or cuts")
+        cuts = range(n_per_chunk, n, n_per_chunk)
+    b = [0] + sorted(int(c) for c in cuts) + [n]
+    if b[1] < 0 or b[-2] > n:
+        raise CrumbleError(f"split_device_batch: cuts must lie in [0, {n}]")
+    host = lambda x: np.asarray(x.cpu()) if hasattr(x, "cpu") else np.asarray(x)
+    lq, nc = host(tensors["l_qseq"]).astype(np.int64), host(tensors["n_cigar"]).astype(np.int64)
+    q = np.concatenate([[0], np.cumsum(lq)]); s = np.concatenate([[0], np.cumsum((lq + 1) // 2)]); c = np.concatenate([[0], np.cumsum(nc)])
+    chunks = []
+    for i0, i1 in zip(b[:-1], b[1:]):
+        d = {k: tensors[k][i0:i1] for k in DEV_PER_RECORD}
+        d["cigar"] = tensors["cigar"][int(c[i0]):int(c[i1])]
+        d["seq"] = tensors["seq"][int(s[i0]):int(s[i1])]
+        d["qual"] = tensors["qual"][int(q[i0]):int(q[i1])]
+        chunks.append(d)
+    return chunks
 
 
 def plan_region_shards(batch: Batch, n_shards: int):

@@ -1282,7 +1282,13 @@ struct CgScalars {
     int64_t bounds[3 * CG_MAX_CHUNKS];                     /* k_bounds */
     char pad_bounds[1600 - 768 - 8 * 3 * CG_MAX_CHUNKS];
     CgChainCarry chain_import;    /* cg_shard_end paints from the carry the shard imported */
-    char pad_end[2048 - 1600 - sizeof(CgChainCarry)];
+    char pad_import[1664 - 1600 - sizeof(CgChainCarry)];
+    struct CgStreamScal {         /* cg_stream_device: the cut of the call and what it holds back, read at its one synchronisation */
+        CgStreamRed red;
+        CgStreamCut cut;
+        int64_t held_n, held_padded, held_cig, held_qual, held_seq;   /* totals of the keep-flag scans */
+    } stream;
+    char pad_end[2048 - 1664 - sizeof(CgStreamScal)];
 };
 #define CG_SCAL_AT(f, off) static_assert(offsetof(CgScalars, f) == (off), "scalar block: " #f " must stay at byte " #off)
 CG_SCAL_AT(h.n_pile, 0); CG_SCAL_AT(h.n_cols, 4); CG_SCAL_AT(h.n_islands, 8); CG_SCAL_AT(h.n_flagged, 12);
@@ -1290,7 +1296,7 @@ CG_SCAL_AT(h.maxdepth, 16); CG_SCAL_AT(h.err, 20); CG_SCAL_AT(h.n_events, 24); C
 CG_SCAL_AT(h.window_max, 36); CG_SCAL_AT(h.n_sitem, 40); CG_SCAL_AT(h.next_col, 44); CG_SCAL_AT(h.qual_total, 48);
 CG_SCAL_AT(h.cigar_total, 56); CG_SCAL_AT(h.cell_groups, 64); CG_SCAL_AT(h.slice.tile_counter, 72); CG_SCAL_AT(h.slice.item_bound, 80);
 CG_SCAL_AT(n_glist, 96); CG_SCAL_AT(counters, 128); CG_SCAL_AT(chain, 512); CG_SCAL_AT(epoch, 640); CG_SCAL_AT(bounds, 768);
-CG_SCAL_AT(chain_import, 1600);
+CG_SCAL_AT(chain_import, 1600); CG_SCAL_AT(stream, 1664);
 #undef CG_SCAL_AT
 static_assert(sizeof(CgScalHead) == 96, "the mirrored head is 24 int32 slots");
 static_assert(sizeof(CgScalars) == 2048, "scalar block size");
@@ -1306,6 +1312,12 @@ struct cg_ctx {
     dbuf b_aggr, b_scal, b_scratch, b_epoch, b_events, b_chain, b_items, b_bed, b_bedpm, b_crec, b_cells, b_seq2, b_qualp, b_exc;
     dbuf b_truns, b_pabs, b_pd8, b_lq8, b_nc8, b_cigx, b_lqd, b_xoff, b_absS;   /* compact planes of the per-record arrays and what their expansion needs */
     dbuf b_qsrc, b_ssrc, b_dvsum;  /* cg_process_device: where each record starts in the caller's arrays, the sums checked on the host */
+    /* cg_stream_device: the held store (records kept for later calls, in the padded working layout) and the keep-flag scans that fill it */
+    dbuf b_htid, b_hpos, b_hflag, b_hmapq, b_hlq, b_hnc, b_hcig, b_hqual, b_hseq, b_keep, b_kidx, b_koff, b_kcig;
+    int st_open, st_unplaced, st_has_key; uint64_t st_kmax;            /* an open stream; the sort order across its chunks */
+    int64_t st_n, st_e0, st_padded, st_cig, st_qual, st_seq;          /* held records (the first st_e0 already emitted) and their sizes */
+    cg_window st_win;                                                  /* first / lo_tid / lo_pos / cnt_pos of the next call */
+    CgScalars::CgStreamScal *h_stream;                                 /* pinned */
     int has_meta; int64_t n_truns, n_pabs, n_cigx;
     int generic;                  /* cg_params_generic(): column and rewrite stages through the plain bodies */
     /* host mirrors */
@@ -1328,6 +1340,13 @@ struct cg_ctx {
     float ms[CG_N_TIMERS];
     int64_t launches;
 };
+
+/* while a stream is open (cg_stream_device) the working buffers, the window state and the stream belong to it */
+static int stream_busy(cg_ctx *ctx) {
+    if (!ctx->st_open) return 0;
+    snprintf(ctx->err, sizeof ctx->err, "a stream is open on this context: finish it with cg_stream_device(last = 1) first");
+    return CG_ERR_STATE;
+}
 
 static int ensure(cg_ctx *ctx, dbuf *b, size_t bytes) {
     if (bytes <= b->cap) return 0;
@@ -1370,6 +1389,7 @@ static void install_hooks(void) {
 extern "C" int cg_enable_pinned(void) { install_hooks(); return cg_pinned_alloc_hook != NULL; }
 
 extern "C" int cg_set_params(cg_ctx *ctx, const cg_params *p) {
+    if (stream_busy(ctx)) return CG_ERR_STATE;
     const char *why = NULL;
     int e = cg_params_check(p, &why);
     if (e) { snprintf(ctx->err, sizeof ctx->err, "not implemented on the device path: %s", why); return e; }
@@ -1425,12 +1445,14 @@ extern "C" void cg_destroy(cg_ctx *ctx) {
         &ctx->b_pmax, &ctx->b_orig, &ctx->b_rbf, &ctx->b_glist, &ctx->b_tlo, &ctx->b_tstart, &ctx->b_isl, &ctx->b_cb, &ctx->b_ev, &ctx->b_depth, &ctx->b_dump,
         &ctx->b_dsum, &ctx->b_csum, &ctx->b_fcol, &ctx->b_trig, &ctx->b_twin, &ctx->b_aggr, &ctx->b_scal, &ctx->b_scratch, &ctx->b_epoch, &ctx->b_events, &ctx->b_chain, &ctx->b_items, &ctx->b_bed, &ctx->b_bedpm, &ctx->b_saved, &ctx->b_crec, &ctx->b_cells, &ctx->b_seq2, &ctx->b_qualp, &ctx->b_exc,
         &ctx->b_truns, &ctx->b_pabs, &ctx->b_pd8, &ctx->b_lq8, &ctx->b_nc8, &ctx->b_cigx, &ctx->b_lqd, &ctx->b_xoff, &ctx->b_absS,
-        &ctx->b_qsrc, &ctx->b_ssrc, &ctx->b_dvsum };
+        &ctx->b_qsrc, &ctx->b_ssrc, &ctx->b_dvsum, &ctx->b_htid, &ctx->b_hpos, &ctx->b_hflag, &ctx->b_hmapq, &ctx->b_hlq, &ctx->b_hnc,
+        &ctx->b_hcig, &ctx->b_hqual, &ctx->b_hseq, &ctx->b_keep, &ctx->b_kidx, &ctx->b_koff, &ctx->b_kcig };
     for (size_t i = 0; i < sizeof(all) / sizeof(all[0]); i++) if (all[i]->p) cudaFree(all[i]->p);
     if (ctx->dT) cudaFree(ctx->dT);
     if (ctx->h_dims) cudaFreeHost(ctx->h_dims);
     if (ctx->h_counters) cudaFreeHost(ctx->h_counters);
     if (ctx->h_carry_io) cudaFreeHost(ctx->h_carry_io);
+    if (ctx->h_stream) cudaFreeHost(ctx->h_stream);
     for (int i = 0; i < CG_N_TIMERS; i++) for (int k = 0; k < 2; k++) if (ctx->ev[i][k]) cudaEventDestroy(ctx->ev[i][k]);
     if (ctx->s_h2d) { cudaStreamDestroy(ctx->s_h2d); cudaStreamDestroy(ctx->s_d2h); for (int i = 0; i < 32; i++) { cudaEventDestroy(ctx->ev_up[i]); cudaEventDestroy(ctx->ev_done[i]); } cudaEventDestroy(ctx->ev_misc); }
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
@@ -1440,6 +1462,7 @@ extern "C" void cg_destroy(cg_ctx *ctx) {
 
 extern "C" const char *cg_last_error(const cg_ctx *ctx) { return ctx ? ctx->err : "no context"; }
 extern "C" int cg_set_stream(cg_ctx *ctx, void *s) {
+    if (stream_busy(ctx)) return CG_ERR_STATE;
     if (ctx->own_stream && ctx->stream) cudaStreamDestroy(ctx->stream);
     ctx->stream = (cudaStream_t)s; ctx->own_stream = 0;
     return 0;
@@ -1596,6 +1619,7 @@ static int expand_bases(cg_ctx *ctx, const cg_batch *in, int64_t b0, int64_t b1,
 }
 
 extern "C" int cg_upload(cg_ctx *ctx, const cg_batch *in) {
+    if (stream_busy(ctx)) return CG_ERR_STATE;
     CG_CHECK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     ctx->resident = 0; ctx->win_on = 0;
@@ -1979,7 +2003,7 @@ static int run_finish(cg_ctx *ctx, int timed) {
 }
 
 extern "C" int cg_run(cg_ctx *ctx) {
-    if (!ctx->resident) return CG_ERR_STATE;
+    if (!ctx->resident || stream_busy(ctx)) return CG_ERR_STATE;
     CG_CHECK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     CgBounds B; memset(&B, 0, sizeof B); B.n = 1; B.rb[0] = ctx->D.n_reads;
@@ -2070,42 +2094,66 @@ static int dev_ptr_check(cg_ctx *ctx, const void *p, int64_t count, const char *
     return CG_ERR_BAD_ARG;
 }
 
-extern "C" int cg_process_device(cg_ctx *ctx, const cg_dev_batch *in, uint8_t *qual_out, cg_result *out) {
-    if (!ctx) return CG_ERR_BAD_ARG;
-    if (!in || !out) { snprintf(ctx->err, sizeof ctx->err, "cg_process_device: no batch or no result"); return CG_ERR_BAD_ARG; }
-    CG_CHECK(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
+/* what cg_process_device and cg_stream_device reject before anything is enqueued; n_total / cig_total / q_total: the working batch */
+static int dev_check(cg_ctx *ctx, const cg_dev_batch *in, const uint8_t *qual_out, int64_t qual_cnt, const cg_result *out, int64_t n_total, int64_t cig_total, int64_t q_total) {
     const int64_t n = in->n_reads;
-    int e;
     if (n < 0 || in->n_cigar_total < 0 || in->seq_len < 0 || in->qual_len < 0) {
         snprintf(ctx->err, sizeof ctx->err, "cg_dev_batch: negative count (n_reads %lld, n_cigar_total %lld, seq_len %lld, qual_len %lld)",
                  (long long)n, (long long)in->n_cigar_total, (long long)in->seq_len, (long long)in->qual_len);
         return CG_ERR_BAD_ARG;
     }
-    if (out->qual_out || out->qual_head) { snprintf(ctx->err, sizeof ctx->err, "cg_process_device: the qualities go to qual_out; out->qual_out and out->qual_head must be NULL"); return CG_ERR_BAD_ARG; }
-    if (n > 0x7fffff00LL || in->n_cigar_total > 0x7fffff00LL || in->qual_len + 8 * n >= (1LL << 35)) { snprintf(ctx->err, sizeof ctx->err, "batch too large: split it"); return CG_ERR_BAD_ARG; }
+    if (out->qual_out || out->qual_head) { snprintf(ctx->err, sizeof ctx->err, "the qualities go to qual_out; out->qual_out and out->qual_head must be NULL"); return CG_ERR_BAD_ARG; }
+    if (n_total > 0x7fffff00LL || cig_total > 0x7fffff00LL || q_total + 8 * n_total >= (1LL << 35)) { snprintf(ctx->err, sizeof ctx->err, "batch too large: split it"); return CG_ERR_BAD_ARG; }
+    int e;
     if ((e = dev_ptr_check(ctx, in->tid, n, "tid")) || (e = dev_ptr_check(ctx, in->pos, n, "pos")) || (e = dev_ptr_check(ctx, in->flag, n, "flag")) ||
         (e = dev_ptr_check(ctx, in->mapq, n, "mapq")) || (e = dev_ptr_check(ctx, in->l_qseq, n, "l_qseq")) || (e = dev_ptr_check(ctx, in->n_cigar, n, "n_cigar")) ||
         (e = dev_ptr_check(ctx, in->cigar, in->n_cigar_total, "cigar")) || (e = dev_ptr_check(ctx, in->seq, in->seq_len, "seq")) ||
-        (e = dev_ptr_check(ctx, in->qual, in->qual_len, "qual")) || (e = dev_ptr_check(ctx, qual_out, in->qual_len, "qual_out"))) return e;
-    ctx->resident = 0; ctx->win_on = 0;
-    ctx->dump_columns = out->columns != NULL;
-    /* working buffers sized for the padded layout: the padded lengths sum to at most qual_len + 7 per record */
-    cg_batch hb; memset(&hb, 0, sizeof hb);
-    hb.n_reads = n; hb.n_cigar_total = in->n_cigar_total; hb.qual_bytes = in->qual_len + 7 * n; hb.seq_bytes = (hb.qual_bytes + 1) / 2; hb.packed = 1;
+        (e = dev_ptr_check(ctx, in->qual, in->qual_len, "qual")) || (e = dev_ptr_check(ctx, qual_out, qual_cnt, "qual_out"))) return e;
+    return 0;
+}
+
+/* The records held for a stream (none for cg_process_device) followed by `in`, as one packed working batch: per-record arrays and CIGARs
+ * copied device to device, the running sums of the padded lengths, n_cigar, l_qseq, (l_qseq + 1) / 2 and the count of negative lengths.
+ * before_sync() enqueues whatever else must come back at the one synchronisation; then the sums are checked.  The held records' bytes are
+ * already in the padded layout and go to the front of the working arrays; `in`'s go through k_ingest (dev_ingest) afterwards. */
+template <class F>
+static int dev_stage(cg_ctx *ctx, const cg_dev_batch *in, F before_sync) {
+    cudaStream_t st = ctx->stream;
+    const int64_t nh = ctx->st_n, ni = in->n_reads, n = nh + ni;
+    int e;
+    cg_batch hb; memset(&hb, 0, sizeof hb);                     /* the padded lengths of `in` sum to at most qual_len + 7 per record */
+    hb.n_reads = n; hb.n_cigar_total = ctx->st_cig + in->n_cigar_total; hb.qual_bytes = ctx->st_padded + in->qual_len + 7 * ni;
+    hb.seq_bytes = (hb.qual_bytes + 1) / 2; hb.packed = 1;
     if ((e = alloc_inputs(ctx, &hb))) return e;
-    if ((e = ensure(ctx, &ctx->b_qsrc, ((size_t)n + 1) * 8)) || (e = ensure(ctx, &ctx->b_ssrc, ((size_t)n + 1) * 8)) || (e = ensure(ctx, &ctx->b_dvsum, 64))) return e;
+    if ((e = ensure(ctx, &ctx->b_qsrc, ((size_t)n + 1) * 8)) || (e = ensure(ctx, &ctx->b_ssrc, ((size_t)n + 1) * 8)) || (e = ensure(ctx, &ctx->b_dvsum, 64)) ||
+        (e = ensure(ctx, &ctx->b_scal, sizeof(CgScalars))) || (e = ensure(ctx, &ctx->b_rspan, ((size_t)n + 1) * 4))) return e;
     CgDev *D = &ctx->D;
-    int64_t padded = 0;
+    D->rspan = (int32_t *)ctx->b_rspan.p; D->err = &((CgScalars *)ctx->b_scal.p)->h.err;
+    int64_t h[5] = { 0, 0, 0, 0, 0 };                            /* [0] padded lengths [1] n_cigar [2] l_qseq [3] (l_qseq + 1) / 2 [4] negative l_qseq */
     if (n > 0) {
-        CG_CHECK(cudaMemcpyAsync(ctx->b_tid.p, in->tid, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
-        CG_CHECK(cudaMemcpyAsync(ctx->b_pos.p, in->pos, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
-        CG_CHECK(cudaMemcpyAsync(ctx->b_flag.p, in->flag, (size_t)n * 2, cudaMemcpyDeviceToDevice, st));
-        CG_CHECK(cudaMemcpyAsync(ctx->b_mapq.p, in->mapq, (size_t)n, cudaMemcpyDeviceToDevice, st));
-        CG_CHECK(cudaMemcpyAsync(ctx->b_lq.p, in->l_qseq, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
-        CG_CHECK(cudaMemcpyAsync(ctx->b_nc.p, in->n_cigar, (size_t)n * 2, cudaMemcpyDeviceToDevice, st));
-        if (in->n_cigar_total) CG_CHECK(cudaMemcpyAsync(ctx->b_cigar.p, in->cigar, (size_t)in->n_cigar_total * 4, cudaMemcpyDeviceToDevice, st));
-        int64_t *sums = (int64_t *)ctx->b_dvsum.p;               /* [0] padded lengths [1] n_cigar [2] l_qseq [3] (l_qseq + 1) / 2 [4] negative l_qseq */
+        if (nh > 0) {
+            CG_CHECK(cudaMemcpyAsync(ctx->b_tid.p, ctx->b_htid.p, (size_t)nh * 4, cudaMemcpyDeviceToDevice, st));
+            CG_CHECK(cudaMemcpyAsync(ctx->b_pos.p, ctx->b_hpos.p, (size_t)nh * 4, cudaMemcpyDeviceToDevice, st));
+            CG_CHECK(cudaMemcpyAsync(ctx->b_flag.p, ctx->b_hflag.p, (size_t)nh * 2, cudaMemcpyDeviceToDevice, st));
+            CG_CHECK(cudaMemcpyAsync(ctx->b_mapq.p, ctx->b_hmapq.p, (size_t)nh, cudaMemcpyDeviceToDevice, st));
+            CG_CHECK(cudaMemcpyAsync(ctx->b_lq.p, ctx->b_hlq.p, (size_t)nh * 4, cudaMemcpyDeviceToDevice, st));
+            CG_CHECK(cudaMemcpyAsync(ctx->b_nc.p, ctx->b_hnc.p, (size_t)nh * 2, cudaMemcpyDeviceToDevice, st));
+            if (ctx->st_cig) CG_CHECK(cudaMemcpyAsync(ctx->b_cigar.p, ctx->b_hcig.p, (size_t)ctx->st_cig * 4, cudaMemcpyDeviceToDevice, st));
+            if (ctx->st_padded) {
+                CG_CHECK(cudaMemcpyAsync((char *)ctx->b_qual.p + CG_FRONT_PAD, ctx->b_hqual.p, (size_t)ctx->st_padded, cudaMemcpyDeviceToDevice, st));
+                CG_CHECK(cudaMemcpyAsync((char *)ctx->b_seq.p + CG_FRONT_PAD, ctx->b_hseq.p, (size_t)ctx->st_padded / 2, cudaMemcpyDeviceToDevice, st));
+            }
+        }
+        if (ni > 0) {
+            CG_CHECK(cudaMemcpyAsync((int32_t *)ctx->b_tid.p + nh, in->tid, (size_t)ni * 4, cudaMemcpyDeviceToDevice, st));
+            CG_CHECK(cudaMemcpyAsync((int32_t *)ctx->b_pos.p + nh, in->pos, (size_t)ni * 4, cudaMemcpyDeviceToDevice, st));
+            CG_CHECK(cudaMemcpyAsync((uint16_t *)ctx->b_flag.p + nh, in->flag, (size_t)ni * 2, cudaMemcpyDeviceToDevice, st));
+            CG_CHECK(cudaMemcpyAsync((uint8_t *)ctx->b_mapq.p + nh, in->mapq, (size_t)ni, cudaMemcpyDeviceToDevice, st));
+            CG_CHECK(cudaMemcpyAsync((int32_t *)ctx->b_lq.p + nh, in->l_qseq, (size_t)ni * 4, cudaMemcpyDeviceToDevice, st));
+            CG_CHECK(cudaMemcpyAsync((uint16_t *)ctx->b_nc.p + nh, in->n_cigar, (size_t)ni * 2, cudaMemcpyDeviceToDevice, st));
+            if (in->n_cigar_total) CG_CHECK(cudaMemcpyAsync((uint32_t *)ctx->b_cigar.p + ctx->st_cig, in->cigar, (size_t)in->n_cigar_total * 4, cudaMemcpyDeviceToDevice, st));
+        }
+        int64_t *sums = (int64_t *)ctx->b_dvsum.p;
         LdPad8 lp = { D->l_qseq }; StExcl64 so = { (int64_t *)ctx->b_off.p };
         LdNCig64 ln = { D->n_cigar }; StExcl32of64 sc = { (int32_t *)ctx->b_coff.p };
         LdLen ll = { D->l_qseq }; StExcl64 sq = { (int64_t *)ctx->b_qsrc.p };
@@ -2114,42 +2162,115 @@ extern "C" int cg_process_device(cg_ctx *ctx, const cg_dev_batch *in, uint8_t *q
         if ((e = run_scan<int64_t, OpSum>(ctx, lp, so, n, (int64_t)0, sums + 0)) || (e = run_scan<int64_t, OpSum>(ctx, ln, sc, n, (int64_t)0, sums + 1)) ||
             (e = run_scan<int64_t, OpSum>(ctx, ll, sq, n, (int64_t)0, sums + 2)) || (e = run_scan<int64_t, OpSum>(ctx, lh, ss, n, (int64_t)0, sums + 3)) ||
             (e = run_scan<int64_t, OpSum>(ctx, lneg, none, n, (int64_t)0, sums + 4))) return e;
-        int64_t h[5];
+        if ((e = before_sync(sums))) return e;
         CG_CHECK(cudaMemcpyAsync(h, sums, sizeof h, cudaMemcpyDeviceToHost, st));
         CG_CHECK(cudaStreamSynchronize(st));
         if (h[4]) { snprintf(ctx->err, sizeof ctx->err, "cg_dev_batch: %lld records have a negative l_qseq", (long long)h[4]); return CG_ERR_BAD_ARG; }
-        if (h[2] != in->qual_len || h[3] != in->seq_len || h[1] != in->n_cigar_total) {
+        if (h[2] != ctx->st_qual + in->qual_len || h[3] != ctx->st_seq + in->seq_len || h[1] != ctx->st_cig + in->n_cigar_total) {
             snprintf(ctx->err, sizeof ctx->err, "cg_dev_batch: the records hold %lld quality bytes (qual_len %lld), %lld sequence bytes (seq_len %lld), %lld CIGAR operations (n_cigar_total %lld)",
-                     (long long)h[2], (long long)in->qual_len, (long long)h[3], (long long)in->seq_len, (long long)h[1], (long long)in->n_cigar_total);
+                     (long long)(h[2] - ctx->st_qual), (long long)in->qual_len, (long long)(h[3] - ctx->st_seq), (long long)in->seq_len,
+                     (long long)(h[1] - ctx->st_cig), (long long)in->n_cigar_total);
             return CG_ERR_BAD_ARG;
         }
-        padded = h[0];
     }
-    ctx->qual_bytes = padded; ctx->offsets_ready = 1;
-    const unsigned io_blocks = (unsigned)nblk(n * 32, IO_THREADS);
+    ctx->qual_bytes = h[0]; ctx->offsets_ready = 1;
+    return 0;
+}
+
+/* `in`'s qualities and sequences into the padded working layout, behind the held records */
+static int dev_ingest(cg_ctx *ctx, const cg_dev_batch *in) {
+    const int64_t nh = ctx->st_n, ni = in->n_reads;
+    if (ni <= 0) return 0;
+    const CgDev *D = &ctx->D;
+    const CgIngest I = { D->l_qseq + nh, D->off + nh, (const int64_t *)ctx->b_qsrc.p + nh, (const int64_t *)ctx->b_ssrc.p + nh, in->qual, in->seq,
+                         (uint8_t *)ctx->b_qual.p + CG_FRONT_PAD, (uint8_t *)ctx->b_seq.p + CG_FRONT_PAD, ctx->st_qual, ctx->st_seq };
+    k_ingest<<<(unsigned)nblk(ni * 32, IO_THREADS), IO_THREADS, 0, ctx->stream>>>(I, ni);
+    CG_CHECK(cudaGetLastError());
+    return 0;
+}
+
+/* the rewritten qualities of working records [r0, r1) to qual_out, which starts at record r0 */
+static int dev_emit(cg_ctx *ctx, int64_t r0, int64_t r1, int64_t qbase, uint8_t *qual_out) {
+    if (r1 <= r0) return 0;
+    const CgDev *D = &ctx->D;
+    const CgEmit E = { D->l_qseq + r0, D->off + r0, (const int64_t *)ctx->b_qsrc.p + r0, (const uint8_t *)ctx->b_qout.p, qual_out, qbase };
+    k_emit<<<(unsigned)nblk((r1 - r0) * 32, IO_THREADS), IO_THREADS, 0, ctx->stream>>>(E, r1 - r0);
+    ctx->launches++;
+    CG_CHECK(cudaGetLastError());
+    return 0;
+}
+
+extern "C" int cg_process_device(cg_ctx *ctx, const cg_dev_batch *in, uint8_t *qual_out, cg_result *out) {
+    if (!ctx) return CG_ERR_BAD_ARG;
+    if (stream_busy(ctx)) return CG_ERR_STATE;
+    if (!in || !out) { snprintf(ctx->err, sizeof ctx->err, "cg_process_device: no batch or no result"); return CG_ERR_BAD_ARG; }
+    CG_CHECK(cudaSetDevice(ctx->device));
+    int e;
+    if ((e = dev_check(ctx, in, qual_out, in->qual_len, out, in->n_reads, in->n_cigar_total, in->qual_len))) return e;
+    ctx->resident = 0; ctx->win_on = 0;
+    ctx->dump_columns = out->columns != NULL;
+    if ((e = dev_stage(ctx, in, [](int64_t *) { return 0; }))) return e;
+    const int64_t n = in->n_reads;
+    cudaStream_t st = ctx->stream;
     T0(CG_T_H2D);
-    if (n > 0) {
-        const CgIngest I = { D->l_qseq, D->off, (const int64_t *)ctx->b_qsrc.p, (const int64_t *)ctx->b_ssrc.p, in->qual, in->seq,
-                             (uint8_t *)ctx->b_qual.p + CG_FRONT_PAD, (uint8_t *)ctx->b_seq.p + CG_FRONT_PAD };
-        k_ingest<<<io_blocks, IO_THREADS, 0, st>>>(I, n);
-        CG_CHECK(cudaGetLastError());
-    }
+    if ((e = dev_ingest(ctx, in))) return e;
     T1(CG_T_H2D);
     ctx->resident = 1;
     if ((e = cg_run(ctx))) return e;
     T0(CG_T_D2H);
-    if (n > 0 && in->qual_len > 0) {
-        const CgEmit E = { D->l_qseq, D->off, (const int64_t *)ctx->b_qsrc.p, (const uint8_t *)ctx->b_qout.p, qual_out };
-        k_emit<<<io_blocks, IO_THREADS, 0, st>>>(E, n);
-        ctx->launches++;
-        CG_CHECK(cudaGetLastError());
-    }
+    if (in->qual_len > 0 && (e = dev_emit(ctx, 0, n, 0, qual_out))) return e;
     T1(CG_T_D2H);
     if ((e = download_results(ctx, out, 0))) return e;          /* events, counters, column dump; synchronises the stream */
     read_copy_timers(ctx);
     ctx->h2d_bytes = 0;
     return 0;
 }
+
+/* ---- streams (cg_stream_device) ----------------------------------------------------------------------------------------------------
+ * k_stream_plan reduces the cut quantities of the working batch (one thread per record, warp reductions, one atomic per warp and field),
+ * k_stream_cut turns them into the cut, k_stream_keep flags the records held for later calls, and three scans over the flag give where
+ * k_retain puts each of them in the held store.  All of it before the call's one synchronisation. */
+__global__ void k_stream_init(CgStreamRed *red) { cg_stream_red_init(red); }
+__global__ void __launch_bounds__(256) k_stream_plan(const __grid_constant__ CgDev D, int64_t n, int64_t n_held, int64_t e0, CgStreamRed *red) {
+    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    CgStreamRed c;
+    if (r < n) c = cg_stream_plan_item(&D, r, n, n_held, e0); else cg_stream_red_init(&c);
+    const unsigned all = 0xffffffffu;
+    c.mmax = __reduce_max_sync(all, c.mmax); c.mtid = __reduce_max_sync(all, c.mtid);
+    c.smin = __reduce_min_sync(all, c.smin); c.fmin = __reduce_min_sync(all, c.fmin);
+    c.unplaced = __reduce_or_sync(all, (unsigned)c.unplaced);
+    for (int o = 16; o > 0; o >>= 1) {
+        const uint64_t a = __shfl_xor_sync(all, c.kmin, o), b = __shfl_xor_sync(all, c.kmax, o);
+        if (a < c.kmin) c.kmin = a;
+        if (b > c.kmax) c.kmax = b;
+    }
+    if ((threadIdx.x & 31) == 0) {
+        if (c.mmax >= 0) atomicMax(&red->mmax, c.mmax);
+        if (c.mtid >= 0) atomicMax(&red->mtid, c.mtid);
+        if (c.smin != 0x7fffffff) atomicMin(&red->smin, c.smin);
+        if (c.fmin != 0x7fffffff) atomicMin(&red->fmin, c.fmin);
+        if (c.kmin <= c.kmax) { atomicMin((unsigned long long *)&red->kmin, (unsigned long long)c.kmin); atomicMax((unsigned long long *)&red->kmax, (unsigned long long)c.kmax); }
+        if (c.unplaced) atomicOr(&red->unplaced, 1);
+    }
+}
+__global__ void k_stream_cut(const __grid_constant__ CgDev D, const CgStreamRed *red, CgStreamCut *cut, int64_t n, int64_t e0, int last, const int64_t *qsrc, const int64_t *q_total) {
+    *cut = cg_stream_cut(&D, red, n, e0, last, qsrc, *q_total);
+}
+__global__ void __launch_bounds__(256) k_stream_keep(const __grid_constant__ CgDev D, const CgStreamCut *cut, uint8_t *keep, int64_t n) {
+    const int64_t r = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (r < n) keep[r] = (uint8_t)cg_stream_keep(&D, r, cut);
+}
+__global__ void __launch_bounds__(IO_THREADS) k_retain(const __grid_constant__ CgRetain K, const uint8_t *__restrict__ keep, int64_t n) {
+    const int64_t r = ((int64_t)blockIdx.x * IO_THREADS + threadIdx.x) >> 5;
+    if (r >= n || !keep[r]) return;
+    const int ni = cg_retain_items(&K, r);
+    for (int j = threadIdx.x & 31; j < ni; j += 32) cg_retain_item(&K, r, j);
+}
+struct LdKeep { const uint8_t *keep; __device__ int64_t operator()(int64_t i) const { return keep[i]; } };
+struct LdKeepPad { const uint8_t *keep; const int32_t *lq; __device__ int64_t operator()(int64_t i) const { return keep[i] ? (((int64_t)lq[i] + 7) & ~(int64_t)7) : 0; } };
+struct LdKeepCig { const uint8_t *keep; const uint16_t *nc; __device__ int64_t operator()(int64_t i) const { return keep[i] ? (int64_t)nc[i] : 0; } };
+struct LdKeepLen { const uint8_t *keep; const int32_t *lq; __device__ int64_t operator()(int64_t i) const { return keep[i] ? (int64_t)lq[i] : 0; } };
+struct LdKeepHalf { const uint8_t *keep; const int32_t *lq; __device__ int64_t operator()(int64_t i) const { return keep[i] ? ((int64_t)lq[i] + 1) >> 1 : 0; } };
 
 /* the qualities of records [r0, r1) go home on the download stream once everything queued on the compute stream so far is done;
  * bytes below out->head_bytes (a region shard's read halo) go to out->qual_head instead of out->qual_out */
@@ -2202,8 +2323,10 @@ static int process_streamed(cg_ctx *ctx, const cg_batch *in, cg_result *out, con
     CG_CHECK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     int e;
-    const int res_mode = in == NULL;                           /* a region shard on the batch cg_upload left on the device (timing the chain alone) */
-    if (res_mode && (!ctx->resident || phase != 1)) return CG_ERR_STATE;
+    /* a resident batch: a region shard on the batch cg_upload left on the device (timing the chain alone, phase 1), or one call of a
+     * stream on the batch cg_stream_device ingested (phase 0 with a window; its qualities stay on the device) */
+    const int res_mode = in == NULL;
+    if (res_mode && !ctx->resident) return CG_ERR_STATE;
     ctx->win_on = 0; ctx->n_sl = 0; ctx->shard_state = 0;
     ctx->dump_columns = out->columns != NULL;
     if (!res_mode) { ctx->resident = 0; if ((e = alloc_inputs(ctx, in))) return e; }
@@ -2302,7 +2425,7 @@ static int process_streamed(cg_ctx *ctx, const cg_batch *in, cg_result *out, con
                 if (sl[k].save_after) { k_carry_save<<<1, 32, 0, st>>>(ccarry, ecarry, (CgSavedCarry *)ctx->b_saved.p); ctx->launches++; }
             } else ctx->sl[ctx->n_sl++] = sl[k];
         }
-        if (phase == 0 && (e = enqueue_d2h(ctx, in, out, rprev, r1, i))) { ctx->win_on = 0; return e; }
+        if (phase == 0 && !res_mode && (e = enqueue_d2h(ctx, in, out, rprev, r1, i))) { ctx->win_on = 0; return e; }
         tprev = t1; rprev = r1; jprev = j1;
         trace_at(trace, "slice enqueued (host passed its column sync)", i);
     }
@@ -2321,6 +2444,7 @@ static int process_streamed(cg_ctx *ctx, const cg_batch *in, cg_result *out, con
  *                  thing that runs shard after shard;
  * cg_shard_end     part B1 of the remaining slices, part B2 (over-depth test, painting, rewrite), downloads: concurrent again. */
 extern "C" int cg_shard_begin(cg_ctx *ctx, const cg_batch *in, const cg_window *win, cg_result *out) {
+    if (stream_busy(ctx)) return CG_ERR_STATE;
     if (!win) return CG_ERR_BAD_ARG;
     if (ctx->params.region_tid >= 0) { snprintf(ctx->err, sizeof ctx->err, "region shards and a -r region do not combine"); return CG_ERR_BAD_ARG; }
     cg_window w = *win;
@@ -2329,7 +2453,7 @@ extern "C" int cg_shard_begin(cg_ctx *ctx, const cg_batch *in, const cg_window *
 }
 
 extern "C" int cg_shard_carry(cg_ctx *ctx, const void *carry_in, void *carry_out) {
-    if (ctx->shard_state != 1) return CG_ERR_STATE;
+    if (ctx->shard_state != 1 || stream_busy(ctx)) return CG_ERR_STATE;
     CG_CHECK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     CgChainCarry *ccarry = &((CgScalars *)ctx->b_scal.p)->chain;
@@ -2366,7 +2490,7 @@ extern "C" int cg_shard_carry(cg_ctx *ctx, const void *carry_in, void *carry_out
 }
 
 extern "C" int cg_shard_end(cg_ctx *ctx, cg_result *out) {
-    if (ctx->shard_state != 2) return CG_ERR_STATE;
+    if (ctx->shard_state != 2 || stream_busy(ctx)) return CG_ERR_STATE;
     CG_CHECK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
     const cg_batch *in = ctx->shard_in;
@@ -2389,14 +2513,19 @@ extern "C" int cg_shard_end(cg_ctx *ctx, cg_result *out) {
     return finish_streamed(ctx, out, &ctx->win, ctx->shard_timed, NULL);
 }
 
-extern "C" int cg_process(cg_ctx *ctx, const cg_batch *in, cg_result *out) { return process_streamed(ctx, in, out, NULL, 0); }
+extern "C" int cg_process(cg_ctx *ctx, const cg_batch *in, cg_result *out) {
+    if (stream_busy(ctx) || !in) return CG_ERR_STATE;
+    return process_streamed(ctx, in, out, NULL, 0);
+}
 
 /* One call of a chain (include/crumble_gpu.h): the streamed driver above with a column window.  The column stage runs over all
  * tiles of the batch (columns outside the window come out inert, cg_window_class); the sparse passes of the slice holding the next
  * call's first column stop there, both carries are saved, and the passes finish the rest. */
 extern "C" int cg_process_window(cg_ctx *ctx, const cg_batch *in, const cg_window *win, cg_result *out) {
+    if (stream_busy(ctx)) return CG_ERR_STATE;
     if (!win) return CG_ERR_BAD_ARG;
     if (ctx->params.region_tid >= 0) { snprintf(ctx->err, sizeof ctx->err, "chained calls and a -r region do not combine"); return CG_ERR_BAD_ARG; }
+    if (!in) return CG_ERR_STATE;
     return process_streamed(ctx, in, out, win, 0);
 }
 
@@ -2426,4 +2555,124 @@ extern "C" int cg_carry_is_neutral(const cg_ctx *ctx, const void *buf, int32_t t
     /* depth average: matters only when the over-depth test could fire at all in that call (run_prep) */
     if (ctx->depth_matters && s.ec.valid && s.ec.tid == tid) return -1;
     return open_window ? 0 : 1;
+}
+
+/* ---- a stream of records in GPU memory (include/crumble_gpu.h, DESIGN.md §3.6) ------------------------------------------------------
+ * One call: held ++ in as one working batch (dev_stage), its cut planned on the device and read back at the call's one synchronisation
+ * together with the checked sums; the held set for later calls is copied out of the pristine working arrays (k_retain) before the chain
+ * runs; the chain is process_streamed's window machinery on the resident batch cut to its first m records; k_emit writes the final
+ * prefix [e0, f) to qual_out. */
+static void stream_close(cg_ctx *ctx) {
+    ctx->st_open = 0; ctx->st_unplaced = 0; ctx->st_has_key = 0; ctx->st_kmax = 0;
+    ctx->st_n = ctx->st_e0 = ctx->st_padded = ctx->st_cig = ctx->st_qual = ctx->st_seq = 0;
+    memset(&ctx->st_win, 0, sizeof ctx->st_win); ctx->st_win.first = 1; ctx->st_win.lo_tid = -1;
+}
+
+static int stream_call(cg_ctx *ctx, const cg_dev_batch *in, int last, uint8_t *qual_out, cg_result *out, cg_stream_out *so) {
+    cudaStream_t st = ctx->stream;
+    const int64_t nh = ctx->st_n, e0 = ctx->st_e0, n = nh + in->n_reads;
+    CgScalars *scal = (CgScalars *)ctx->b_scal.p;
+    int e;
+    if (!ctx->h_stream && cudaHostAlloc((void **)&ctx->h_stream, sizeof(CgScalars::CgStreamScal), cudaHostAllocDefault) != cudaSuccess) {
+        cudaGetLastError(); ctx->h_stream = NULL; return CG_ERR_NOMEM;
+    }
+    uint8_t *keep = NULL;
+    e = dev_stage(ctx, in, [&](int64_t *sums) -> int {
+        int e2;
+        if ((e2 = ensure(ctx, &ctx->b_keep, (size_t)n + 1)) || (e2 = ensure(ctx, &ctx->b_kidx, ((size_t)n + 1) * 4)) ||
+            (e2 = ensure(ctx, &ctx->b_koff, ((size_t)n + 1) * 8)) || (e2 = ensure(ctx, &ctx->b_kcig, ((size_t)n + 1) * 4))) return e2;
+        scal = (CgScalars *)ctx->b_scal.p;
+        keep = (uint8_t *)ctx->b_keep.p;
+        CgScalars::CgStreamScal *ss = &scal->stream;
+        const CgDev *D = &ctx->D;
+        k_stream_init<<<1, 1, 0, st>>>(&ss->red);
+        k_prep_read<<<nblk(n, 256), 256, 0, st>>>(*D);
+        k_stream_plan<<<nblk(n, 256), 256, 0, st>>>(*D, n, nh, e0, &ss->red);
+        k_stream_cut<<<1, 1, 0, st>>>(*D, &ss->red, &ss->cut, n, e0, last, (const int64_t *)ctx->b_qsrc.p, sums + 2);
+        k_stream_keep<<<nblk(n, 256), 256, 0, st>>>(*D, &ss->cut, keep, n);
+        CG_CHECK(cudaGetLastError());
+        LdKeep lk = { keep }; StExcl32of64 sk = { (int32_t *)ctx->b_kidx.p };
+        LdKeepPad lp = { keep, D->l_qseq }; StExcl64 sp = { (int64_t *)ctx->b_koff.p };
+        LdKeepCig lc = { keep, D->n_cigar }; StExcl32of64 sc = { (int32_t *)ctx->b_kcig.p };
+        LdKeepLen ll = { keep, D->l_qseq }; LdKeepHalf lh = { keep, D->l_qseq }; StNone none;
+        if ((e2 = run_scan<int64_t, OpSum>(ctx, lk, sk, n, (int64_t)0, &ss->held_n)) || (e2 = run_scan<int64_t, OpSum>(ctx, lp, sp, n, (int64_t)0, &ss->held_padded)) ||
+            (e2 = run_scan<int64_t, OpSum>(ctx, lc, sc, n, (int64_t)0, &ss->held_cig)) || (e2 = run_scan<int64_t, OpSum>(ctx, ll, none, n, (int64_t)0, &ss->held_qual)) ||
+            (e2 = run_scan<int64_t, OpSum>(ctx, lh, none, n, (int64_t)0, &ss->held_seq))) return e2;
+        CG_CHECK(cudaMemcpyAsync(ctx->h_stream, ss, sizeof *ss, cudaMemcpyDeviceToHost, st));
+        ctx->launches += 5;
+        return 0;
+    });
+    if (e) return e;
+    memset(so, 0, sizeof *so);
+    memset(out->counters, 0, sizeof out->counters); out->n_events = 0; out->n_columns = 0;
+    if (n == 0) return 0;                                      /* closing an empty stream */
+    const CgScalars::CgStreamScal hs = *ctx->h_stream;
+    const CgStreamCut c = hs.cut;
+    /* the chunk's first pileup record must not sort before the stream's last one, nor after an unplaced record */
+    if (hs.red.kmin <= hs.red.kmax && ((ctx->st_has_key && hs.red.kmin < ctx->st_kmax) || ctx->st_unplaced)) {
+        snprintf(ctx->err, sizeof ctx->err, "cg_stream_device: this chunk's records sort before records of an earlier chunk");
+        return CG_ERR_UNSORTED;
+    }
+    /* the held set, out of the pristine working arrays, before the chain runs */
+    int64_t hn = hs.held_n, hpad = hs.held_padded, hcig = hs.held_cig;
+    const CgDev *D = &ctx->D;
+    if ((e = ensure(ctx, &ctx->b_htid, (size_t)hn * 4 + 4)) || (e = ensure(ctx, &ctx->b_hpos, (size_t)hn * 4 + 4)) || (e = ensure(ctx, &ctx->b_hflag, (size_t)hn * 2 + 2)) ||
+        (e = ensure(ctx, &ctx->b_hmapq, (size_t)hn + 1)) || (e = ensure(ctx, &ctx->b_hlq, (size_t)hn * 4 + 4)) || (e = ensure(ctx, &ctx->b_hnc, (size_t)hn * 2 + 2)) ||
+        (e = ensure(ctx, &ctx->b_hcig, (size_t)hcig * 4 + 4)) || (e = ensure(ctx, &ctx->b_hqual, (size_t)hpad + 8)) || (e = ensure(ctx, &ctx->b_hseq, (size_t)hpad / 2 + 8))) return e;
+    if ((e = dev_ingest(ctx, in))) return e;
+    if (hn > 0) {
+        const CgRetain K = { D->tid, D->pos, D->l_qseq, D->flag, D->n_cigar, D->mapq, D->off, D->cigar_off, D->cigar, D->qual, D->seq,
+                             (const int32_t *)ctx->b_kidx.p, (const int32_t *)ctx->b_kcig.p, (const int64_t *)ctx->b_koff.p,
+                             (int32_t *)ctx->b_htid.p, (int32_t *)ctx->b_hpos.p, (int32_t *)ctx->b_hlq.p, (uint16_t *)ctx->b_hflag.p, (uint16_t *)ctx->b_hnc.p,
+                             (uint8_t *)ctx->b_hmapq.p, (uint32_t *)ctx->b_hcig.p, (uint8_t *)ctx->b_hqual.p, (uint8_t *)ctx->b_hseq.p };
+        k_retain<<<(unsigned)nblk(n * 32, IO_THREADS), IO_THREADS, 0, st>>>(K, (const uint8_t *)ctx->b_keep.p, n);
+        CG_CHECK(cudaGetLastError());
+    }
+    int64_t n_emit = 0;
+    if (!c.skip) {
+        /* the chain over records [0, m) with this call's window; columns at/after X wait for later calls */
+        cg_window w = ctx->st_win;
+        w.hi_tid = c.hi_tid; w.hi_pos = c.hi_pos; w.next_lo_pos = c.S;
+        ctx->D.n_reads = c.m;
+        ctx->resident = 1; ctx->dump_columns = 0;
+        if ((e = process_streamed(ctx, NULL, out, &w, 0))) return e;
+        n_emit = c.f - e0;
+        if ((e = dev_emit(ctx, e0, c.f, c.q_e0, qual_out))) return e;
+        if (c.hi_tid >= 0) { ctx->st_win.first = 0; ctx->st_win.lo_tid = c.hi_tid; ctx->st_win.lo_pos = c.S; ctx->st_win.cnt_pos = c.hi_pos; }
+        else { ctx->st_win.first = 1; ctx->st_win.lo_tid = -1; ctx->st_win.lo_pos = ctx->st_win.cnt_pos = 0; }
+    } else ctx->resident = 0;                                  /* no chain ran: no events to fetch again */
+    if (hs.red.kmin <= hs.red.kmax) { ctx->st_kmax = hs.red.kmax; ctx->st_has_key = 1; }
+    ctx->st_unplaced |= hs.red.unplaced;
+    ctx->st_n = hn; ctx->st_padded = hpad; ctx->st_cig = hcig; ctx->st_qual = hs.held_qual; ctx->st_seq = hs.held_seq;
+    ctx->st_e0 = hn - (n - c.f);                               /* every record from f on is held: the ones before it are the emitted halo */
+    so->n_records = n_emit; so->qual_len = n_emit ? c.q_f - c.q_e0 : 0;
+    return 0;
+}
+
+extern "C" int cg_stream_device(cg_ctx *ctx, const cg_dev_batch *in, int last, uint8_t *qual_out, int64_t qual_cap, cg_result *out, cg_stream_out *so) {
+    if (!ctx) return CG_ERR_BAD_ARG;
+    cg_dev_batch none; memset(&none, 0, sizeof none);
+    if (!in) in = &none;
+    if (!out || !so) { snprintf(ctx->err, sizeof ctx->err, "cg_stream_device: no result or no cg_stream_out"); return CG_ERR_BAD_ARG; }
+    if (out->columns) { snprintf(ctx->err, sizeof ctx->err, "cg_stream_device: the per-column dump is not available on streams (out->columns must be NULL)"); return CG_ERR_BAD_ARG; }
+    if (ctx->params.region_tid >= 0) { snprintf(ctx->err, sizeof ctx->err, "streams and a -r region do not combine"); return CG_ERR_BAD_ARG; }
+    if (!ctx->st_open) stream_close(ctx);                      /* the state a new stream starts from */
+    if (qual_cap < ctx->st_qual + in->qual_len) {
+        snprintf(ctx->err, sizeof ctx->err, "cg_stream_device: qual_cap %lld < %lld held + %lld new quality bytes", (long long)qual_cap, (long long)ctx->st_qual, (long long)in->qual_len);
+        return CG_ERR_BAD_ARG;
+    }
+    CG_CHECK(cudaSetDevice(ctx->device));
+    int e;
+    if ((e = dev_check(ctx, in, qual_out, qual_cap, out, ctx->st_n + in->n_reads, ctx->st_cig + in->n_cigar_total, ctx->st_qual + in->qual_len))) return e;
+    ctx->st_open = 1;
+    if (in->n_reads == 0 && !last) {                           /* nothing new: nothing can turn final */
+        memset(so, 0, sizeof *so); memset(out->counters, 0, sizeof out->counters); out->n_events = 0; out->n_columns = 0;
+        so->held_records = ctx->st_n; so->held_qual_len = ctx->st_qual;
+        return 0;
+    }
+    ctx->win_on = 0;
+    if ((e = stream_call(ctx, in, last, qual_out, out, so))) { stream_close(ctx); ctx->resident = 0; ctx->win_on = 0; cudaGetLastError(); return e; }
+    if (last) stream_close(ctx);
+    so->held_records = ctx->st_n; so->held_qual_len = ctx->st_qual;
+    return 0;
 }

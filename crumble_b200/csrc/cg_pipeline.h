@@ -703,6 +703,7 @@ typedef struct CgIngest {
     const int64_t *qsrc, *ssrc;                      /* running sums of l_qseq and (l_qseq + 1) / 2: record r in the caller's arrays */
     const uint8_t *qual_in, *seq_in;                 /* the caller's concatenated arrays */
     uint8_t *qual, *seq;                             /* working arrays (past their front padding) */
+    int64_t qbase, sbase;                            /* qsrc / ssrc of the caller's first record (a stream: the held records come first) */
 } CgIngest;
 
 /* ingest, one item per (record r, group k < (l_qseq + 7) / 8): working qual bytes [off + 8k, off + 8k + 8) and seq bytes
@@ -715,8 +716,8 @@ CG_HD void cg_ingest_group(const CgIngest *I, int64_t r, int k) {
     uint64_t q = 0; uint32_t s = 0;
     if (nq > 0) {
         const int ns = ((L + 1) >> 1) - 4 * k;                                  /* > 0 whenever nq > 0 */
-        q = cg_gather8(I->qual_in + I->qsrc[r] + 8 * k, nq < 8 ? nq : 8);
-        s = (uint32_t)cg_gather8(I->seq_in + I->ssrc[r] + 4 * k, ns < 4 ? ns : 4);
+        q = cg_gather8(I->qual_in + (I->qsrc[r] - I->qbase) + 8 * k, nq < 8 ? nq : 8);
+        s = (uint32_t)cg_gather8(I->seq_in + (I->ssrc[r] - I->sbase) + 4 * k, ns < 4 ? ns : 4);
     }
     cg_st_dword(I->qual + o + 8 * k, q);
     cg_st_word(I->seq + (o >> 1) + 4 * k, s);
@@ -726,6 +727,7 @@ typedef struct CgEmit {
     const int32_t *l_qseq; const int64_t *off, *qdst;   /* qdst = qsrc of CgIngest: the concatenated layout */
     const uint8_t *qout;                               /* rewritten qualities, working layout */
     uint8_t *qual_out;                                 /* the caller's concatenated array */
+    int64_t qbase;                                     /* qdst of the record that goes to qual_out[0] */
 } CgEmit;
 
 /* emit, one item per (record r, j < cg_emit_words): the 8-byte aligned words of the caller's array that hold bytes of record r.
@@ -733,17 +735,122 @@ typedef struct CgEmit {
 CG_HD int cg_emit_words(const CgEmit *E, int64_t r) {
     const int L = E->l_qseq[r];
     if (L <= 0) return 0;
-    const uintptr_t d0 = (uintptr_t)(E->qual_out + E->qdst[r]);
+    const uintptr_t d0 = (uintptr_t)(E->qual_out + (E->qdst[r] - E->qbase));
     return (int)(((d0 + (uintptr_t)L - 1) >> 3) - (d0 >> 3) + 1);
 }
 CG_HD void cg_emit_word(const CgEmit *E, int64_t r, int j) {
     const int64_t L = E->l_qseq[r];
-    uint8_t *dst = E->qual_out + E->qdst[r];
+    uint8_t *dst = E->qual_out + (E->qdst[r] - E->qbase);
     const int64_t x = -(int64_t)((uintptr_t)dst & 7) + 8 * (int64_t)j;        /* record byte at the word's first address */
     const int64_t x0 = x > 0 ? x : 0, x1 = x + 8 < L ? x + 8 : L;
     const uint64_t v = cg_gather8(E->qout + E->off[r] + x0, (int)(x1 - x0));
     if (x0 == x && x1 == x + 8) cg_st_dword(dst + x, v);
     else for (int64_t b = x0; b < x1; b++) dst[b] = (uint8_t)(v >> (8 * (b - x0)));
+}
+
+/* ---- streams (cg_stream_device, DESIGN.md §3.6) ----------------------------------------------------------------------------------
+ * One call works on held ++ in (n records; the first e0 of them were emitted by earlier calls).  Every quantity of the cut is a min or
+ * max over the records, so the device reduces them with atomics and the emulation with plain loops over the same per-record body. */
+typedef struct CgStreamRed {
+    int32_t mmax;             /* last record whose key differs from the last record's (-1: none): m = mmax + 1 */
+    int32_t mtid;             /* the same among records on the last record's contig: the held-back run continues record m-1's contig iff equal */
+    int32_t smin;             /* smallest start of a pileup record on the last record's contig that ends beyond its position (INT_MAX: none) */
+    int32_t fmin;             /* first such record at or after e0 (INT_MAX: none) */
+    uint64_t kmin, kmax;      /* smallest / largest key of the pileup records of `in` (kmin > kmax: none) */
+    int32_t unplaced;         /* `in` holds a record with tid < 0 */
+    int32_t pad;
+} CgStreamRed;
+
+CG_HD void cg_stream_red_init(CgStreamRed *R) {
+    R->mmax = -1; R->mtid = -1; R->smin = 0x7fffffff; R->fmin = 0x7fffffff; R->kmin = ~0ull; R->kmax = 0; R->unplaced = 0; R->pad = 0;
+}
+/* record r's contribution (identities where it has none); rspan[] as cg_prep_read leaves it, so the end is the pileup's own */
+CG_HD CgStreamRed cg_stream_plan_item(const CgDev *D, int64_t r, int64_t n, int64_t n_held, int64_t e0) {
+    CgStreamRed c; cg_stream_red_init(&c);
+    const int32_t tL = D->tid[n - 1], pL = D->pos[n - 1], t = D->tid[r], p = D->pos[r], sp = D->rspan[r];
+    if (t != tL || p != pL) { c.mmax = (int32_t)r; if (t == tL) c.mtid = (int32_t)r; }
+    if (sp && t == tL && (int64_t)p + sp > pL) { c.smin = p; if (r >= e0) c.fmin = (int32_t)r; }
+    if (r >= n_held) {
+        if (sp) c.kmin = c.kmax = (uint64_t)cg_key(t, p);
+        if (t < 0) c.unplaced = 1;
+    }
+    return c;
+}
+CG_HD void cg_stream_red_merge(CgStreamRed *a, const CgStreamRed *b) {
+    if (b->mmax > a->mmax) a->mmax = b->mmax;
+    if (b->mtid > a->mtid) a->mtid = b->mtid;
+    if (b->smin < a->smin) a->smin = b->smin;
+    if (b->fmin < a->fmin) a->fmin = b->fmin;
+    if (b->kmin < a->kmin) a->kmin = b->kmin;
+    if (b->kmax > a->kmax) a->kmax = b->kmax;
+    a->unplaced |= b->unplaced;
+}
+
+typedef struct CgStreamCut {
+    int32_t m;                /* the call covers records [0, m); [m, n) is the held-back run */
+    int32_t f;                /* records [e0, f) are final and emitted */
+    int32_t hi_tid, hi_pos;   /* X: the columns at/after it are left to later calls (hi_tid < 0: none) */
+    int32_t S;                /* next_lo_pos: the smallest start of a record of the call reaching beyond X (X if none) */
+    int32_t skip;             /* m <= e0: the call covers no record that is not emitted yet; it runs nothing and holds everything */
+    int64_t q_e0, q_f;        /* concatenated quality offsets of records e0 and f */
+} CgStreamCut;
+
+/* the cut from the reductions; qsrc[] = running sum of l_qseq over the working batch, q_total its total */
+CG_HD CgStreamCut cg_stream_cut(const CgDev *D, const CgStreamRed *R, int64_t n, int64_t e0, int last, const int64_t *qsrc, int64_t q_total) {
+    CgStreamCut c; memset(&c, 0, sizeof c);
+    c.hi_tid = -1;
+    c.m = (int32_t)n;
+    if (!last && n > 0 && D->tid[n - 1] >= 0) {              /* after an unplaced record only unplaced ones follow: nothing to hold back */
+        c.m = R->mmax + 1;
+        if (R->mmax >= 0 && R->mtid == R->mmax) { c.hi_tid = D->tid[n - 1]; c.hi_pos = D->pos[n - 1]; }
+    }
+    c.S = c.hi_tid >= 0 && R->smin < c.hi_pos ? R->smin : c.hi_pos;
+    c.f = c.hi_tid >= 0 && R->fmin < c.m ? R->fmin : c.m;
+    c.skip = c.m <= e0;
+    if (c.skip) c.f = (int32_t)e0;
+    c.q_e0 = e0 < n ? qsrc[e0] : q_total;
+    c.q_f = c.f < n ? qsrc[c.f] : q_total;
+    return c;
+}
+
+/* record r stays for later calls: the read halo before f (pileup records on hi_tid reaching beyond S), then everything from f on */
+CG_HD int cg_stream_keep(const CgDev *D, int64_t r, const CgStreamCut *c) {
+    if (c->skip || r >= c->f) return 1;
+    return c->hi_tid >= 0 && D->rspan[r] && D->tid[r] == c->hi_tid && (int64_t)D->pos[r] + D->rspan[r] > c->S;
+}
+
+typedef struct CgRetain {
+    const int32_t *tid, *pos, *l_qseq; const uint16_t *flag, *n_cigar; const uint8_t *mapq;
+    const int64_t *off; const int32_t *cigar_off; const uint32_t *cigar; const uint8_t *qual, *seq;   /* working batch */
+    const int32_t *didx, *dcig; const int64_t *doff;                   /* where kept record r goes: exclusive scans over the keep flag */
+    int32_t *h_tid, *h_pos, *h_lq; uint16_t *h_flag, *h_nc; uint8_t *h_mapq;
+    uint32_t *h_cigar; uint8_t *h_qual, *h_seq;                        /* the held store, in the working layout */
+} CgRetain;
+
+/* one item per (kept record r, j < cg_retain_items): item 0 moves the per-record fields; item j moves the j-th 8-byte word of the padded
+ * qualities, the j-th 4-byte word of the sequence and the j-th CIGAR operation, where they exist */
+CG_HD int cg_retain_items(const CgRetain *K, int64_t r) {
+    const int w = (K->l_qseq[r] + 7) >> 3, nc = K->n_cigar[r];
+    const int v = w > nc ? w : nc;
+    return v > 1 ? v : 1;
+}
+CG_HD void cg_retain_item(const CgRetain *K, int64_t r, int j) {
+    const int64_t d = K->didx[r];
+    if (j == 0) {
+        K->h_tid[d] = K->tid[r]; K->h_pos[d] = K->pos[r]; K->h_lq[d] = K->l_qseq[r];
+        K->h_flag[d] = K->flag[r]; K->h_nc[d] = K->n_cigar[r]; K->h_mapq[d] = K->mapq[r];
+    }
+    if (j < K->n_cigar[r]) K->h_cigar[K->dcig[r] + j] = K->cigar[K->cigar_off[r] + j];
+    if (j < (K->l_qseq[r] + 7) >> 3) {
+        const int64_t s = K->off[r] + 8 * (int64_t)j, t = K->doff[r] + 8 * (int64_t)j;
+#ifdef __CUDA_ARCH__
+        *(uint64_t *)(K->h_qual + t) = *(const uint64_t *)(K->qual + s);
+        *(uint32_t *)(K->h_seq + (t >> 1)) = *(const uint32_t *)(K->seq + (s >> 1));
+#else
+        memcpy(K->h_qual + t, K->qual + s, 8);
+        memcpy(K->h_seq + (t >> 1), K->seq + (s >> 1), 4);
+#endif
+    }
 }
 
 #endif /* CG_PIPELINE_H */

@@ -215,6 +215,28 @@ typedef struct cg_dev_batch {
  * and cg_last_h2d_bytes reads 0. */
 int cg_process_device(cg_ctx *ctx, const cg_dev_batch *in, uint8_t *qual_out, cg_result *out);
 
+/* ---- a stream of records in GPU memory, pushed in chunks of any size (DESIGN.md §3.6) ---------------------------------------------
+ * The first call opens a stream on the context; each call appends `in` (the next records of one coordinate-sorted stream; NULL or
+ * n_reads 0 allowed) and writes to qual_out (device) the rewritten qualities of the FINAL PREFIX of the stream, back to back in the
+ * concatenated layout of cg_process_device: every record not emitted yet, up to the first one that is not final yet.  Records come out
+ * in exactly the order they went in, so a producer that keeps names and aux data on its side pairs them up as a FIFO.  last = 1 ends
+ * the stream: everything held is flushed and the stream closes.  out gets the BED events and counters of the columns this call owns:
+ * the events of all calls concatenated and the counters summed equal one cg_process_device on the whole stream, as do the qualities.
+ * out->qual_out, out->qual_head and out->columns must be NULL; a longer event list comes again through cg_download (qual_out = NULL).
+ * in's buffers are free once the stream has passed the call, and qual_out may alias in->qual.
+ * CG_ERR_BAD_ARG before anything is enqueued, with the context and the open stream unchanged: whatever cg_process_device rejects,
+ * qual_cap < held_qual_len + in->qual_len, out->columns set, a -r region in the parameters.  Any later error (sums that disagree, a
+ * chunk that breaks the sort order: CG_ERR_UNSORTED, CUDA errors) closes the stream and drops what it held; the context stays usable.
+ * While a stream is open, cg_process, cg_process_device, cg_process_window, cg_upload, cg_run, cg_shard_*, cg_set_params and
+ * cg_set_stream return CG_ERR_STATE. */
+typedef struct cg_stream_out {
+    int64_t n_records;        /* records whose final qualities this call wrote: the next n_records of the stream, in stream order */
+    int64_t qual_len;         /* bytes written to qual_out = sum of their l_qseq */
+    int64_t held_records;     /* records the context now holds for later calls (read halo + not yet final + held-back tail) */
+    int64_t held_qual_len;    /* their quality bytes: the next call needs qual_cap >= held_qual_len + its in->qual_len */
+} cg_stream_out;
+int cg_stream_device(cg_ctx *ctx, const cg_dev_batch *in, int last, uint8_t *qual_out, int64_t qual_cap, cg_result *out, cg_stream_out *so);
+
 /* ---- chained calls: a coordinate-sorted stream of any length in bounded memory ------------
  * (region shards with a read halo, SURVEY.md §8(e): the reference keeps its state in a streaming loop, snp_score.c:1437-1975)
  * The caller cuts the stream wherever it likes.  Let X be the position of the first record AFTER call k (same contig),
