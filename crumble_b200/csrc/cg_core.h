@@ -83,11 +83,15 @@ CG_HD int cg_cig_type(int op)    { return (0x3C1A7 >> (op << 1)) & 3; }   /* bit
 CG_HD bool cg_is_refop(int op)   { return op == 0 || op == 2 || op == 3 || op == 7 || op == 8; }
 CG_HD bool cg_is_mop(int op)     { return op == 0 || op == 7 || op == 8; }
 
-/* reference span and "no ref-consuming op" test (bam_endpos; pileup_callback snp_score.c:1135-1146) */
-CG_HD int cg_ref_span(const uint32_t *cig, int n) {
-    int s = 0;
-    for (int k = 0; k < n; k++) if (cg_cig_type(cg_cig_op(cig[k])) & 2) s += cg_cig_len(cig[k]);
-    return s;
+/* A record's pileup span, the one definition every cut, halo and batch end derives from (its end is pos + span): 0 outside the pileup
+ * (unplaced, unmapped, or no op consumes the reference; bam_plp_push + pileup_callback snp_score.c:1125-1149), else the reference
+ * span, at least 1 (bam_endpos: pos+1 when the ops that consume the reference have length 0) */
+CG_HD int cg_pileup_span(int32_t tid, int flag, const uint32_t *cig, int n) {
+    int span = 0, hasref = 0;
+    for (int k = 0; k < n; k++)
+        if (cg_cig_type(cg_cig_op(cig[k])) & 2) { span += cg_cig_len(cig[k]); hasref = 1; }
+    if (tid < 0 || (flag & 4) || !hasref) return 0;
+    return span ? span : 1;
 }
 
 /* One pileup cell: what htslib's bam_plp_auto reports for (read, column) — restated in

@@ -12,6 +12,7 @@
 #include <unistd.h>
 #include "cg_pipeline.h"
 #include "cg_host.h"
+#include "crumble_host.h"
 
 /* Which option combinations the device path implements today. */
 int cg_params_check(const cg_params *p, const char **why) {
@@ -225,10 +226,7 @@ extern "C" int cgb_add(cg_batch_builder *b, int32_t tid, int32_t pos, uint16_t f
     b->tid.n = b->pos.n = b->l_qseq.n = b->cigar_off.n = b->flag.n = b->n_cigar.n = b->mapq.n = b->off.n = i + 1;
     {   /* running max of the record ends inside the contig (cg_batch.pmax_end) */
         if (b->pmax.reserve(i + 1)) return CG_ERR_NOMEM;
-        int span = 0, hasref = 0;
-        for (uint32_t k = 0; k < n_cigar; k++) if (cg_cig_type(cg_cig_op(cigar[k])) & 2) { span += cg_cig_len(cigar[k]); hasref = 1; }
-        const int inp = tid >= 0 && !(flag & 4) && hasref;
-        const int32_t e = pos + (inp ? (span ? span : 1) : 0);
+        const int32_t e = pos + cg_pileup_span(tid, flag, cigar, (int)n_cigar);
         b->pmax.p[i] = (i > 0 && b->tid.p[i - 1] == tid && b->pmax.p[i - 1] > e) ? b->pmax.p[i - 1] : e;
         b->pmax.n = i + 1;
     }
@@ -477,30 +475,23 @@ extern "C" int64_t cgb_bytes(const cg_batch_builder *b) {
     return (int64_t)(b->tid.n * (4 + 4 + 4 + 4 + 2 + 2 + 1 + 8) + b->cigar.n * 4 + b->seq.n + b->qual.n);
 }
 
-static int batch_in_pileup(const cg_batch *in, int64_t i) {
-    if (in->tid[i] < 0 || (in->flag[i] & 4)) return 0;
-    const uint32_t *c = in->cigar + in->cigar_off[i];
-    for (int k = 0; k < in->n_cigar[i]; k++) if (cg_cig_type(cg_cig_op(c[k])) & 2) return 1;
-    return 0;
+extern "C" int32_t cg_record_end(int32_t tid, int32_t pos, uint16_t flag, const uint32_t *cigar, int n_cigar) {
+    return pos + cg_pileup_span(tid, flag, cigar, n_cigar);
+}
+static int batch_span(const cg_batch *in, int64_t i) {
+    return cg_pileup_span(in->tid[i], in->flag[i], in->cigar + in->cigar_off[i], in->n_cigar[i]);
 }
 extern "C" void cg_batch_ends(const cg_batch *in, int32_t *end_out) {
-    for (int64_t i = 0; i < in->n_reads; i++) {
-        int span = 0, hasref = 0;
-        const uint32_t *c = in->cigar + in->cigar_off[i];
-        for (int k = 0; k < in->n_cigar[i]; k++) if (cg_cig_type(cg_cig_op(c[k])) & 2) { span += cg_cig_len(c[k]); hasref = 1; }
-        const int inp = in->tid[i] >= 0 && !(in->flag[i] & 4) && hasref;
-        if (inp && span == 0) span = 1;
-        end_out[i] = in->pos[i] + (inp ? span : 0);
-    }
+    for (int64_t i = 0; i < in->n_reads; i++) end_out[i] = in->pos[i] + batch_span(in, i);
 }
 extern "C" int64_t cg_algorithmic_bytes(const cg_batch *in) {           /* SURVEY.md §8(d) */
     int64_t s = 0;
     for (int64_t i = 0; i < in->n_reads; i++)
-        if (batch_in_pileup(in, i)) { int64_t l = in->l_qseq[i]; s += ((l + 1) >> 1) + 2 * l + 4 * (int64_t)in->n_cigar[i] + 16; }
+        if (batch_span(in, i)) { int64_t l = in->l_qseq[i]; s += ((l + 1) >> 1) + 2 * l + 4 * (int64_t)in->n_cigar[i] + 16; }
     return s;
 }
 extern "C" int64_t cg_aligned_bases(const cg_batch *in) {
     int64_t s = 0;
-    for (int64_t i = 0; i < in->n_reads; i++) if (batch_in_pileup(in, i)) s += in->l_qseq[i];
+    for (int64_t i = 0; i < in->n_reads; i++) if (batch_span(in, i)) s += in->l_qseq[i];
     return s;
 }

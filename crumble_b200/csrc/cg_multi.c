@@ -18,7 +18,7 @@
 #include <stdlib.h>
 #include <string.h>
 #include <pthread.h>
-#include "../../include/crumble_gpu.h"
+#include "crumble_host.h"
 
 typedef struct {
     struct cg_multi *m; int k;
@@ -177,14 +177,11 @@ static void *shard_main(void *v) {
     return NULL;
 }
 
-/* pos + reference span of one record (pos itself outside the pileup), as cg_batch_ends computes it for all */
-static int32_t rec_end(const cg_batch *in, int64_t i) {
-    if (in->tid[i] < 0 || (in->flag[i] & 4)) return in->pos[i];
-    const uint32_t *c = in->cigar + in->cigar_off[i];
-    int span = 0, hasref = 0;
-    for (int k = 0; k < in->n_cigar[i]; k++) { const int op = (int)(c[k] & 15); if ((0x3C1A7 >> (op << 1)) & 2) { span += (int)(c[k] >> 4); hasref = 1; } }
-    if (!hasref) return in->pos[i];
-    return in->pos[i] + (span ? span : 1);
+/* record i is open at the cut (tid, limit): a pileup record (end > pos) on contig tid that ends beyond limit */
+static int open_at(const cg_batch *in, int64_t i, int32_t tid, int32_t limit) {
+    if (in->tid[i] != tid) return 0;
+    const int32_t e = cg_record_end(in->tid[i], in->pos[i], in->flag[i], in->cigar + in->cigar_off[i], in->n_cigar[i]);
+    return e > in->pos[i] && e > limit;
 }
 /* first record of contig tid (records are sorted by (tid, pos), unplaced ones last) at or after index lo */
 static int64_t contig_start(const cg_batch *in, int32_t tid, int64_t hi) {
@@ -210,7 +207,10 @@ int cgm_process_window(cg_multi *m, const cg_batch *in, const cg_window *win, cg
     if (!pmax && n > 0) {
         own_pmax = (int32_t *)malloc(sizeof(int32_t) * (size_t)n);
         if (!own_pmax) return CG_ERR_NOMEM;
-        for (int64_t i = 0; i < n; i++) { const int32_t e = rec_end(in, i); own_pmax[i] = (i > 0 && in->tid[i] == in->tid[i - 1] && own_pmax[i - 1] > e) ? own_pmax[i - 1] : e; }
+        for (int64_t i = 0; i < n; i++) {
+            const int32_t e = cg_record_end(in->tid[i], in->pos[i], in->flag[i], in->cigar + in->cigar_off[i], in->n_cigar[i]);
+            own_pmax[i] = (i > 0 && in->tid[i] == in->tid[i - 1] && own_pmax[i - 1] > e) ? own_pmax[i - 1] : e;
+        }
         pmax = own_pmax;
     }
     m->n_sh = N; m->first_needs_carry = 0;
@@ -238,7 +238,7 @@ int cgm_process_window(cg_multi *m, const cg_batch *in, const cg_window *win, cg
             if (a < s->h0) a = s->h0;
             const int64_t iS = first_reaching(pmax, a, s->r1, X);
             /* pmax may carry an end from before `a`: the first record of [a, r1) that really reaches X */
-            int64_t ii = iS; while (ii < s->r1 && rec_end(in, ii) <= X) ii++;
+            int64_t ii = iS; while (ii < s->r1 && !open_at(in, ii, t, X)) ii++;
             int32_t S = ii < s->r1 ? in->pos[ii] : X;
             /* a chained call whose first shards hold nothing but halo records: a cut below the first column this CALL owns (X < cnt_pos) must
              * neither make the next shard count the columns in between again (the previous call of the chain counted them), nor start its
@@ -288,10 +288,8 @@ int cgm_process_window(cg_multi *m, const cg_batch *in, const cg_window *win, cg
                 const cgm_shard *l = &m->sh[k - 1];
                 const int64_t base = in->off[s->h0];
                 for (int64_t i = s->h0; i < s->r0; i++) {
-                    if (in->tid[i] != l->win.hi_tid || in->l_qseq[i] <= 0) continue;
-                    const int32_t e = rec_end(in, i);
-                    if (!(e > in->pos[i] && e > l->win.hi_pos)) continue;                 /* was final in an earlier shard */
-                    if (s->win.hi_tid >= 0 && in->tid[i] == s->win.hi_tid && e > s->win.hi_pos) continue;   /* still open: a later shard has it in its halo too */
+                    if (in->l_qseq[i] <= 0 || !open_at(in, i, l->win.hi_tid, l->win.hi_pos)) continue;   /* was final in an earlier shard */
+                    if (open_at(in, i, s->win.hi_tid, s->win.hi_pos)) continue;     /* still open: a later shard has it in its halo too */
                     /* open at every cut since its own shard, closed here: but only the FIRST shard after its last open cut holds the final bytes, and
                      * that is this one, because it was still open at the cut just before */
                     memcpy(out->qual_out + in->off[i], s->head + (in->off[i] - base), (size_t)in->l_qseq[i]);

@@ -102,20 +102,11 @@ typedef struct CgDev {
 CG_HD int64_t cg_key(int32_t tid, int32_t pos) { return ((int64_t)tid << 32) | (uint32_t)pos; }
 
 /* ---- stage: prep_read (one per record) ------------------------------------------------
- * pileup eligibility as bam_plp_push + pileup_callback (snp_score.c:1125-1149; SURVEY §9.2) */
+ * rspan[r] = cg_pileup_span: pileup eligibility as bam_plp_push + pileup_callback (SURVEY §9.2) */
 CG_HD void cg_prep_read(const CgDev *D, int64_t r) {
-    int32_t tid = D->tid[r];
     int n = D->n_cigar[r];
     if (D->cigar_off[r] < 0 || (int64_t)D->cigar_off[r] + n > D->n_cigar_total) { *D->err = CG_ERR_BAD_ARG; D->rspan[r] = 0; return; }   /* a layout that lies about its CIGARs */
-    const uint32_t *cig = D->cigar + D->cigar_off[r];
-    int span = 0, hasref = 0;
-    for (int k = 0; k < n; k++) {
-        int t = cg_cig_type(cg_cig_op(cig[k]));
-        if (t & 2) { span += cg_cig_len(cig[k]); hasref = 1; }
-    }
-    int in = (tid >= 0) && !(D->flag[r] & 4) && hasref;
-    if (in && span == 0) span = 1;                 /* bam_endpos: pos+1 when nothing consumes the reference */
-    D->rspan[r] = in ? span : 0;
+    D->rspan[r] = cg_pileup_span(D->tid[r], D->flag[r], D->cigar + D->cigar_off[r], n);
 }
 
 /* after the pileup-flag scan: fill compact keys */
@@ -764,12 +755,18 @@ typedef struct CgStreamRed {
 CG_HD void cg_stream_red_init(CgStreamRed *R) {
     R->mmax = -1; R->mtid = -1; R->smin = 0x7fffffff; R->fmin = 0x7fffffff; R->kmin = ~0ull; R->kmax = 0; R->unplaced = 0; R->pad = 0;
 }
+/* A record is open at the cut (cut_tid, limit): a pileup record (span = cg_pileup_span) on contig cut_tid that ends beyond limit.
+ * With limit = X it is not final yet; with limit = S it belongs to the next call's read halo. */
+CG_HD bool cg_open_at(int32_t tid, int32_t pos, int32_t span, int32_t cut_tid, int32_t limit) {
+    return span && tid == cut_tid && (int64_t)pos + span > limit;
+}
+
 /* record r's contribution (identities where it has none); rspan[] as cg_prep_read leaves it, so the end is the pileup's own */
 CG_HD CgStreamRed cg_stream_plan_item(const CgDev *D, int64_t r, int64_t n, int64_t n_held, int64_t e0) {
     CgStreamRed c; cg_stream_red_init(&c);
     const int32_t tL = D->tid[n - 1], pL = D->pos[n - 1], t = D->tid[r], p = D->pos[r], sp = D->rspan[r];
     if (t != tL || p != pL) { c.mmax = (int32_t)r; if (t == tL) c.mtid = (int32_t)r; }
-    if (sp && t == tL && (int64_t)p + sp > pL) { c.smin = p; if (r >= e0) c.fmin = (int32_t)r; }
+    if (cg_open_at(t, p, sp, tL, pL)) { c.smin = p; if (r >= e0) c.fmin = (int32_t)r; }
     if (r >= n_held) {
         if (sp) c.kmin = c.kmax = (uint64_t)cg_key(t, p);
         if (t < 0) c.unplaced = 1;
@@ -816,7 +813,8 @@ CG_HD CgStreamCut cg_stream_cut(const CgDev *D, const CgStreamRed *R, int64_t n,
 /* record r stays for later calls: the read halo before f (pileup records on hi_tid reaching beyond S), then everything from f on */
 CG_HD int cg_stream_keep(const CgDev *D, int64_t r, const CgStreamCut *c) {
     if (c->skip || r >= c->f) return 1;
-    return c->hi_tid >= 0 && D->rspan[r] && D->tid[r] == c->hi_tid && (int64_t)D->pos[r] + D->rspan[r] > c->S;
+    const int32_t sp = D->rspan[r];
+    return sp && cg_open_at(D->tid[r], D->pos[r], sp, c->hi_tid, c->S);    /* rspan first: tid and pos are loaded for pileup records only */
 }
 
 typedef struct CgRetain {

@@ -37,6 +37,8 @@ void crumble_print_counters(const crumble_opts *o);        /* -v block, snp_scor
 void crumble_purge_tags(const crumble_opts *o, bam1_t *b); /* snp_score.c:989-1054 */
 cg_bed_reg *crumble_bed_load(const char *fn, bam_hdr_t *header, int *nreg);   /* bed.c:42-103 */
 int  transcode_gpu(crumble_opts *o, samFile *in, samFile *out, bam_hdr_t *header, hts_itr_t *h_iter);
+/* pos + cg_pileup_span (cg_core.h): a pileup record's end (exclusive), pos itself for any other record (cg_host.cpp) */
+int32_t cg_record_end(int32_t tid, int32_t pos, uint16_t flag, const uint32_t *cigar, int n_cigar);
 int  crumble_main(int argc, char **argv);
 
 #ifdef __cplusplus

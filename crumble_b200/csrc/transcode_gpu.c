@@ -101,8 +101,8 @@ static void *writer_main(void *v) {
 typedef struct {
     bam1_t  *b;             /* NULL once written and destroyed (then oq/meta below serve the halo) */
     uint8_t *oq;            /* original qualities, saved when the record turns final while later calls still need it */
-    int32_t  end;           /* pos + reference span (exclusive) for pileup records */
-    uint8_t  in_pileup, final, is_new;
+    int32_t  end;           /* cg_record_end: pos + pileup span, pos itself outside the pileup */
+    uint8_t  final, is_new;
     int64_t  slot;          /* index in the current batch, -1 when not part of it */
 } live_rec;
 
@@ -124,15 +124,14 @@ static int lq_push(live_q *q, bam1_t *b) {
     live_rec *r = &q->v[q->n++];
     memset(r, 0, sizeof(*r));
     r->b = b; r->is_new = 1; r->slot = -1;
-    /* pileup eligibility and reference span exactly as the device decides them (cg_prep_read; snp_score.c:1125-1149) */
-    int span = 0, hasref = 0;
-    const uint32_t *cig = bam_get_cigar(b);
-    for (uint32_t k = 0; k < b->core.n_cigar; k++)
-        if (bam_cigar_type(bam_cigar_op(cig[k])) & 2) { span += (int)bam_cigar_oplen(cig[k]); hasref = 1; }
-    r->in_pileup = b->core.tid >= 0 && !(b->core.flag & BAM_FUNMAP) && hasref;
-    if (r->in_pileup && span == 0) span = 1;
-    r->end = b->core.pos + (r->in_pileup ? span : 0);
+    r->end = cg_record_end(b->core.tid, b->core.pos, b->core.flag, bam_get_cigar(b), (int)b->core.n_cigar);
     return 0;
+}
+
+/* r is open at the cut (tid, limit): a pileup record (end > pos) on contig tid that ends beyond limit.  With limit = the cut's
+ * position the record is not final yet; with limit = S it belongs to the next call's read halo. */
+static int reaches(const live_rec *r, int32_t tid, int32_t limit) {
+    return r->b->core.tid == tid && r->end > r->b->core.pos && r->end > limit;
 }
 
 static void lq_free(live_q *q) {
@@ -260,13 +259,13 @@ int transcode_gpu(crumble_opts *o, samFile *in, samFile *out, bam_hdr_t *header,
         for (size_t i = lq.head; i < lq.n; i++) {
             live_rec *r = &lq.v[i];
             r->slot = -1;
-            if (!r->is_new && !(r->b && r->in_pileup && !first && r->b->core.tid == lo_tid && r->end > lo_pos)) continue;
+            if (!r->is_new && !(r->b && !first && reaches(r, lo_tid, lo_pos))) continue;
             const bam1_t *b = r->b;
             int e = cgb_add(bb, b->core.tid, b->core.pos, b->core.flag, b->core.qual, b->core.l_qseq, b->core.n_cigar,
                             bam_get_cigar(b), bam_get_seq(b), r->oq ? r->oq : bam_get_qual(b));
             if (e) { fprintf(stderr, "crumble: %s\n", cg_strerror(e)); goto done; }
             r->slot = nb++;
-            if (win.hi_tid >= 0 && r->in_pileup && b->core.tid == win.hi_tid && r->end > win.hi_pos && b->core.pos < S) S = b->core.pos;
+            if (reaches(r, win.hi_tid, win.hi_pos) && b->core.pos < S) S = b->core.pos;
         }
         win.next_lo_pos = S;
         cg_batch batch;
@@ -310,9 +309,9 @@ int transcode_gpu(crumble_opts *o, samFile *in, samFile *out, bam_hdr_t *header,
             r->is_new = 0;
             if (r->final || r->slot < 0) continue;
             bam1_t *b = r->b;
-            if (win.hi_tid >= 0 && r->in_pileup && b->core.tid == win.hi_tid && r->end > win.hi_pos) continue;
+            if (reaches(r, win.hi_tid, win.hi_pos)) continue;
             if (b->core.l_qseq) {
-                if (win.hi_tid >= 0 && r->in_pileup && b->core.tid == win.hi_tid && r->end > S) {   /* part of the next halo */
+                if (reaches(r, win.hi_tid, S)) {                                /* part of the next halo */
                     r->oq = (uint8_t *)malloc((size_t)b->core.l_qseq);
                     if (!r->oq) goto done;
                     memcpy(r->oq, bam_get_qual(b), (size_t)b->core.l_qseq);
@@ -330,7 +329,7 @@ int transcode_gpu(crumble_opts *o, samFile *in, samFile *out, bam_hdr_t *header,
                 if (!r->final) blocked = 1;
                 if (!blocked && r->final != 2) {
                     /* to the writer thread, which owns what it gets; a record the next call still needs as halo goes as a copy */
-                    const int needed = win.hi_tid >= 0 && r->in_pileup && r->b->core.tid == win.hi_tid && r->end > S;
+                    const int needed = reaches(r, win.hi_tid, S);
                     bam1_t *w = needed ? bam_dup1(r->b) : r->b;
                     if (!w) goto done;
                     if (!needed) r->b = NULL;
@@ -345,7 +344,7 @@ int transcode_gpu(crumble_opts *o, samFile *in, samFile *out, bam_hdr_t *header,
             for (i = lq.head; i < lq.n; i++) {
                 live_rec *r = &lq.v[i];
                 if (r->final != 2 || !r->b) continue;
-                if (!(win.hi_tid >= 0 && r->in_pileup && r->b->core.tid == win.hi_tid && r->end > S)) { bam_destroy1(r->b); r->b = NULL; }
+                if (!reaches(r, win.hi_tid, S)) { bam_destroy1(r->b); r->b = NULL; }
             }
             /* drop from the head every written record the next call does not need as halo */
             while (lq.head < lq.n) {
